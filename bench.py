@@ -16,7 +16,7 @@ The same JSON line carries
     gathered on rank 0's host memory inside the clock (C2: 1 Mi pairs in total; C5: 64 pairs in total,
     8 per GPU at N = 8).  Strong scaling; no NCCL on the data path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--pairs P]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--pairs P] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 Prints ONE JSON line on rank 0.  The oracle (oracle/) is executed only for the `cpu_baseline` objects and for
@@ -230,6 +230,41 @@ def roofline_of(tm, mode_key, k_ms, sm_max_mhz, hbm_peak, peak_src, seq_bytes):
     return r
 
 
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(res, out_dir):
+    """Write what the caller of the timed path receives (scores, start / end cells, CIGARs) as out_dir/<name>.npy, so
+    that two builds run with the same arguments can be compared output for output.  When the whole result would exceed
+    DUMP_MAX_BYTES, the dump is the largest prefix of a fixed, seeded permutation of the pairs that fits, in pair
+    order (pair_index.npy).  Scores, cells and packed CIGAR ops are below 2^24, so float32 holds them exactly; CIGAR
+    offsets are float64."""
+    n = res.n
+    off = res.cigar_off.astype(np.int64)
+    lens_all = np.diff(off[:n + 1])
+    # bytes per pair: five float32 fields, a float64 offset (and a float64 pair_index when sampled), 4 per CIGAR op;
+    # the budget keeps room for the final offset and the .npy headers
+    budget = DUMP_MAX_BYTES - 8 - 4096
+    if 28 * n + 4 * int(lens_all.sum()) <= budget:
+        idx = np.arange(n)
+    else:
+        perm = np.random.default_rng(0).permutation(n)
+        cost = np.cumsum(36 + 4 * lens_all[perm])
+        idx = np.sort(perm[:int(np.searchsorted(cost, budget, side="right"))])
+    lens = lens_all[idx]
+    sub_off = np.zeros(len(idx) + 1, np.int64)
+    np.cumsum(lens, out=sub_off[1:])
+    take = np.repeat(off[idx] - sub_off[:-1], lens) + np.arange(sub_off[-1])
+    arrs = {k: getattr(res, k)[idx].astype(np.float32) for k in ("score", "end_i", "end_j", "beg_i", "beg_j")}
+    arrs["cigar_off"] = sub_off.astype(np.float64)
+    arrs["cigar"] = res.cigar[take].astype(np.float32)
+    if len(idx) < n:
+        arrs["pair_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def mode_key_of(w):
     return "fitjump" if (w["mode"] == "fit" and w["params"]["jump"]) else w["mode"]
 
@@ -405,7 +440,10 @@ def main():
     ap.add_argument("--c5-pairs", type=int, default=8, help="C5 pairs per GPU (BASELINE: 64 pairs over 8 GPUs)")
     ap.add_argument("--cfg-steps", type=int, default=3)
     ap.add_argument("--bytes-e2e", action="store_true", help="C2 e2e leg hands over byte-encoded sequences instead of AT_SEQ_2BIT")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed C2 step's results (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
 
@@ -440,6 +478,8 @@ def main():
     t_end = time.perf_counter()
     clocks = sampler.stop(t_begin, t_end)
     dev_ms, wall_ms, launches, res, tm = raw["dev_ms"], raw["wall_ms"], raw["launches"], raw["res"], raw["tm"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(res, args.dump_outputs)
     cells = tm.cells
     if use_dist:
         tt = torch.tensor([dev_ms, wall_ms], device="cuda", dtype=torch.float64)

@@ -79,10 +79,37 @@ def test_port_ops_rescore(oracle_mod):
     assert n >= 200
 
 
+def _stored_reference_cases(mode):
+    """The compiled reference's answers kept in tests/golden/fuzz_vectors.json for one mode variant."""
+    return [c for c in load_fuzz() if ("fitjump" if c["jump"] else c["mode"]) == mode]
+
+
+def _port_batch_vs_stored_reference(oracle_mod, mode):
+    cases = _stored_reference_cases(mode)
+    assert len(cases) >= 100
+    for c in cases:
+        s1, s2 = c["s1"].encode("latin-1"), c["s2"].encode("latin-1")
+        qb, qo, ql = pack_batch([s1])
+        tb, to, tl = pack_batch([s2])
+        sa = so = None
+        if c["jump"]:
+            sites = c["sites"] or []
+            sa = np.array(sites + [0], dtype=np.int32)
+            so = np.array([0, len(sites)], dtype=np.uint64)
+        p = oracle_mod.Params(c["m"], c["u"], c["o"], c["e"], c["j"], bool(c["jump"]))
+        a = oracle_mod.port_batch(c["mode"], p, qb, qo, ql, tb, to, tl, sa, so, threads=2)
+        assert int(a.score[0]) == c["score"], c
+        if c["mode"] != "edit":
+            assert a.aln(0) == (c["r1"].encode("latin-1"), c["r2"].encode("latin-1")), c
+
+
 @pytest.mark.parametrize("mode", ["global", "local", "fit", "fitjump", "overlap", "edit"])
 def test_port_matches_live_reference(oracle_mod, mode):
+    """The port's batch entry point against the reference: live on random batches where oracle/_ref was built,
+    otherwise against the reference's stored answers for this mode."""
     if not oracle_mod.have_ref():
-        pytest.skip("oracle/_ref not built (no /root/reference here)")
+        _port_batch_vs_stored_reference(oracle_mod, mode)
+        return
     rng = random.Random(hash(mode) & 0xffff)
     q, t, sites, site_off = [], [], [], [0]
     for _ in range(120):
@@ -181,9 +208,19 @@ def test_port_20kbp_vs_reference(oracle_mod, mode):
 def test_port_whitelist_mode_is_blacklist_of_the_complement(oracle_mod):
     """SURVEY.md 8(f) #3: the "intended" junction semantics (src/alignment.h:542-544: entering J only AT the listed
     target indices).  The reference cannot run it, but it is its own blacklist mode on the complement of the list --
-    which pins the port's whitelist restatement on the compiled reference."""
+    which pins the port's whitelist restatement on the compiled reference (live where oracle/_ref was built,
+    otherwise on the reference's stored fit -s answers, whose site lists are blacklists)."""
     if not oracle_mod.have_ref():
-        pytest.skip("oracle/_ref not built")
+        n_jump = 0
+        for c in _stored_reference_cases("fitjump"):
+            s1, s2 = c["s1"].encode("latin-1"), c["s2"].encode("latin-1")
+            black = set(c["sites"] or [])
+            white = [x for x in range(len(s2)) if x not in black]
+            w = oracle_mod.port_align("fit", s1, s2, oracle_mod.Params(c["m"], c["u"], c["o"], c["e"], c["j"], jump=2), white)
+            assert (w.score, w.r1, w.r2) == (c["score"], c["r1"].encode("latin-1"), c["r2"].encode("latin-1")), c
+            n_jump += w.ops.count(b"N") > 0
+        assert n_jump > 20
+        return
     rng = random.Random(8)
     n_jump = 0
     for k in range(120):
