@@ -30,7 +30,8 @@ EXPORTS = ["at_default_params", "at_strerror", "at_version", "at_create", "at_de
            "at_device_count", "at_launch_count", "at_align_gla", "at_align_local_affine",
            "at_align_fit_affine_jump", "at_align_overlap", "at_edit_dist", "at_batch_create",
            "at_batch_run", "at_batch_sizes", "at_batch_fetch", "at_batch_free", "at_batch_align",
-           "at_pack_2bit", "at_cigar_to_string", "at_plan_slices", "at_host_alloc", "at_host_free", "at_host_register", "at_host_unregister"]
+           "at_pack_2bit", "at_cigar_to_string", "at_plan_slices", "at_host_alloc", "at_host_free", "at_host_register", "at_host_unregister",
+           "at_batch_create_banded", "at_batch_align_banded"]
 
 
 class AtError(RuntimeError):
@@ -49,6 +50,18 @@ class _Input(C.Structure):
                 ("q", C.c_void_p), ("q_off", C.c_void_p), ("q_len", C.c_void_p),
                 ("t", C.c_void_p), ("t_off", C.c_void_p), ("t_len", C.c_void_p),
                 ("sites", C.c_void_p), ("site_off", C.c_void_p)]
+
+
+class _Band(C.Structure):
+    _fields_ = [("lo", C.c_void_p), ("hi", C.c_void_p)]
+
+
+def _band_arrays(band, n):
+    """band = (lo, hi): per-pair int32 diagonals d = j - i (include/aligntools_b200.h, at_band); None = unbanded."""
+    if band is None:
+        return None
+    lo, hi = (np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype=np.int32), (n,))) for x in band)
+    return lo, hi
 
 
 class _Output(C.Structure):
@@ -106,6 +119,10 @@ def load_library():
     lib.at_batch_free.argtypes = [C.c_void_p]
     lib.at_batch_align.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Params), C.POINTER(_Input), C.c_uint32,
                                    C.POINTER(_Output), C.POINTER(_Timing)]
+    lib.at_batch_create_banded.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Params), C.POINTER(_Input), C.POINTER(_Band),
+                                           C.c_uint32, C.POINTER(C.c_void_p)]
+    lib.at_batch_align_banded.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Params), C.POINTER(_Input), C.POINTER(_Band),
+                                          C.c_uint32, C.POINTER(_Output), C.POINTER(_Timing)]
     lib.at_pack_2bit.restype = C.c_int64
     lib.at_pack_2bit.argtypes = [C.c_char_p, C.c_uint64, C.c_void_p]
     lib.at_cigar_to_string.restype = C.c_int64
@@ -251,7 +268,9 @@ class Batch:
     """A batch resident on the device(s): create (H2D) -> run (kernels) -> fetch (D2H)."""
 
     def __init__(self, aligner, mode, opt, q, q_off, q_len, t, t_off, t_len, sites=None, site_off=None,
-                 out_flags=OUT_CIGAR | OUT_ALN, encoding=SEQ_BYTES):
+                 out_flags=OUT_CIGAR | OUT_ALN, encoding=SEQ_BYTES, band=None):
+        """band: None, or (lo, hi) -- per-pair int32 diagonals (d = j - i) of a banded overlap alignment
+        (at_batch_create_banded); a scalar applies to every pair."""
         self.al = aligner
         self.lib = aligner.lib
         self.n = int(len(q_len))
@@ -271,7 +290,13 @@ class Batch:
             assert sites.dtype == np.int32 and site_off.dtype == np.uint64
         self.h = C.c_void_p()
         prm = opt.c()
-        rc = self.lib.at_batch_create(aligner.h, self.mode, C.byref(prm), C.byref(inp), out_flags, C.byref(self.h))
+        self._band = _band_arrays(band, self.n)
+        if self._band is None:
+            rc = self.lib.at_batch_create(aligner.h, self.mode, C.byref(prm), C.byref(inp), out_flags, C.byref(self.h))
+        else:
+            bd = _Band(self._band[0].ctypes.data, self._band[1].ctypes.data)
+            rc = self.lib.at_batch_create_banded(aligner.h, self.mode, C.byref(prm), C.byref(inp), C.byref(bd), out_flags,
+                                                 C.byref(self.h))
         if rc:
             raise AtError(rc, aligner.last_error())
 
@@ -344,12 +369,13 @@ class Aligner:
 
     def align_arrays(self, mode, opt, q, q_off, q_len, t, t_off, t_len, sites=None, site_off=None,
                      out_flags=OUT_CIGAR, encoding=SEQ_BYTES, out: BatchResult = None,
-                     cigar_cap=None, aln_cap=None) -> BatchResult:
+                     cigar_cap=None, aln_cap=None, band=None) -> BatchResult:
         """One-shot at_batch_align (host arrays in, host arrays out; large batches are pipelined
         H2D / kernels / D2H inside the library).  `out` may be a BatchResult from a previous call
         whose buffers are reused; capacities default to the worst case (l1 + l2 per pair) for
         the alignment strings and for the CIGARs (32 ops per pair once that exceeds 64 Mi ops;
-        AT_E_NOSPACE tells when to pass a larger cigar_cap)."""
+        AT_E_NOSPACE tells when to pass a larger cigar_cap).  band: (lo, hi) per-pair diagonals of a banded overlap
+        alignment (at_batch_align_banded), or None."""
         md = _mode(mode)
         n = int(len(q_len))
         res = out if out is not None else BatchResult(n)
@@ -379,15 +405,20 @@ class Aligner:
                      site_off.ctypes.data if site_off is not None else None)
         prm = opt.c()
         tm = _Timing()
-        rc = self.lib.at_batch_align(self.h, md, C.byref(prm), C.byref(inp), out_flags, C.byref(o), C.byref(tm))
+        bnd = _band_arrays(band, n)
+        if bnd is None:
+            rc = self.lib.at_batch_align(self.h, md, C.byref(prm), C.byref(inp), out_flags, C.byref(o), C.byref(tm))
+        else:
+            bd = _Band(bnd[0].ctypes.data, bnd[1].ctypes.data)
+            rc = self.lib.at_batch_align_banded(self.h, md, C.byref(prm), C.byref(inp), C.byref(bd), out_flags, C.byref(o), C.byref(tm))
         if rc:
             raise AtError(rc, self.last_error())
         res.timing = Timing(tm.fill_ms, tm.traceback_ms, tm.device_ms, tm.cells, tm.launches, tm.ptr_bytes,
                             tm.fill_kernel_ms, tm.fill_kernel_cells, tm.fill_kernel_kind, tm.fill_kernel_rows, tm.fill_kernel_flags)
         return res
 
-    def align(self, mode, reads, targets, opt: Opt = None, sites=None, out_flags=OUT_CIGAR | OUT_ALN) -> BatchResult:
-        """Lists of bytes in, BatchResult out (create + run + fetch)."""
+    def align(self, mode, reads, targets, opt: Opt = None, sites=None, out_flags=OUT_CIGAR | OUT_ALN, band=None) -> BatchResult:
+        """Lists of bytes in, BatchResult out (create + run + fetch).  band: (lo, hi) diagonals, overlap only."""
         opt = opt or Opt()
         q, qo, ql = pack_seqs(reads)
         t, to, tl = pack_seqs(targets)
@@ -398,7 +429,7 @@ class Aligner:
             sa = np.array(flat + [0], dtype=np.int32)
             so = np.zeros(len(reads) + 1, np.uint64)
             np.cumsum([len(s or []) for s in sites], out=so[1:])
-        b = Batch(self, mode, opt, q, qo, ql, t, to, tl, sites=sa, site_off=so, out_flags=out_flags)
+        b = Batch(self, mode, opt, q, qo, ql, t, to, tl, sites=sa, site_off=so, out_flags=out_flags, band=band)
         try:
             tm = b.run()
             res = b.fetch()

@@ -211,6 +211,9 @@ struct Shard {
 	bool prof = false; uint32_t syms = 0;      // query-profile variant of K1: the targets use <= 4 distinct bytes
 	bool bits = false;                         // bit-parallel edit distance: `-u 1` and reads of <= 8 distinct bytes
 	bool twobit = false;                       // the sequences stay 2-bit packed in HBM (AT_SEQ_2BIT input consumed directly by K1 / K2 / K3)
+	bool banded = false;                       // overlap with a per-pair band: h_band / d_band hold it clipped (at_band.h)
+	std::vector<int2> h_band;
+	DevBuf<int2> d_band;
 	std::vector<uint64_t> h_t_rel;             // twobit + jump: device offsets of the packed targets (the jump masks copy their alignment)
 	DevBuf<uint64_t> d_j_off;                  // twobit + jump: per-pair offsets into d_jmask (byte-encoded targets use d_t_off)
 	BufCache cache;                            // released device blocks, reused by this shard's next allocations
@@ -363,7 +366,7 @@ static void free_shard(Shard &s)
 	s.d_beg_j.release(); s.d_n_ops.release(); s.d_n_cols.release(); s.d_counter.release();
 	s.ws_cigar.release(); s.ws_aln1.release(); s.ws_aln2.release();
 	s.d_score.release(); s.d_sites.release(); s.d_ptr.release(); s.d_scratch.release(); s.d_bnd.release(); s.d_scan_tmp.release();
-	s.d_prog.release(); s.d_chain.release(); s.d_symmap.release(); s.d_symset.release();
+	s.d_prog.release(); s.d_chain.release(); s.d_symmap.release(); s.d_symset.release(); s.d_band.release();
 	release_chunks(s);
 	for (auto &e : s.ev) if (e) cudaEventDestroy(e);
 	for (auto &e : s.evk) if (e) cudaEventDestroy(e);
@@ -504,16 +507,16 @@ static void order_wave_tasks(std::vector<WaveTask> &t)
 		for (size_t x = 0; x < n; ++x) t[x].prev = (uint32_t)(t[x].stripe ? x - 1 : x);
 		return;
 	}
-	struct Run { uint32_t pair, n, last; };
+	struct Run { uint32_t pair, n, last; size_t x0; };      // x0: the pair's first task in `t` (its stripes need not start at 0: banded pairs)
 	std::vector<Run> active;
-	for (size_t x = 0; x < n;) { size_t y = x; while (y < n && t[y].pair == t[x].pair) ++y; active.push_back(Run{t[x].pair, (uint32_t)(y - x), 0}); x = y; }
+	for (size_t x = 0; x < n;) { size_t y = x; while (y < n && t[y].pair == t[x].pair) ++y; active.push_back(Run{t[x].pair, (uint32_t)(y - x), 0, x}); x = y; }
 	std::vector<WaveTask> out;
 	out.reserve(n);
 	for (uint32_t s = 0; !active.empty(); ++s) {
 		size_t keep = 0;
 		for (Run &r : active) {
 			const uint32_t idx = (uint32_t)out.size();
-			out.push_back(WaveTask{r.pair, s, s ? r.last : idx, 0});
+			out.push_back(WaveTask{r.pair, t[r.x0 + s].stripe, s ? r.last : idx, 0});
 			r.last = idx;
 			if (s + 1 < r.n) active[keep++] = r;
 		}
@@ -522,7 +525,8 @@ static void order_wave_tasks(std::vector<WaveTask> &t)
 	t.swap(out);
 }
 
-static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in)
+// `band` (NULL: unbanded): the caller's band arrays, indexed like `in` (band->lo[s.p0 + k] is the shard's pair k)
+static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at_band *band)
 {
 	at_handle *h = b->h;
 	CU(h, cudaSetDevice(s.dev->id));
@@ -568,6 +572,22 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in)
 	s.d_q2.release(); s.d_t2.release();
 	mark("upload");
 	const bool jump = b->mode == AT_FIT && b->prm.jump;
+	s.banded = band != nullptr;
+	if (s.banded) {
+		s.h_band.resize(n);
+		for (uint32_t k = 0; k < n; ++k) {
+			int32_t elo, ehi;
+			band_clip(in->q_len[s.p0 + k], in->t_len[s.p0 + k], band->lo[s.p0 + k], band->hi[s.p0 + k], elo, ehi);
+			s.h_band[k] = make_int2(elo, ehi);
+		}
+		CU(h, s.d_band.alloc(n));
+		CU(h, cudaMemcpyAsync(s.d_band.p, s.h_band.data(), n * sizeof(int2), cudaMemcpyHostToDevice, st));      // staged before the set-up's synchronisation
+	}
+	// banded pairs: the in-band cells, the pointer words of their stripe windows (at_band.h)
+	auto pair_cells = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t { return s.banded ? band_cells(l1, l2, s.h_band[k].x, s.h_band[k].y) : (uint64_t)l1 * l2; };
+	auto pair_ptr_words = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t {
+		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass_of(l1)) : ptr_words_of(b->mode, jump, l1, l2);
+	};
 	if ((rc = choose_variants(b, s, in, q_span))) return rc;
 	if (jump && (rc = build_jump_mask(b, s, in))) return rc;
 	mark("alphabet+jmask");
@@ -583,7 +603,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in)
 		for (uint32_t k = 0; k < n; ++k) {
 			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
 			s.h_rclass[k] = (uint8_t)rclass_of(l1);
-			s.cells += (uint64_t)l1 * l2;
+			s.cells += pair_cells(k, l1, l2);
 		}
 	}
 	CU(h, s.d_score.alloc(n)); CU(h, s.d_end_i.alloc(n)); CU(h, s.d_end_j.alloc(n)); CU(h, s.d_end_state.alloc(n));
@@ -603,7 +623,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in)
 	uint64_t need_words = 0;
 	auto pair_words = [&](uint32_t k) -> uint64_t {
 		const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-		return b->traceback ? ptr_words_of(b->mode, jump, l1, l2) + 64ull * rclass_of(l1) : 0;   // + rounding slack of the packed layout
+		return b->traceback ? pair_ptr_words(k, l1, l2) + 64ull * rclass_of(l1) : 0;   // + rounding slack of the packed layout
 	};
 	if (uniform) need_words = (uint64_t)n * pair_words(0);
 	else for (uint32_t k = 0; k < n; ++k) need_words += pair_words(k);
@@ -754,9 +774,16 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in)
 			const uint32_t rows = s.bits ? 1024u * r : 32u * r;
 			Launch &lw = s.bits ? lbit[r] : lwv[r];
 			const uint32_t n_stripes = (l1 + rows - 1) / rows;
-			for (uint32_t st2 = 0; st2 < n_stripes; ++st2) lw.h_tasks.push_back(WaveTask{k, st2, 0, 0});
-			lw.cells += cells_of(k);
-			if (n_stripes > 1) { c.h_bnd_off[k - c.k0] = c.bnd_elems; c.bnd_elems += 2ull * ((l2 + 4u) & ~3u); }
+			uint32_t queued = 0;
+			for (uint32_t st2 = 0; st2 < n_stripes; ++st2) {
+				// banded: only stripes with a window run; the last stripe always does (it writes the end cell)
+				BandWin w;
+				if (s.banded && st2 + 1 < n_stripes && !band_stripe(l1, l2, s.h_band[k].x, s.h_band[k].y, rows, st2, w)) continue;
+				lw.h_tasks.push_back(WaveTask{k, st2, 0, 0});
+				++queued;
+			}
+			lw.cells += s.banded ? pair_cells(k, l1, l2) : cells_of(k);
+			if (queued > 1) { c.h_bnd_off[k - c.k0] = c.bnd_elems; c.bnd_elems += 2ull * ((l2 + 4u) & ~3u); }
 		}
 		for (int r = 1; r <= MAXR; ++r) {
 			if (!l32[r].h_jobs.empty()) { l32[r].kind = LK_INT32; l32[r].r = r; c.launches.push_back(std::move(l32[r])); }
@@ -788,7 +815,14 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in)
 				} else if (l.kind == LK_INT32) {
 					for (const FillJob &jb : l.h_jobs) { const uint32_t k = jb.a; c.h_ptr_off[k - c.k0] = words; words += ptr_words_of(b->mode, jump, in->q_len[s.p0 + k], in->t_len[s.p0 + k]); }
 				} else {
-					for (const WaveTask &tk : l.h_tasks) if (tk.stripe == 0) { const uint32_t k = tk.pair; c.h_ptr_off[k - c.k0] = words; words += ptr_words_of(b->mode, jump, in->q_len[s.p0 + k], in->t_len[s.p0 + k]); }
+					// a pair's block goes where its first task is queued (stripe 0 unless the band leaves stripe 0 out)
+					std::vector<uint8_t> placed(nc, 0);
+					for (const WaveTask &tk : l.h_tasks) {
+						const uint32_t k = tk.pair;
+						if (placed[k - c.k0]) continue;
+						placed[k - c.k0] = 1;
+						c.h_ptr_off[k - c.k0] = words; words += pair_ptr_words(k, in->q_len[s.p0 + k], in->t_len[s.p0 + k]);
+					}
 				}
 			}
 		}
@@ -975,12 +1009,30 @@ static at_batch *new_batch(at_handle *h, int mode, const at_params *p, uint32_t 
 	return b;
 }
 
+// a band is for AT_OVERLAP only, with both arrays and lo[p] <= hi[p] for every pair
+static int validate_band(at_handle *h, int mode, const at_batch_input *in, const at_band *band)
+{
+	if (!band) return AT_OK;
+	if (mode != AT_OVERLAP) { set_err(h, "band: only overlap alignment takes a band (mode %d)", mode); return AT_E_ARG; }
+	if (!band->lo || !band->hi) { set_err(h, "band: %s is NULL", band->lo ? "hi" : "lo"); return AT_E_ARG; }
+	for (uint64_t k = 0; k < in->n_pairs; ++k)
+		if (band->lo[k] > band->hi[k]) { set_err(h, "band: lo > hi at pair %llu (%d > %d)", (unsigned long long)k, band->lo[k], band->hi[k]); return AT_E_ARG; }
+	return AT_OK;
+}
+
 extern "C" int at_batch_create(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
                                uint32_t out_flags, at_batch **out)
+{
+	return at_batch_create_banded(h, mode, p, in, nullptr, out_flags, out);
+}
+
+extern "C" int at_batch_create_banded(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
+                                      const at_band *band, uint32_t out_flags, at_batch **out)
 {
 	if (!h || !p || !in || !out) return AT_E_ARG;
 	*out = nullptr;
 	if (int rc = validate_batch(h, mode, p, in)) return rc;
+	if (int rc = validate_band(h, mode, in, band)) return rc;
 	at_batch *b = new_batch(h, mode, p, out_flags, in->n_pairs);
 	// contiguous slices balanced by cells
 	const size_t nd = h->devs.size();
@@ -992,7 +1044,7 @@ extern "C" int at_batch_create(at_handle *h, int mode, const at_params *p, const
 		Shard &s = b->shards[d];
 		s.dev = &h->devs[d]; s.stream = s.dev->stream; s.p0 = cut[d]; s.p1 = cut[d + 1]; s.out_base = s.p0; s.n = (uint32_t)(s.p1 - s.p0);
 	}
-	auto work = [&](size_t d) { Shard &s = b->shards[d]; s.rc = s.n ? setup_shard(b, s, in) : AT_OK; };
+	auto work = [&](size_t d) { Shard &s = b->shards[d]; s.rc = s.n ? setup_shard(b, s, in, band) : AT_OK; };
 	if (nd == 1) work(0);
 	else { for (size_t d = 0; d < nd; ++d) th.emplace_back(work, d); for (auto &t : th) t.join(); }
 	for (auto &s : b->shards) if (s.rc) { int rc = s.rc; at_batch_free(b); return rc; }
@@ -1028,14 +1080,16 @@ template <bool PROF> static fill2_fn affine_kernel_r(int kind, int R)
 	}
 }
 static fill2_fn affine_kernel(int kind, int R, bool prof) { return prof ? affine_kernel_r<true>(kind, R) : affine_kernel_r<false>(kind, R); }
-template <int MODE, bool PROF> static wave_fn wave_linear_fn(int R)
+template <int MODE, bool PROF, bool BANDED = false> static wave_fn wave_linear_fn(int R)
 {
 	switch (R) {
-	case 1: return at_wave_linear<MODE, 1, PROF>; case 2: return at_wave_linear<MODE, 2, PROF>; case 3: return at_wave_linear<MODE, 3, PROF>;
-	case 4: return at_wave_linear<MODE, 4, PROF>; case 5: return at_wave_linear<MODE, 5, PROF>; case 6: return at_wave_linear<MODE, 6, PROF>;
-	case 7: return at_wave_linear<MODE, 7, PROF>; default: return at_wave_linear<MODE, 8, PROF>;
+	case 1: return at_wave_linear<MODE, 1, PROF, BANDED>; case 2: return at_wave_linear<MODE, 2, PROF, BANDED>; case 3: return at_wave_linear<MODE, 3, PROF, BANDED>;
+	case 4: return at_wave_linear<MODE, 4, PROF, BANDED>; case 5: return at_wave_linear<MODE, 5, PROF, BANDED>; case 6: return at_wave_linear<MODE, 6, PROF, BANDED>;
+	case 7: return at_wave_linear<MODE, 7, PROF, BANDED>; default: return at_wave_linear<MODE, 8, PROF, BANDED>;
 	}
 }
+// banded overlap (validate_band admits a band with AT_OVERLAP only)
+static wave_fn wave_banded_kernel(int R, bool prof) { return prof ? wave_linear_fn<MODE_OVERLAP, true, true>(R) : wave_linear_fn<MODE_OVERLAP, false, true>(R); }
 static wave_fn bits_kernel(int R) { return R == 1 ? at_wave_edit_bits<1> : (R == 2 ? at_wave_edit_bits<2> : at_wave_edit_bits<4>); }
 static wave_fn wave_kernel(int mode, bool jump, int R, bool prof)
 {
@@ -1085,7 +1139,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 		if (first) { CU(h, cudaEventRecord(e_first, st)); first = false; }
 		for (size_t li = 0; li < c.launches.size(); ++li) {
 			Launch &l = c.launches[li];
-			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r) : l.kind == LK_WAVE ? (const void *)wave_kernel(b->mode, jump, l.r, s.prof)
+			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r) : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(l.r, s.prof) : (const void *)wave_kernel(b->mode, jump, l.r, s.prof))
 			                                   : (const void *)affine_kernel(l.kind == LK_PACKED ? (b->mode == AT_LOCAL ? 4 : b->mode == AT_GLOBAL ? 5 : 6) : (b->mode == AT_FIT ? (jump ? 3 : 2) : b->mode), l.r, s.prof);
 			const int warps = l.kind >= LK_WAVE ? AT_WAVE_WARPS : AT_FILL_WARPS;
 			const size_t dyn_smem = l.kind >= LK_WAVE ? 0 : fill_smem_bytes(l.r, l.kind == LK_PACKED, s.prof);
@@ -1113,6 +1167,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 				wa.m = b->prm.m; wa.u = b->prm.u; wa.o = b->prm.o; wa.e = b->prm.e; wa.jp = b->prm.j;
 				wa.want_ptr = b->traceback ? 1 : 0;
 				wa.k_and = cell_k_and<false>(); wa.k_or = cell_k_or<false>();
+				wa.band = s.banded ? s.d_band.p : nullptr;
 				void *kargs[] = {(void *)&wa};
 				CU(h, cudaLaunchKernel(fn, dim3(blocks), dim3(32 * warps), kargs, 0, st));
 			} else {
@@ -1151,11 +1206,13 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 			ta.scratch = s.d_scratch.p; ta.scratch_off = c.d_scratch_off.p;
 			ta.cigar = nullptr; ta.aln1 = nullptr; ta.aln2 = nullptr;
 			ta.mode = b->mode; ta.jump = jump ? 1 : 0; ta.twobit = s.twobit ? 1 : 0;
+			ta.band = s.banded ? s.d_band.p : nullptr;
 			// few long walks: one walker per warp, prefetching ahead; with many walks, or short ones (a few hundred
 			// steps: nothing to prefetch far ahead of), the chase is throughput-bound and the prefetches only add traffic
 			ta.lookahead = nc < 32768u && c.scratch_words / nc >= 2048 ? 1 : 0;
 			const int walk_blocks = ta.lookahead ? (int)(((uint64_t)nc * 32 + 127) / 128) : (int)((nc + 127) / 128);   // one walker per warp | per thread
-			if (s.workspace && tb_overlap) at_traceback_walk<true><<<walk_blocks, 128, 0, st>>>(ta);
+			if (s.banded) at_traceback_walk<false, true><<<walk_blocks, 128, 0, st>>>(ta);
+			else if (s.workspace && tb_overlap) at_traceback_walk<true><<<walk_blocks, 128, 0, st>>>(ta);
 			else at_traceback_walk<false><<<walk_blocks, 128, 0, st>>>(ta);
 			CU(h, cudaGetLastError());
 			s.launches++;

@@ -68,6 +68,7 @@ struct WaveArgs {
 	uint32_t        k_and, k_or;   // affine kernel: cell_k_and / cell_k_or (at_cell.cuh: constants that must stay in registers)
 	int             twobit;  // q / t hold 2-bit codes (AT_SEQ_2BIT resident: four symbols per byte, A C G T = 0..3, byte-aligned records)
 	uint32_t        start_lag;   // a stripe starts once the stripe above it has published this many columns (0: as soon as it can)
+	const int2     *band;        // at_wave_linear<.., BANDED>: [pair] clipped band (lo, hi) on j - i (at_band.h)
 };
 
 // ---- TMA (bulk async copy) + mbarrier + release/acquire helpers ----
@@ -496,7 +497,15 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 // multiply-add with a 0/1 lane mask, not a branch.
 // (no minimum-blocks hint: ptxas's own choice, 72-80 registers = 6 CTAs per SM, measured best on C4 -- 24.6 ms against
 // 26.3 ms when held to 64 registers for 8 CTAs and 27.8 ms with a hint of 1; profiles/ab_wave_linear_occupancy_r02.txt)
-template <int MODE, int R, bool PROF>
+//
+// BANDED (overlap only): the pair's band (at_band.h) limits every stripe to its column window.  The steps run from the
+// window's t0 to (c1 + 31) | 31; 16-step blocks whose cells may leave the band force those cells to -inf (the band
+// test is one unsigned compare per cell), blocks wholly inside the band run the plain body.  Target tiles keep their
+// absolute numbering (tile c = ring bytes 256 c ..), only those the window reads are staged.  The stripe above is the
+// predecessor when it has a window; otherwise the row above is -inf, as row 0 is.  Pointer words are stored relative to
+// t0 at the stripe's offset in the pair's block.  A queued stripe without a window is the pair's last one: it only
+// writes the end cell M[l1][0] = 0.
+template <int MODE, int R, bool PROF, bool BANDED = false>
 __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveArgs a)
 {
 	constexpr int RPP = 32 * R;
@@ -538,12 +547,31 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 		const uint8_t *tbase16 = tbase - sh16;
 		const uint32_t sh = twobit ? 4u * sh16 : sh16;                        // ring position of target index 0
 		const uint32_t tile_wait = twobit ? 192u : 224u;                      // step (mod 256) at which the next tile must have landed: lane 0 is up to sh + 1 columns ahead of the step counter
-		const uint32_t n_tiles = (l2 + sh + 255u) >> 8;
+		uint32_t n_tiles = (l2 + sh + 255u) >> 8;
 		uint32_t *__restrict__ ptr = OV ? a.ptr + a.ptr_off[p - a.pair_base] : nullptr;
 		const uint32_t G = (((l2 + 31u) | 15u) >> 4) + 1;                 // pointer-block geometry shared with K3
-		const uint32_t t_last = (l2 + 31u) | 31u;
+		uint32_t t_last = (l2 + 31u) | 31u;
 		const uint32_t n_stripes = (l1 + RPP - 1) / RPP;
 		const bool last_stripe = stripe + 1 == n_stripes;
+		// banded: this stripe's window (bw), the one above (pw), whether the stripes above / below take part
+		BandWin bw = {1u, l2, 0u, G}, bwp = bw, bwn = bw;
+		int32_t elo = 0, ehi = 0;
+		bool has_prev = stripe > 0, has_next = !last_stripe;
+		if constexpr (BANDED) {
+			const int2 bd = a.band[p];
+			elo = bd.x; ehi = bd.y;
+			if (!band_stripe(l1, l2, elo, ehi, RPP, stripe, bw)) {
+				if (lane == 0) { a.score[p] = 0; a.end_i[p] = l1; a.end_j[p] = 0; a.end_state[p] = ST_MID; }      // M[l1][0] (:938)
+				__syncwarp();
+				continue;
+			}
+			has_prev = stripe > 0 && band_stripe(l1, l2, elo, ehi, RPP, stripe - 1u, bwp);
+			has_next = !last_stripe && band_stripe(l1, l2, elo, ehi, RPP, stripe + 1u, bwn);
+			t_last = band_t_last(bw);
+			n_tiles = min(n_tiles, ((bw.c1 - 1u + sh) >> 8) + 1u);         // tiles the window reads
+			if (want_ptr) ptr += band_stripe_off(l1, l2, elo, ehi, RPP, stripe);
+		}
+		const uint32_t tile0 = bw.t0 >> 8;                                 // first tile the stripe reads (0 unbanded)
 		const uint32_t slab = (l2 + 4u) & ~3u;
 		// boundary hand-off without fences: one 64-bit word per column = (stripe + 1) << 32 | value; the consumer
 		// validates the tag of every word it loads (the slabs are zeroed by the host before each run)
@@ -553,12 +581,12 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 		const uint64_t tag_out = (uint64_t)(stripe + 1u) << 32;
 		const uint32_t tag_in = stripe;                                   // the predecessor's (stripe - 1) + 1
 		const uint32_t row0 = stripe * RPP + lane * R;
-		const bool feed = lane == 0 && stripe > 0;                        // this lane reads the boundary ring
-		const bool park = lane == 31 && !last_stripe;                     // this lane parks its last row for the next stripe
+		const bool feed = lane == 0 && has_prev;                          // this lane reads the boundary ring
+		const bool park = lane == 31 && has_next;                         // this lane parks its last row for the next stripe
 
 		__syncwarp();
-		if (n_tiles > 0) ring_issue<false>(sm.rg, tbase16, nullptr, 0, lane, twobit);
-		if (n_tiles > 1) ring_issue<false>(sm.rg, tbase16, nullptr, 1, lane, twobit);
+		if (n_tiles > tile0) ring_issue<false>(sm.rg, tbase16, nullptr, tile0, lane, twobit);
+		if (n_tiles > tile0 + 1u) ring_issue<false>(sm.rg, tbase16, nullptr, tile0 + 1u, lane, twobit);
 
 		// carried value: overlap a = 4*M + 4*o (LinRow keeps a + 2), edit M.  Column 0: M[i][0] = 0 (:938) | i (:301)
 		uint32_t ac[R];
@@ -589,21 +617,30 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 		// what lane 0 adds instead of a neighbour's row (zero in every other lane): matrix row 0 in the first stripe
 		// (overlap: -inf, :937; edit: j, :302), the boundary ring's element otherwise (loaded per step by lane 0 alone)
 		int bq = 0, b0E = 0;
-		if (lane == 0 && stripe == 0) { if (OV) bq = AT_NEGL; else b0E = 1; }
+		if (lane == 0 && !has_prev) { if (OV) bq = AT_NEGL; else b0E = 1; }
 
 		uint64_t pre = 0;
-		if (stripe) {
+		if (has_prev) {
 			// start lag: three hand-off blocks behind the predecessor, so that blocks requested one block ahead are valid on arrival
-			if (lane == 0) { const uint32_t c = min(l2, max(96u, a.start_lag)); while ((uint32_t)(ld_relaxed_u64(bnd_in + c) >> 32) != tag_in) __nanosleep(200); }
+			if (lane == 0) {
+				const uint32_t c = BANDED ? band_first_wait(bwp, bw.t0, a.start_lag) : min(l2, max(96u, a.start_lag));
+				while ((uint32_t)(ld_relaxed_u64(bnd_in + c) >> 32) != tag_in) __nanosleep(200);
+			}
 			__syncwarp();
-			if ((uint32_t)lane <= l2) pre = ld_relaxed_u64(bnd_in + lane);
+			if (bw.t0 + (uint32_t)lane <= l2) pre = ld_relaxed_u64(bnd_in + bw.t0 + lane);
 		}
-		mbar_wait(&sm.rg.bar[0], ring_par & 1u); ring_par ^= 1u;
-		if (twobit) ring_expand(sm.rg, 0, lane);
+		mbar_wait(&sm.rg.bar[tile0 & 1u], (ring_par >> (tile0 & 1u)) & 1u); ring_par ^= 1u << (tile0 & 1u);
+		if (twobit) ring_expand(sm.rg, tile0, lane);
+		if (BANDED && (bw.t0 & 255u) > tile_wait && tile0 + 1u < n_tiles) {      // the window starts past the point where the next tile is awaited
+			const uint32_t c = tile0 + 1u;
+			mbar_wait(&sm.rg.bar[c & 1u], (ring_par >> (c & 1u)) & 1u); ring_par ^= 1u << (c & 1u); if (twobit) ring_expand(sm.rg, c, lane);
+		}
 
 		// `cap`: std::true_type in the pair's last stripe (only there can a lane hold the pair's last row)
-		auto step = [&](const uint32_t t, const bool checked, auto cap) {
+		// `msk`: std::true_type where cells of the step may lie outside the pair's band (BANDED only): they become -inf
+		auto step = [&](const uint32_t t, const bool checked, auto cap, auto msk) {
 			constexpr bool CAP = decltype(cap)::value;
+			constexpr bool MSK = decltype(msk)::value;
 			const int j = (int)t - lane;
 			if (feed) bq = sm.cring[t & 63u];
 			int rV = __shfl_up_sync(0xffffffffu, sV, 1) * nz + bq;
@@ -630,6 +667,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 						int dn;
 						v = lin_update(stl[r], D, sub, Vup, gap, dn);
 						D = dn;
+						if (MSK && (uint32_t)(j - (int)row0 - 1 - r - elo) > (uint32_t)(ehi - elo)) { v = AT_NEGL; stl[r].a2 = AT_NEGL + 2; }   // d = j - i out of band
 					} else {
 						const int diag = D + sub;
 						D = Vl[r];
@@ -651,24 +689,27 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 			}
 		};
 
-		for (uint32_t tb = 0; tb <= t_last; tb += 16) {
+		// columns this stripe publishes, and those it takes from the stripe above (banded: their windows; the rest is -inf)
+		const int pub0 = BANDED ? (int)bw.c0 : 1, pub1 = BANDED ? (int)bw.c1 : (int)l2;
+		const uint32_t in0 = BANDED ? bwp.c0 : 1u, in1 = BANDED ? bwp.c1 : l2;
+		for (uint32_t tb = bw.t0; tb <= t_last; tb += 16) {
 			if ((tb & 31u) == 0) {
 				__syncwarp();
-				if (!last_stripe && tb >= 64u) {
+				if (has_next && tb >= 64u) {
 					const int cidx = (int)tb - 63 + lane;
-					if (cidx >= 1 && cidx <= (int)l2) st_relaxed_u64(bnd_out + cidx, tag_out | (uint32_t)sm.stage[(uint32_t)cidx & 63u]);
+					if (cidx >= pub0 && cidx <= pub1) st_relaxed_u64(bnd_out + cidx, tag_out | (uint32_t)sm.stage[(uint32_t)cidx & 63u]);
 				}
-				if (stripe) {
+				if (has_prev) {
 					const uint32_t col = tb + lane;                       // `pre` was requested a block ago: make sure it is the predecessor's
-					if (col >= 1u && col <= l2)
+					if (col >= in0 && col <= in1)
 						while ((uint32_t)(pre >> 32) != tag_in) { __nanosleep(40); pre = ld_relaxed_u64(bnd_in + col); }
-					sm.cring[col & 63u] = (int)(uint32_t)pre;
+					sm.cring[col & 63u] = BANDED && (col < in0 || col > in1) ? AT_NEGL : (int)(uint32_t)pre;
 					const uint32_t nxt = col + 32u;
 					if (nxt <= l2) pre = ld_relaxed_u64(bnd_in + nxt);
 					__syncwarp();
 				}
 			}
-			if ((tb & 255u) == 32u && tb > 32u) {
+			if ((tb & 255u) == 32u && (BANDED ? (tb >> 8) > tile0 : tb > 32u)) {
 				const uint32_t c = (tb >> 8) + 1u;
 				__syncwarp();
 				if (c < n_tiles) ring_issue<false>(sm.rg, tbase16, nullptr, c, lane, twobit);
@@ -677,19 +718,35 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 				const uint32_t c = (tb >> 8) + 1u;
 				if (c < n_tiles) { mbar_wait(&sm.rg.bar[c & 1u], (ring_par >> (c & 1u)) & 1u); ring_par ^= 1u << (c & 1u); if (twobit) ring_expand(sm.rg, c, lane); }
 			}
-			if (tb >= 32u && tb + 15u <= l2) {
+			// banded: d = j - i of the block's cells spans [tb - row(stripe) - RPP - 31, tb + 14 - row(stripe)]
+			const bool inner = !BANDED || ((int64_t)tb - (int64_t)stripe * RPP - RPP - 31 >= elo && (int64_t)tb + 14 - (int64_t)stripe * RPP <= ehi);
+			if (tb >= 32u && tb + 15u <= l2 && inner) {
 				if (last_stripe) {
 #pragma unroll UNR
-					for (uint32_t k = 0; k < 16; ++k) step(tb + k, false, std::true_type());
+					for (uint32_t k = 0; k < 16; ++k) step(tb + k, false, std::true_type(), std::false_type());
 				} else {
 #pragma unroll UNR
-					for (uint32_t k = 0; k < 16; ++k) step(tb + k, false, std::false_type());
+					for (uint32_t k = 0; k < 16; ++k) step(tb + k, false, std::false_type(), std::false_type());
+				}
+			} else if (BANDED && tb >= 32u && tb + 15u <= l2) {
+				if (last_stripe) {
+#pragma unroll UNR
+					for (uint32_t k = 0; k < 16; ++k) step(tb + k, false, std::true_type(), std::true_type());
+				} else {
+#pragma unroll UNR
+					for (uint32_t k = 0; k < 16; ++k) step(tb + k, false, std::false_type(), std::true_type());
 				}
 			} else {
 #pragma unroll 1
-				for (uint32_t k = 0; k < 16; ++k) step(tb + k, true, std::true_type());
+				for (uint32_t k = 0; k < 16; ++k) step(tb + k, true, std::true_type(), std::integral_constant<bool, BANDED>());
 			}
-			if (want_ptr && (tb >> 4) < G) {
+			if constexpr (BANDED) {
+				if (want_ptr && ((tb - bw.t0) >> 4) < bw.groups) {
+					uint32_t *w = ptr + ((size_t)((tb - bw.t0) >> 4) * 32 + lane) * R;
+#pragma unroll
+					for (int r = 0; r < R; ++r) w[r] = lin_word(stl[r].x);
+				}
+			} else if (want_ptr && (tb >> 4) < G) {
 				uint32_t *w = ptr + ((size_t)(stripe * G + (tb >> 4)) * 32 + lane) * R;
 #pragma unroll
 				for (int r = 0; r < R; ++r) w[r] = lin_word(stl[r].x);
@@ -697,9 +754,9 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 		}
 		__syncwarp();
 
-		if (!last_stripe) {
+		if (has_next) {
 			const int cidx = (int)t_last - 62 + lane;
-			if (cidx >= 1 && cidx <= (int)l2) st_relaxed_u64(bnd_out + cidx, tag_out | (uint32_t)sm.stage[(uint32_t)cidx & 63u]);
+			if (cidx >= pub0 && cidx <= pub1) st_relaxed_u64(bnd_out + cidx, tag_out | (uint32_t)sm.stage[(uint32_t)cidx & 63u]);
 		} else if (cap_r >= 0) {
 			if (OV) { a.score[p] = (capV - gap) / S; a.end_i[p] = l1; a.end_j[p] = capJ; a.end_state[p] = ST_MID; }
 			else { a.score[p] = capV; a.end_i[p] = l1; a.end_j[p] = l2; a.end_state[p] = ST_MID; }

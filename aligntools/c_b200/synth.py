@@ -133,11 +133,12 @@ def _mutate(rng, s, sub, ins, dele):
     return out
 
 
-def config4_overlap(n_pairs=32, lo=10000, hi=20000, stream=0):
+def config4_overlap(n_pairs=32, lo=10000, hi=20000, stream=0, with_diag=False):
     """C4: overlap (defaults m=1 u=-2 o=-5): s2's prefix is a mutated (5 % sub, 2.5 % ins,
-    2.5 % del) copy of a suffix of s1."""
+    2.5 % del) copy of a suffix of s1.  with_diag: the result also carries `diag`, each pair's true start
+    diagonal -(l1 - ov) (int32; what a seed chain would give a banded overlap alignment)."""
     rng = _rng(4, stream)
-    reads, tgts = [], []
+    reads, tgts, diag = [], [], []
     for _ in range(n_pairs):
         l1 = int(rng.integers(lo, hi + 1))
         l2 = int(rng.integers(lo, hi + 1))
@@ -147,10 +148,14 @@ def config4_overlap(n_pairs=32, lo=10000, hi=20000, stream=0):
         s2 = np.concatenate([pre, rng.integers(0, 4, size=max(0, l2 - pre.size), dtype=np.uint8)])
         reads.append(ACGT[s1])
         tgts.append(ACGT[s2])
+        diag.append(-(l1 - ov))
     q, qo, ql = _ragged_batch(reads)
     t, to, tl = _ragged_batch(tgts)
-    return dict(mode="overlap", params=dict(m=1, u=-2, o=-5, e=-1, j=-10, jump=False),
-                q=q, q_off=qo, q_len=ql, t=t, t_off=to, t_len=tl, sites=None, site_off=None)
+    out = dict(mode="overlap", params=dict(m=1, u=-2, o=-5, e=-1, j=-10, jump=False),
+               q=q, q_off=qo, q_len=ql, t=t, t_off=to, t_len=tl, sites=None, site_off=None)
+    if with_diag:
+        out["diag"] = np.array(diag, dtype=np.int32)
+    return out
 
 
 def config5_edit(n_pairs=8, length=100000, stream=0):

@@ -160,7 +160,7 @@ typedef struct at_timing {
 	double   fill_ms;        /* device time in the fill kernels (CUDA events), max over devices      */
 	double   traceback_ms;   /* device time in the traceback kernels, max over devices               */
 	double   device_ms;      /* first kernel start -> last kernel end, max over devices              */
-	uint64_t cells;          /* sum of l1*l2 over all pairs                                          */
+	uint64_t cells;          /* sum of l1*l2 over all pairs; banded batches: the in-band cells exactly */
 	uint64_t launches;       /* kernels launched by this run                                         */
 	uint64_t ptr_bytes;      /* traceback-pointer bytes written to HBM                               */
 	double   fill_kernel_ms; /* average duration of ONE launch of the dominant fill kernel           */
@@ -196,6 +196,26 @@ void at_batch_free(at_batch *b);
 /* One-shot: create + run + fetch + free (host buffers in, host buffers out). */
 int  at_batch_align(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
                     uint32_t out_flags, at_batch_output *out, at_timing *timing);
+
+/* Banded overlap alignment: pair p only fills the cells (i, j) of its band lo[p] <= j - i <= hi[p] (diagonals of the DP
+ * matrix, 1 <= i <= l1, 1 <= j <= l2; the band is clipped to [1 - l1, l2 - 1] in 64 bits, and may be empty).  Cells
+ * outside it are -inf; row 0 stays -inf and M[i][0] = 0, ties, the end search (last row, columns 0 .. l2-1) and the
+ * traceback are the reference's.  An empty band gives score 0, end cell (l1, 0) and an empty alignment.
+ * Identity: when every cell of the unbanded traceback path (its end cell included, its column-0 start excluded) lies
+ * in the band, the banded result equals the unbanded one in every field -- a full band gives exactly at_batch_align's.
+ * Only K2's stripe windows are filled and only their pointers are stored, so a caller that knows where the overlap lies
+ * (seed or minimizer chains) pays for the band, not for l1 x l2.  at_timing.cells counts the in-band cells; ptr_bytes is
+ * what the banded pointer blocks took.  band == NULL is the unbanded path.  AT_E_ARG (at_last_error names the reason
+ * and the pair): a band with a mode other than AT_OVERLAP, a NULL lo or hi, lo[p] > hi[p].  Results are sized and
+ * fetched with at_batch_run / at_batch_sizes / at_batch_fetch as for any batch. */
+typedef struct at_band {
+	const int32_t *lo;     /* [n_pairs] lowest diagonal d = j - i of the band  */
+	const int32_t *hi;     /* [n_pairs] highest diagonal                        */
+} at_band;
+int  at_batch_create_banded(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
+                            const at_band *band, uint32_t out_flags, at_batch **out);
+int  at_batch_align_banded(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
+                           const at_band *band, uint32_t out_flags, at_batch_output *out, at_timing *timing);
 
 /* Sharding plan (SURVEY.md 8e): cut pairs [0, n) into `parts` CONTIGUOUS slices holding nearly equal
  * numbers of DP cells (sum of l1*l2).  cut[] receives parts+1 ascending indices, cut[0] = 0 and
