@@ -269,8 +269,9 @@ class Batch:
 
     def __init__(self, aligner, mode, opt, q, q_off, q_len, t, t_off, t_len, sites=None, site_off=None,
                  out_flags=OUT_CIGAR | OUT_ALN, encoding=SEQ_BYTES, band=None):
-        """band: None, or (lo, hi) -- per-pair int32 diagonals (d = j - i) of a banded overlap alignment
-        (at_batch_create_banded); a scalar applies to every pair."""
+        """band: None, or (lo, hi) -- per-pair int32 diagonals (d = j - i) of a banded "overlap" or "global" alignment
+        (at_batch_create_banded; a global pair's band must hold its end diagonal l2 - l1); a scalar applies to every
+        pair."""
         self.al = aligner
         self.lib = aligner.lib
         self.n = int(len(q_len))
@@ -374,8 +375,8 @@ class Aligner:
         H2D / kernels / D2H inside the library).  `out` may be a BatchResult from a previous call
         whose buffers are reused; capacities default to the worst case (l1 + l2 per pair) for
         the alignment strings and for the CIGARs (32 ops per pair once that exceeds 64 Mi ops;
-        AT_E_NOSPACE tells when to pass a larger cigar_cap).  band: (lo, hi) per-pair diagonals of a banded overlap
-        alignment (at_batch_align_banded), or None."""
+        AT_E_NOSPACE tells when to pass a larger cigar_cap).  band: (lo, hi) per-pair diagonals of a banded "overlap" or
+        "global" alignment (at_batch_align_banded), or None."""
         md = _mode(mode)
         n = int(len(q_len))
         res = out if out is not None else BatchResult(n)
@@ -418,7 +419,7 @@ class Aligner:
         return res
 
     def align(self, mode, reads, targets, opt: Opt = None, sites=None, out_flags=OUT_CIGAR | OUT_ALN, band=None) -> BatchResult:
-        """Lists of bytes in, BatchResult out (create + run + fetch).  band: (lo, hi) diagonals, overlap only."""
+        """Lists of bytes in, BatchResult out (create + run + fetch).  band: (lo, hi) diagonals, "overlap" or "global"."""
         opt = opt or Opt()
         q, qo, ql = pack_seqs(reads)
         t, to, tl = pack_seqs(targets)

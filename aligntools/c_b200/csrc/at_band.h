@@ -1,5 +1,5 @@
-// at_band.h -- geometry of a BANDED overlap pair: the caller's static band lo <= j - i <= hi on the diagonals of the
-// DP matrix, and what it means for K2's stripes and K3's pointer blocks.  Host + device: the runtime sizes pointer
+// at_band.h -- geometry of a BANDED pair (overlap or global): the caller's static band lo <= j - i <= hi on the diagonals
+// of the DP matrix, and what it means for K2's stripes and K3's pointer blocks.  Host + device: the runtime sizes pointer
 // blocks and counts cells, K2 fills and hands off, K3 walks with these functions and nothing else
 // (tests/test_banded_oracle.py compiles this header with g++ and checks the properties below without a GPU).
 //
@@ -7,8 +7,9 @@
 // ia..ib is [max(1, ia + lo), min(l2, ib + hi)]; stripes without in-band cells form a run at the top and one at the
 // bottom of the pair (the in-band rows are one interval).  The stripe's steps start at t0 = (c0 - 1) rounded down to a
 // 32-column hand-off block (lane 0 primes its diagonal input at column c0 - 1, as at column 0 unbanded) and end at
-// (c1 + 31) | 31.  Pointer words are stored relative to t0: `groups` blocks of 16 steps, 32 * R words each, stripes
-// packed one after the other.  A stripe publishes the last row of its window; every other column of that row is out of
+// (c1 + 31) | 31.  Pointer words are stored relative to t0: `groups` blocks of 2^wsh steps, 32 * R words each, stripes
+// packed one after the other (wsh = 4: overlap's 2-bit pointers, 16 steps per word; wsh = 3: the affine kernel's nibbles,
+// 8 steps per word).  A stripe publishes the last row of its window; every other column of that row is out of
 // band (-inf), so the stripe below waits only for columns in [c0, c1] of the stripe above.
 #pragma once
 #include <stdint.h>
@@ -19,7 +20,7 @@ namespace atb2 {
 struct BandWin {
 	uint32_t c0, c1;        // column window, 1 <= c0 <= c1 <= l2
 	uint32_t t0;            // first step: a multiple of 32, <= c0 - 1
-	uint32_t groups;        // 16-step pointer groups of the stripe
+	uint32_t groups;        // pointer groups (2^wsh steps) of the stripe
 };
 
 // The band clipped to the matrix's diagonals [1 - l1, l2 - 1], in 64 bits (int32 extremes do not overflow); an empty
@@ -33,7 +34,7 @@ AT_HD void band_clip(uint32_t l1, uint32_t l2, int64_t lo, int64_t hi, int32_t &
 }
 
 // Window of stripe s (rows s*RPP+1 .. min((s+1)*RPP, l1)) of a clipped band; false when the stripe has no in-band cell.
-AT_HD bool band_stripe(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP, uint32_t s, BandWin &w)
+AT_HD bool band_stripe(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP, uint32_t s, BandWin &w, uint32_t wsh = 4)
 {
 	if (elo > ehi) return false;
 	const int64_t ia = (int64_t)s * RPP + 1, ibx = ((int64_t)s + 1) * RPP, ib = ibx < (int64_t)l1 ? ibx : (int64_t)l1;
@@ -42,30 +43,30 @@ AT_HD bool band_stripe(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint3
 	if (a > b) return false;
 	w.c0 = (uint32_t)a; w.c1 = (uint32_t)b;
 	w.t0 = (w.c0 - 1u) & ~31u;
-	w.groups = ((w.c1 + 31u - w.t0) >> 4) + 1u;
+	w.groups = ((w.c1 + 31u - w.t0) >> wsh) + 1u;
 	return true;
 }
 
 AT_HD uint32_t band_t_last(const BandWin &w) { return (w.c1 + 31u) | 31u; }
 
 // pointer words of stripe s (0 when it is empty)
-AT_HD uint64_t band_stripe_words(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP, uint32_t s)
+AT_HD uint64_t band_stripe_words(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP, uint32_t s, uint32_t wsh = 4)
 {
 	BandWin w;
-	return band_stripe(l1, l2, elo, ehi, RPP, s, w) ? (uint64_t)w.groups * RPP : 0;
+	return band_stripe(l1, l2, elo, ehi, RPP, s, w, wsh) ? (uint64_t)w.groups * RPP : 0;
 }
 
 // word offset of stripe s in the pair's pointer block (the words of the stripes above it)
-AT_HD uint64_t band_stripe_off(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP, uint32_t s)
+AT_HD uint64_t band_stripe_off(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP, uint32_t s, uint32_t wsh = 4)
 {
 	uint64_t off = 0;
-	for (uint32_t x = 0; x < s; ++x) off += band_stripe_words(l1, l2, elo, ehi, RPP, x);
+	for (uint32_t x = 0; x < s; ++x) off += band_stripe_words(l1, l2, elo, ehi, RPP, x, wsh);
 	return off;
 }
 
-AT_HD uint64_t band_pair_words(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP)
+AT_HD uint64_t band_pair_words(uint32_t l1, uint32_t l2, int32_t elo, int32_t ehi, uint32_t RPP, uint32_t wsh = 4)
 {
-	return band_stripe_off(l1, l2, elo, ehi, RPP, (l1 + RPP - 1) / RPP);
+	return band_stripe_off(l1, l2, elo, ehi, RPP, (l1 + RPP - 1) / RPP, wsh);
 }
 
 // The column the first stripe below a producer waits for before it starts (three hand-off blocks past its own first

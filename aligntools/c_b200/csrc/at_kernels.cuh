@@ -37,7 +37,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "at_cell.cuh"      // Lanes<>, cell_update(), AT_NEG: the cell arithmetic shared by K1 and K2
-#include "at_band.h"        // banded overlap: stripe windows and pointer layout shared by the runtime, K2 and K3
+#include "at_band.h"        // banded overlap / global: stripe windows and pointer layout shared by the runtime, K2 and K3
 
 // traceback walker's look-ahead: how far ahead (steps) and how often (every PERIOD-th step, a power of two) it prefetches
 #ifndef AT_TB_PF_AHEAD
@@ -137,22 +137,22 @@ struct PtrView {
 		const uint32_t w = __ldg(ptrJ + rowJ + (size_t)(t >> 5) * RPP);
 		return (w >> (31 - (t & 31))) & 1u;
 	}
-	// Banded overlap pairs (at_band.h): stripe s's words start at off(s) and count 16-step groups from the stripe's first
-	// step t0, so rowA folds in - (t0 / 16) * RPP and two() stays as it is.  Crossing to the stripe above moves `off` back
-	// by that stripe's words.
-	uint32_t l1, l2, stripe, t0;
+	// Banded pairs (at_band.h): stripe s's words start at off(s) and count groups of 2^wsh steps (overlap 16, global 8) from
+	// the stripe's first step t0, so rowA folds in - (t0 >> wsh) * RPP and two() / nib() stay as they are.  Crossing to the
+	// stripe above moves `off` back by that stripe's words.
+	uint32_t l1, l2, stripe, t0, wsh;
 	int32_t elo, ehi;
 	uint64_t off;
 	__device__ __forceinline__ void band_base() {                 // rowA of row 0 of lane 0 of `stripe` (row -1 of a stripe without a window: never read)
 		BandWin w;
-		const uint32_t t = band_stripe(l1, l2, elo, ehi, RPP, stripe, w) ? w.t0 : 0u;
+		const uint32_t t = band_stripe(l1, l2, elo, ehi, RPP, stripe, w, wsh) ? w.t0 : 0u;
 		t0 = t;
-		rowA = (size_t)off - (size_t)(t >> 4) * RPP;
+		rowA = (size_t)off - (size_t)(t >> wsh) * RPP;
 	}
 	__device__ __forceinline__ void seek_band(uint32_t i) {       // i >= 1
 		const uint32_t ri = i - 1, rem = ri % RPP;
 		stripe = ri / RPP; lane = rem / R; r = rem - lane * R;
-		off = band_stripe_off(l1, l2, elo, ehi, RPP, stripe);
+		off = band_stripe_off(l1, l2, elo, ehi, RPP, stripe, wsh);
 		band_base();
 		rowA += (size_t)lane * R + r;
 	}
@@ -163,7 +163,7 @@ struct PtrView {
 		lane = 31;
 		if (stripe == 0) return;                                  // leaving row 1: the walk stops at row 0
 		--stripe;
-		off -= band_stripe_words(l1, l2, elo, ehi, RPP, stripe);
+		off -= band_stripe_words(l1, l2, elo, ehi, RPP, stripe, wsh);
 		band_base();
 		rowA += RPP - 1;
 	}
@@ -185,8 +185,9 @@ struct RunWriter {
 // BESIDE_FILL only makes two distinct functions: the <true> instances are given the fill kernels'
 // shared-memory carve-out (they run beside another stream's persistent fill grid in the pipelined
 // path), the <false> instances keep the default carve-out -- the walk lives on L1 hits.
-// BANDED (overlap with a per-pair band): the pointer block has the banded layout (PtrView::seek_band / up_band) and a
-// walk that reaches a cell outside the band stops, as at row 0 -- cells on a finite path are in band.
+// BANDED (overlap or global with a per-pair band): the pointer block has the banded layout (PtrView::seek_band / up_band)
+// and a walk that reaches a cell outside the band stops, as at row 0 -- cells on a finite path are in band.  Global's
+// flush after the walk is the unbanded one.
 template <bool BESIDE_FILL, bool BANDED = false>
 __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 {
@@ -212,17 +213,26 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 	w.dst = a.scratch + a.scratch_off[k]; w.n_ops = w.n_cols = w.run = 0; w.op = 0;
 	uint32_t i = a.end_i[p], j = a.end_j[p], state = a.end_state[p], tick = 3;
 	if constexpr (BANDED) {
-		pv.l1 = l1; pv.l2 = l2; pv.elo = a.band[p].x; pv.ehi = a.band[p].y;
+		const bool ov = a.mode == MODE_OVERLAP;
+		pv.l1 = l1; pv.l2 = l2; pv.elo = a.band[p].x; pv.ehi = a.band[p].y; pv.wsh = ov ? 4u : 3u;
 		if (i && j) pv.seek_band(i);
 		while (j > 0) {
 			if (i == 0) break;
 			if ((int)j - (int)i < pv.elo || (int)j - (int)i > pv.ehi) break;      // out of band: not on a finite path
 			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u)) && pv.lane * pv.R + pv.r >= AT_TB_PF_AHEAD && j > pv.t0 + AT_TB_PF_AHEAD + 1)
-				pv.prefetch(i, j, 4);                                              // rows and columns of the look-ahead stay in the stripe's block
-			const uint32_t c = pv.two(j);
-			if (c & 2u)      { --i; pv.up_band(); w.col(CIG_I); }
-			else if (c & 1u) { --i; pv.up_band(); --j; w.col(CIG_M); }
-			else             { --j; w.col(CIG_D); }
+				pv.prefetch(i, j, (int)pv.wsh);                                    // rows and columns of the look-ahead stay in the stripe's block
+			if (ov) {
+				const uint32_t c = pv.two(j);
+				if (c & 2u)      { --i; pv.up_band(); w.col(CIG_I); }
+				else if (c & 1u) { --i; pv.up_band(); --j; w.col(CIG_M); }
+				else             { --j; w.col(CIG_D); }
+			} else {                                                               // global (:377-397)
+				const uint32_t nb = pv.nib(j);
+				if (state == ST_LOW)      { state = (nb & 4u) ? ST_MID : ST_LOW; --i; pv.up_band(); w.col(CIG_I); }
+				else if (state == ST_MID) { state = nb & 3u; --i; pv.up_band(); --j; w.col(CIG_M); }
+				else if (state == ST_UPP) { state = (nb & 8u) ? ST_UPP : ST_MID; --j; w.col(CIG_D); }
+				else break;                                                        // no JUMP / HOME state in global: corrupt pointers
+			}
 		}
 	} else {
 	if (i) pv.seek(i);

@@ -211,7 +211,7 @@ struct Shard {
 	bool prof = false; uint32_t syms = 0;      // query-profile variant of K1: the targets use <= 4 distinct bytes
 	bool bits = false;                         // bit-parallel edit distance: `-u 1` and reads of <= 8 distinct bytes
 	bool twobit = false;                       // the sequences stay 2-bit packed in HBM (AT_SEQ_2BIT input consumed directly by K1 / K2 / K3)
-	bool banded = false;                       // overlap with a per-pair band: h_band / d_band hold it clipped (at_band.h)
+	bool banded = false;                       // overlap / global with a per-pair band: h_band / d_band hold it clipped (at_band.h)
 	std::vector<int2> h_band;
 	DevBuf<int2> d_band;
 	std::vector<uint64_t> h_t_rel;             // twobit + jump: device offsets of the packed targets (the jump masks copy their alignment)
@@ -583,17 +583,20 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		CU(h, s.d_band.alloc(n));
 		CU(h, cudaMemcpyAsync(s.d_band.p, s.h_band.data(), n * sizeof(int2), cudaMemcpyHostToDevice, st));      // staged before the set-up's synchronisation
 	}
-	// banded pairs: the in-band cells, the pointer words of their stripe windows (at_band.h)
+	// banded pairs: the in-band cells, the pointer words of their stripe windows (at_band.h).  Banded global pairs all run
+	// on K2's affine kernel, short ones included: R = 8 rows per lane, 8-step pointer groups
+	const bool band_affine = s.banded && b->mode == AT_GLOBAL;
+	auto rclass = [&](uint32_t l1) -> uint32_t { return band_affine ? (uint32_t)MAXR : rclass_of(l1); };
 	auto pair_cells = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t { return s.banded ? band_cells(l1, l2, s.h_band[k].x, s.h_band[k].y) : (uint64_t)l1 * l2; };
 	auto pair_ptr_words = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t {
-		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass_of(l1)) : ptr_words_of(b->mode, jump, l1, l2);
+		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass(l1), band_affine ? 3u : 4u) : ptr_words_of(b->mode, jump, l1, l2);
 	};
 	if ((rc = choose_variants(b, s, in, q_span))) return rc;
 	if (jump && (rc = build_jump_mask(b, s, in))) return rc;
 	mark("alphabet+jmask");
 	// a UNIFORM shard (every pair of the same shape, all on K1) needs no per-pair work on the host at all: see below
 	const uint32_t l1u = in->q_len[s.p0], l2u = in->t_len[s.p0];
-	bool uniform = b->mode <= AT_FIT && l1u <= 32u * MAXR && !getenv("AT_NO_UNIFORM_PLAN");
+	bool uniform = b->mode <= AT_FIT && l1u <= 32u * MAXR && !band_affine && !getenv("AT_NO_UNIFORM_PLAN");
 	for (uint32_t k = 1; k < n && uniform; ++k) uniform = in->q_len[s.p0 + k] == l1u && in->t_len[s.p0 + k] == l2u;
 	// per-pair class, result arrays
 	s.cells = 0;
@@ -602,7 +605,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		s.h_rclass.resize(n);
 		for (uint32_t k = 0; k < n; ++k) {
 			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-			s.h_rclass[k] = (uint8_t)rclass_of(l1);
+			s.h_rclass[k] = (uint8_t)rclass(l1);
 			s.cells += pair_cells(k, l1, l2);
 		}
 	}
@@ -623,7 +626,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 	uint64_t need_words = 0;
 	auto pair_words = [&](uint32_t k) -> uint64_t {
 		const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-		return b->traceback ? pair_ptr_words(k, l1, l2) + 64ull * rclass_of(l1) : 0;   // + rounding slack of the packed layout
+		return b->traceback ? pair_ptr_words(k, l1, l2) + 64ull * rclass(l1) : 0;   // + rounding slack of the packed layout
 	};
 	if (uniform) need_words = (uint64_t)n * pair_words(0);
 	else for (uint32_t k = 0; k < n; ++k) need_words += pair_words(k);
@@ -729,7 +732,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		std::vector<uint32_t> scalar_pairs, wave_pairs, cand;
 		for (uint32_t k = c.k0; k < c.k1; ++k) {
 			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-			if (linear || l1 > 32u * MAXR) wave_pairs.push_back(k);
+			if (linear || band_affine || l1 > 32u * MAXR) wave_pairs.push_back(k);
 			else if (p16_ok(l1, l2)) cand.push_back(k);
 			else scalar_pairs.push_back(k);
 		}
@@ -776,7 +779,8 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 			const uint32_t n_stripes = (l1 + rows - 1) / rows;
 			uint32_t queued = 0;
 			for (uint32_t st2 = 0; st2 < n_stripes; ++st2) {
-				// banded: only stripes with a window run; the last stripe always does (it writes the end cell)
+				// banded: only stripes with a window run; the last stripe always does (it writes the end cell; banded global:
+				// the end diagonal is in band, so the last stripe has a window)
 				BandWin w;
 				if (s.banded && st2 + 1 < n_stripes && !band_stripe(l1, l2, s.h_band[k].x, s.h_band[k].y, rows, st2, w)) continue;
 				lw.h_tasks.push_back(WaveTask{k, st2, 0, 0});
@@ -1009,15 +1013,37 @@ static at_batch *new_batch(at_handle *h, int mode, const at_params *p, uint32_t 
 	return b;
 }
 
-// a band is for AT_OVERLAP only, with both arrays and lo[p] <= hi[p] for every pair
+// a band is for AT_OVERLAP and AT_GLOBAL, with both arrays and lo[p] <= hi[p] for every pair; a global pair's band must
+// hold its end diagonal l2 - l1 (then every in-band cell is finite and a banded global result always exists)
 static int validate_band(at_handle *h, int mode, const at_batch_input *in, const at_band *band)
 {
 	if (!band) return AT_OK;
-	if (mode != AT_OVERLAP) { set_err(h, "band: only overlap alignment takes a band (mode %d)", mode); return AT_E_ARG; }
+	if (mode != AT_OVERLAP && mode != AT_GLOBAL) { set_err(h, "band: only overlap alignment takes a band (mode %d)", mode); return AT_E_ARG; }
 	if (!band->lo || !band->hi) { set_err(h, "band: %s is NULL", band->lo ? "hi" : "lo"); return AT_E_ARG; }
-	for (uint64_t k = 0; k < in->n_pairs; ++k)
+	for (uint64_t k = 0; k < in->n_pairs; ++k) {
 		if (band->lo[k] > band->hi[k]) { set_err(h, "band: lo > hi at pair %llu (%d > %d)", (unsigned long long)k, band->lo[k], band->hi[k]); return AT_E_ARG; }
+		const int64_t d = (int64_t)in->t_len[k] - (int64_t)in->q_len[k];
+		if (mode == AT_GLOBAL && (d < band->lo[k] || d > band->hi[k])) {
+			set_err(h, "band: pair %llu: global alignment's end diagonal l2 - l1 = %lld lies outside the band [%d, %d]",
+			        (unsigned long long)k, (long long)d, band->lo[k], band->hi[k]);
+			return AT_E_ARG;
+		}
+	}
 	return AT_OK;
+}
+
+// K2 tasks of a banded global batch: every pair runs on K2, one task per stripe of 256 rows with a window (at_band.h)
+static uint64_t banded_global_tasks(const at_batch_input *in, const at_band *band)
+{
+	uint64_t n = 0;
+	for (uint64_t k = 0; k < in->n_pairs; ++k) {
+		const uint32_t l1 = in->q_len[k], l2 = in->t_len[k], RPP = 32u * MAXR;
+		int32_t elo, ehi;
+		band_clip(l1, l2, band->lo[k], band->hi[k], elo, ehi);
+		BandWin w;
+		for (uint32_t s = (l1 + RPP - 1) / RPP; s-- > 0 && band_stripe(l1, l2, elo, ehi, RPP, s, w, 3u);) ++n;      // the windows are the bottom run
+	}
+	return n;
 }
 
 extern "C" int at_batch_create(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
@@ -1088,8 +1114,12 @@ template <int MODE, bool PROF, bool BANDED = false> static wave_fn wave_linear_f
 	case 7: return at_wave_linear<MODE, 7, PROF, BANDED>; default: return at_wave_linear<MODE, 8, PROF, BANDED>;
 	}
 }
-// banded overlap (validate_band admits a band with AT_OVERLAP only)
-static wave_fn wave_banded_kernel(int R, bool prof) { return prof ? wave_linear_fn<MODE_OVERLAP, true, true>(R) : wave_linear_fn<MODE_OVERLAP, false, true>(R); }
+// banded overlap / global (validate_band admits a band with AT_OVERLAP and AT_GLOBAL only)
+static wave_fn wave_banded_kernel(int mode, int R, bool prof)
+{
+	if (mode == AT_GLOBAL) return prof ? at_wave_affine<MODE_GLOBAL, false, true, true> : at_wave_affine<MODE_GLOBAL, false, false, true>;
+	return prof ? wave_linear_fn<MODE_OVERLAP, true, true>(R) : wave_linear_fn<MODE_OVERLAP, false, true>(R);
+}
 static wave_fn bits_kernel(int R) { return R == 1 ? at_wave_edit_bits<1> : (R == 2 ? at_wave_edit_bits<2> : at_wave_edit_bits<4>); }
 static wave_fn wave_kernel(int mode, bool jump, int R, bool prof)
 {
@@ -1139,7 +1169,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 		if (first) { CU(h, cudaEventRecord(e_first, st)); first = false; }
 		for (size_t li = 0; li < c.launches.size(); ++li) {
 			Launch &l = c.launches[li];
-			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r) : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(l.r, s.prof) : (const void *)wave_kernel(b->mode, jump, l.r, s.prof))
+			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r) : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(b->mode, l.r, s.prof) : (const void *)wave_kernel(b->mode, jump, l.r, s.prof))
 			                                   : (const void *)affine_kernel(l.kind == LK_PACKED ? (b->mode == AT_LOCAL ? 4 : b->mode == AT_GLOBAL ? 5 : 6) : (b->mode == AT_FIT ? (jump ? 3 : 2) : b->mode), l.r, s.prof);
 			const int warps = l.kind >= LK_WAVE ? AT_WAVE_WARPS : AT_FILL_WARPS;
 			const size_t dyn_smem = l.kind >= LK_WAVE ? 0 : fill_smem_bytes(l.r, l.kind == LK_PACKED, s.prof);

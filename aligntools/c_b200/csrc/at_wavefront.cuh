@@ -35,6 +35,9 @@ namespace atb2 {
 #ifndef AT_WAVE_AFFINE_MINB
 #define AT_WAVE_AFFINE_MINB 4      // resident CTAs per SM the affine kernel is compiled for (128 registers)
 #endif
+#ifndef AT_WAVE_AFFINE_BANDED_MINB
+#define AT_WAVE_AFFINE_BANDED_MINB 3      // the banded instantiation: its band masks spill at 128 registers
+#endif
 #ifndef AT_WAVE_UNROLL_AFFINE_N
 #define AT_WAVE_UNROLL_AFFINE_N 2
 #endif
@@ -199,9 +202,21 @@ __device__ __forceinline__ void wait_columns(const uint32_t *prog, uint32_t need
 // Lane 0's upper neighbour is matrix row 0 (first stripe) or the boundary row of the stripe above (a predicated
 // LDS from the boundary ring); it enters through a multiply-add with a 0/1 lane mask, not a branch.
 // Boundary element (int4 per column): x = M + o (tag 3), y = L (tag 3), z = H (tagged), w unused.
-template <int MODE, bool JUMP, bool PROF>
-__global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wave_affine(const WaveArgs a)
+//
+// BANDED (global only): the pair's band (at_band.h, 8-step pointer groups: wsh = 3) limits every stripe to its column
+// window.  The band holds the end diagonal l2 - l1 (the host checks it), so the stripes without a window are a run at the
+// top of the pair and the host queues none of them.  The steps run from the window's t0 to (c1 + 31) | 31; 8-step blocks
+// whose cells may leave the band force M, L and U of those cells to -inf, blocks wholly inside the band run the plain body.
+// With t0 > 0 every cell left of the window is out of band: the lanes' left state and lane 0's diagonal start at -inf.
+// The first stripe with a window below empty ones has no predecessor: its row above is -inf at every column j >= 1 and
+// keeps the column-0 border H(row0, 0).  A stripe publishes the window columns of its last row; the stripe below waits
+// only for columns inside the producer's window and takes -inf for the others (the slab entries outside the window hold
+// values of the stripe two above).  Target tiles keep their absolute numbering, only those the window reads are staged.
+// Pointer words are stored relative to t0 at the stripe's offset in the pair's block (band_stripe_off).
+template <int MODE, bool JUMP, bool PROF, bool BANDED = false>
+__global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BANDED_MINB : AT_WAVE_AFFINE_MINB) at_wave_affine(const WaveArgs a)
 {
+	static_assert(!BANDED || (MODE == MODE_GLOBAL && !JUMP), "banded affine kernel: global alignment only");
 	typedef Lanes<false> V;
 	constexpr int R = 8, RPP = 32 * R;
 	constexpr bool LOCAL = MODE == MODE_LOCAL;
@@ -243,14 +258,28 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 		const uint32_t sh = twobit ? 4u * sh16 : sh16;                        // ring position of target index 0
 		const uint32_t tile_wait = twobit ? 192u : 224u;                      // step (mod 256) at which the next tile must have landed: lane 0 is up to sh + 1 columns ahead of the step counter
 		const uint8_t *jbase16 = JUMP ? a.jmask + a.j_off[p] - sh : nullptr;     // the host lays the masks out with the targets' ring alignment
-		const uint32_t n_tiles = (l2 + sh + 255u) >> 8;
+		uint32_t n_tiles = (l2 + sh + 255u) >> 8;
 		uint32_t *__restrict__ ptr = a.ptr + a.ptr_off[p - a.pair_base];
 		const uint32_t t_ptr_last = (l2 + 31u) | (JUMP ? 31u : 7u);       // pointer-block geometry shared with K1 / K3
 		const uint32_t G = (t_ptr_last >> 3) + 1, GJ = (t_ptr_last >> 5) + 1;
-		const uint32_t t_last = (l2 + 31u) | 31u;
+		uint32_t t_last = (l2 + 31u) | 31u;
 		const uint32_t n_stripes = (l1 + RPP - 1) / RPP;
 		uint32_t *__restrict__ ptrJ = ptr + (size_t)n_stripes * G * RPP;
 		const bool last_stripe = stripe + 1 == n_stripes;
+		// banded: this stripe's window (bw), the one above (bwp), whether the stripe above takes part
+		BandWin bw = {1u, l2, 0u, G}, bwp = bw;
+		int32_t elo = 0, ehi = 0;
+		bool has_prev = stripe > 0;
+		if constexpr (BANDED) {
+			const int2 bd = a.band[p];
+			elo = bd.x; ehi = bd.y;
+			band_stripe(l1, l2, elo, ehi, RPP, stripe, bw, 3u);             // queued stripes have a window
+			has_prev = stripe > 0 && band_stripe(l1, l2, elo, ehi, RPP, stripe - 1u, bwp, 3u);
+			t_last = band_t_last(bw);
+			n_tiles = min(n_tiles, ((bw.c1 - 1u + sh) >> 8) + 1u);         // tiles the window reads
+			if (want_ptr) ptr += band_stripe_off(l1, l2, elo, ehi, RPP, stripe, 3u);
+		}
+		const uint32_t tile0 = bw.t0 >> 8;                                 // first tile the stripe reads (0 unbanded)
 		const uint32_t slab = (l2 + 4u) & ~3u;
 		int4 *bnd_pair = (int4 *)a.bnd + a.bnd_off[p - a.pair_base];
 		int4 *bnd_out = bnd_pair + (size_t)(stripe & 1u) * slab;
@@ -258,12 +287,13 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 		const uint32_t *prog_in = a.prog + tk.prev;
 		uint32_t seen = 0;
 		const uint32_t row0 = stripe * RPP + lane * R;
-		const bool feed = lane == 0 && stripe > 0;                         // this lane reads the boundary ring
+		const bool feed = lane == 0 && has_prev;                           // this lane reads the boundary ring
 		const bool park = lane == 31 && !last_stripe;                      // this lane parks its last row for the next stripe
+		const bool left_neg = BANDED && bw.t0 > 0;                         // banded: the cells left of the window are -inf
 
 		__syncwarp();
-		if (n_tiles > 0) ring_issue<JUMP>(sm.rg, tbase16, jbase16, 0, lane, twobit);
-		if (n_tiles > 1) ring_issue<JUMP>(sm.rg, tbase16, jbase16, 1, lane, twobit);
+		if (n_tiles > tile0) ring_issue<JUMP>(sm.rg, tbase16, jbase16, tile0, lane, twobit);
+		if (n_tiles > tile0 + 1u) ring_issue<JUMP>(sm.rg, tbase16, jbase16, tile0 + 1u, lane, twobit);
 
 		RowState<false, JUMP> st[R];
 		int crow[R];
@@ -280,7 +310,8 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 			}
 			crow[r] = ri < l1 ? 5 - r : -(1 << 28);                       // on top of Mk = 8 M + 2: key = 8 M + 7 - r
 			// column 0 (left border), tags as cell_update leaves them
-			if (MODE == MODE_GLOBAL)     { st[r].mo = NEGV | 3; st[r].u = NEGV | 1; st[r].h = 8 * (o + e * i) | TAG_L; }      // :432-436
+			if (left_neg)                { st[r].mo = NEGV | 3; st[r].u = NEGV | 1; st[r].h = NEGV | TAG_M; }
+			else if (MODE == MODE_GLOBAL) { st[r].mo = NEGV | 3; st[r].u = NEGV | 1; st[r].h = 8 * (o + e * i) | TAG_L; }     // :432-436
 			else if (MODE == MODE_LOCAL) { st[r].mo = ZERO + o8 + 3; st[r].u = ZERO | 1; st[r].h = ZERO | TAG_L; }            // calloc zeros
 			else                         { st[r].mo = NEGV | 3; st[r].u = NEGV | 1; st[r].h = NEGV | TAG_M; }                 // :612-617
 			st[r].j = NEGV; st[r].x = 0; st[r].xj = 0;
@@ -288,8 +319,10 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 		if (PROF) __syncwarp();
 		int sM = st[R - 1].mo, sH = st[R - 1].h;
 		int sL = MODE == MODE_GLOBAL ? (8 * (o + e * (int)(row0 + R)) | 3) : (MODE == MODE_LOCAL ? (ZERO | 3) : (NEGV | 3));
-		int pH;      // H(row0, 0): the row above this lane's strip, column 0
-		if (row0 == 0) {
+		if (left_neg) sL = NEGV | 3;
+		int pH;      // H(row0, 0): the row above this lane's strip, column 0 (banded, t0 > 0: H(row0, t0 - 1) = -inf)
+		if (left_neg) pH = NEGV | TAG_M;
+		else if (row0 == 0) {
 			if (MODE == MODE_GLOBAL)     pH = 8 * (o < 0 ? 0 : o) | (o < 0 ? TAG_M : TAG_L);                                 // max5(L=o, M=0, U=o)
 			else if (MODE == MODE_LOCAL) pH = ZERO | TAG_L;
 			else                         pH = ZERO | TAG_M;                                                                  // M[0][0]=U[0][0]=0
@@ -300,13 +333,15 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 		}
 		// what lane 0 adds instead of a neighbour's row (zero in every other lane): matrix row 0 in the first stripe,
 		// the boundary ring's element of the column otherwise (loaded per step by lane 0 alone)
+		// (banded, first stripe with a window below empty ones: the row above is out of band, -inf)
 		int4 bq = make_int4(0, 0, 0, 0);
 		int b0E = 0;
+		const int4 neg4 = make_int4(NEGV | 3, NEGV | 3, NEGV | TAG_M, 0);      // banded: a boundary column outside the producer's window
 		if (lane == 0 && stripe == 0) {
 			if (MODE == MODE_GLOBAL)     { bq.x = NEGV | 3; bq.y = NEGV | 3; bq.z = 8 * o | TAG_U; b0E = e8; }                // :437-441, U[0][j] = o + e j
 			else if (MODE == MODE_LOCAL) { bq.x = ZERO + o8 + 3; bq.y = ZERO | 3; bq.z = ZERO | TAG_L; }
 			else                         { bq.x = ZERO + o8 + 3; bq.y = NEGV | 3; bq.z = ZERO | TAG_M; }                      // :619-624
-		}
+		} else if (BANDED && lane == 0 && !has_prev) bq = neg4;
 		const int cap_r = (last_stripe && lane == (int)(((l1 - 1) % RPP) / R)) ? (int)((l1 - 1) % R) : -1;
 		int hot[R];
 #pragma unroll
@@ -316,18 +351,32 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 		int gH = 0;                                                                 // global
 
 		// first boundary block of the stripe above
+		// (banded: the columns [in0, in1] the stripe above publishes -- its window; only those are awaited and read)
+		const uint32_t in0 = BANDED ? bwp.c0 : 1u, in1 = BANDED ? bwp.c1 : l2;
 		int4 pre = make_int4(0, 0, 0, 0);
-		if (stripe) {
-			wait_columns(prog_in, min(l2, max(31u, a.start_lag)), seen, lane);
-			if ((uint32_t)lane <= l2) pre = __ldcg(bnd_in + lane);
+		if (has_prev) {
+			if constexpr (BANDED) {
+				wait_columns(prog_in, min(max(bw.t0 + max(31u, a.start_lag), in0), in1), seen, lane);
+				const uint32_t col = bw.t0 + lane;
+				pre = col >= in0 && col <= in1 ? __ldcg(bnd_in + col) : neg4;
+			} else {
+				wait_columns(prog_in, min(l2, max(31u, a.start_lag)), seen, lane);
+				if ((uint32_t)lane <= l2) pre = __ldcg(bnd_in + lane);
+			}
 		}
-		mbar_wait(&sm.rg.bar[0], ring_par & 1u); ring_par ^= 1u;
-		if (twobit) ring_expand(sm.rg, 0, lane);
+		mbar_wait(&sm.rg.bar[tile0 & 1u], (ring_par >> (tile0 & 1u)) & 1u); ring_par ^= 1u << (tile0 & 1u);
+		if (twobit) ring_expand(sm.rg, tile0, lane);
+		if (BANDED && (bw.t0 & 255u) > tile_wait && tile0 + 1u < n_tiles) {      // the window starts past the point where the next tile is awaited
+			const uint32_t c = tile0 + 1u;
+			mbar_wait(&sm.rg.bar[c & 1u], (ring_par >> (c & 1u)) & 1u); ring_par ^= 1u << (c & 1u); if (twobit) ring_expand(sm.rg, c, lane);
+		}
 
 		// `cap`: std::true_type in the pair's last stripe -- only there can a lane hold the row whose cells the
 		// end-cell search looks at; the other stripes run a body without it
-		auto step = [&](const uint32_t t, const bool checked, auto cap) {
+		// `msk`: std::true_type where cells of the step may lie outside the pair's band (BANDED only): they become -inf
+		auto step = [&](const uint32_t t, const bool checked, auto cap, auto msk) {
 			constexpr bool CAP = decltype(cap)::value;
+			constexpr bool MSK = decltype(msk)::value;
 			const int j = (int)t - lane;
 			if (feed) bq = sm.cring[t & 63u];
 			const int rM = __shfl_up_sync(0xffffffffu, sM, 1) * nz + bq.x;
@@ -358,6 +407,10 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 					if (PROF) s8 = pw[r];
 					else { const int tt = (int)min(ac[r] ^ c, mu8); s8 = tt * nsg + m8; }   // tt: 0 on a match, 8|m-u| otherwise
 					D = cell_update<LOCAL, JUMP, false, true>(cc, st[r], D, s8, lup, mo_up, jadd, 16u, 2u, out);
+					if (MSK && (uint32_t)(j - (int)row0 - 1 - r - elo) > (uint32_t)(ehi - elo)) {     // d = j - i out of band
+						out.mo = out.lk = NEGV | 3; out.h = NEGV | TAG_M;
+						st[r].mo = out.mo; st[r].u = NEGV | 1; st[r].h = out.h;
+					}
 					lup = out.lk; mo_up = out.mo;
 					if (LOCAL) kbest = __viaddmax_s32(out.mk, crow[r], kbest);
 					if (MODE == MODE_FIT && CAP) { rowM += out.mk * hot[r]; rowL += out.lk * hot[r]; }      // one-hot pick of the pair's last row (FMA pipe)
@@ -379,26 +432,31 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 			}
 		};
 
-		for (uint32_t tb = 0; tb <= t_last; tb += 8) {
+		// columns this stripe publishes (banded: its window)
+		const int pub0 = (int)bw.c0, pub1 = (int)bw.c1;
+		for (uint32_t tb = bw.t0; tb <= t_last; tb += 8) {
 			if ((tb & 31u) == 0) {
 				__syncwarp();
 				if (!last_stripe && tb >= 64u) {      // lane 31 has finished the columns up to tb-32: flush (tb-64, tb-32]
 					const int cidx = (int)tb - 63 + lane;
-					if (cidx >= 1 && cidx <= (int)l2) __stcg(bnd_out + cidx, sm.stage[(uint32_t)cidx & 63u]);
+					if (cidx >= pub0 && cidx <= pub1) __stcg(bnd_out + cidx, sm.stage[(uint32_t)cidx & 63u]);
 					__syncwarp();
 					if (lane == 0) st_release(a.prog + job, min(tb - 32u, l2));
 				}
-				if (stripe) {                         // block tb of the stripe above -> ring; fetch block tb+32
+				if (has_prev) {                       // block tb of the stripe above -> ring; fetch block tb+32
 					sm.cring[(tb + lane) & 63u] = pre;
 					const uint32_t nxt = tb + 32u + lane;
-					if (tb + 32u <= l2) {
+					if constexpr (BANDED) {
+						if (tb + 32u <= in1 && tb + 63u >= in0) wait_columns(prog_in, min(in1, tb + 63u), seen, lane);
+						pre = nxt >= in0 && nxt <= in1 ? __ldcg(bnd_in + nxt) : neg4;
+					} else if (tb + 32u <= l2) {
 						wait_columns(prog_in, min(l2, tb + 63u), seen, lane);
 						if (nxt <= l2) pre = __ldcg(bnd_in + nxt);
 					}
 					__syncwarp();
 				}
 			}
-			if ((tb & 255u) == 32u && tb > 32u) {     // tile tb/256 - 1 is dead: refill its slot two tiles ahead
+			if ((tb & 255u) == 32u && (BANDED ? (tb >> 8) > tile0 : tb > 32u)) {     // tile tb/256 - 1 is dead: refill its slot two tiles ahead
 				const uint32_t c = (tb >> 8) + 1u;
 				__syncwarp();
 				if (c < n_tiles) ring_issue<JUMP>(sm.rg, tbase16, jbase16, c, lane, twobit);
@@ -409,19 +467,35 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 			}
 			// two steps per loop body: 8 rows x 2 steps already is ~400 instructions; a fully unrolled pointer
 			// word (8 steps) overflows the instruction cache (ncu: stall_no_instruction was the top stall)
-			if (tb >= 32u && tb + 7u <= l2) {
+			// banded: d = j - i of the block's cells spans [tb - row(stripe) - RPP - 31, tb + 6 - row(stripe)]
+			const bool inner = !BANDED || ((int64_t)tb - (int64_t)stripe * RPP - RPP - 31 >= elo && (int64_t)tb + 6 - (int64_t)stripe * RPP <= ehi);
+			if (tb >= 32u && tb + 7u <= l2 && inner) {
 				if (last_stripe) {
 #pragma unroll AT_WAVE_UNROLL_AFFINE
-					for (uint32_t k = 0; k < 8; ++k) step(tb + k, false, std::true_type());
+					for (uint32_t k = 0; k < 8; ++k) step(tb + k, false, std::true_type(), std::false_type());
 				} else {
 #pragma unroll AT_WAVE_UNROLL_AFFINE
-					for (uint32_t k = 0; k < 8; ++k) step(tb + k, false, std::false_type());
+					for (uint32_t k = 0; k < 8; ++k) step(tb + k, false, std::false_type(), std::false_type());
+				}
+			} else if (BANDED && tb >= 32u && tb + 7u <= l2) {
+				if (last_stripe) {
+#pragma unroll AT_WAVE_UNROLL_AFFINE
+					for (uint32_t k = 0; k < 8; ++k) step(tb + k, false, std::true_type(), std::true_type());
+				} else {
+#pragma unroll AT_WAVE_UNROLL_AFFINE
+					for (uint32_t k = 0; k < 8; ++k) step(tb + k, false, std::false_type(), std::true_type());
 				}
 			} else {
 #pragma unroll 1
-				for (uint32_t k = 0; k < 8; ++k) step(tb + k, true, std::true_type());
+				for (uint32_t k = 0; k < 8; ++k) step(tb + k, true, std::true_type(), std::integral_constant<bool, BANDED>());
 			}
-			if (want_ptr && (tb >> 3) < G) {
+			if constexpr (BANDED) {
+				if (want_ptr && ((tb - bw.t0) >> 3) < bw.groups) {
+					uint32_t *w = ptr + ((size_t)((tb - bw.t0) >> 3) * 32 + lane) * R;
+#pragma unroll
+					for (int r = 0; r < R; ++r) w[r] = ptr_word(st[r].x);
+				}
+			} else if (want_ptr && (tb >> 3) < G) {
 				uint32_t *w = ptr + ((size_t)(stripe * G + (tb >> 3)) * 32 + lane) * R;
 #pragma unroll
 				for (int r = 0; r < R; ++r) w[r] = ptr_word(st[r].x);
@@ -434,9 +508,9 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, AT_WAVE_AFFINE_MINB) at_wa
 		}
 		__syncwarp();
 
-		if (!last_stripe) {       // rest of the boundary row: columns (t_last-63, t_last-31], and t_last-31 >= l2
+		if (!last_stripe) {       // rest of the boundary row: columns (t_last-63, t_last-31], and t_last-31 >= l2 (banded: >= c1)
 			const int cidx = (int)t_last - 62 + lane;
-			if (cidx >= 1 && cidx <= (int)l2) __stcg(bnd_out + cidx, sm.stage[(uint32_t)cidx & 63u]);
+			if (cidx >= pub0 && cidx <= pub1) __stcg(bnd_out + cidx, sm.stage[(uint32_t)cidx & 63u]);
 			__syncwarp();
 			if (lane == 0) st_release(a.prog + job, l2);
 		}

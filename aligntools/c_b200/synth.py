@@ -177,6 +177,29 @@ def config5_edit(n_pairs=8, length=100000, stream=0):
                 q=q, q_off=qo, q_len=ql, t=t, t_off=to, t_len=tl, sites=None, site_off=None)
 
 
+def long_global(n_pairs=256, lo=10000, hi=20000, stream=0):
+    """Long global pairs (defaults m=1 u=-2 o=-5 e=-1): s1 random of lo..hi bp, s2 a mutated full-length copy of it (1 %
+    substitutions, 1 % insertions, 1 % deletions) -- a read against its reference window, or one assembly against
+    another.  The path keeps close to the diagonals between 0 and l2 - l1: global_corridor() gives a band around them."""
+    rng = _rng(6, stream)
+    reads, tgts = [], []
+    for _ in range(n_pairs):
+        s1 = rng.integers(0, 4, size=int(rng.integers(lo, hi + 1)), dtype=np.uint8)
+        reads.append(ACGT[s1])
+        tgts.append(ACGT[_mutate(rng, s1, 0.01, 0.01, 0.01)])
+    q, qo, ql = _ragged_batch(reads)
+    t, to, tl = _ragged_batch(tgts)
+    return dict(mode="global", params=dict(m=1, u=-2, o=-5, e=-1, j=-10, jump=False),
+                q=q, q_off=qo, q_len=ql, t=t, t_off=to, t_len=tl, sites=None, site_off=None)
+
+
+def global_corridor(q_len, t_len, w):
+    """Per-pair band (lo, hi) = (min(0, l2 - l1) - w, max(0, l2 - l1) + w) as int32 arrays: the diagonals between the
+    start and the end cell of a global alignment, widened by w on both sides."""
+    d = t_len.astype(np.int64) - q_len.astype(np.int64)
+    return (np.minimum(0, d) - w).astype(np.int32), (np.maximum(0, d) + w).astype(np.int32)
+
+
 def global_short(n_pairs=4096, l1=150, l2=150, stream=0):
     """Extra parity workload: global, l1 x l2 with ~8 % divergence."""
     rng = _rng(1, stream)

@@ -206,8 +206,19 @@ int  at_batch_align(at_handle *h, int mode, const at_params *p, const at_batch_i
  * Only K2's stripe windows are filled and only their pointers are stored, so a caller that knows where the overlap lies
  * (seed or minimizer chains) pays for the band, not for l1 x l2.  at_timing.cells counts the in-band cells; ptr_bytes is
  * what the banded pointer blocks took.  band == NULL is the unbanded path.  AT_E_ARG (at_last_error names the reason
- * and the pair): a band with a mode other than AT_OVERLAP, a NULL lo or hi, lo[p] > hi[p].  Results are sized and
- * fetched with at_batch_run / at_batch_sizes / at_batch_fetch as for any batch. */
+ * and the pair): a band with a mode other than AT_OVERLAP or AT_GLOBAL, a NULL lo or hi, lo[p] > hi[p], a global pair
+ * whose band misses its end diagonal (below).  Results are sized and fetched with at_batch_run / at_batch_sizes /
+ * at_batch_fetch as for any batch.
+ *
+ * Banded global alignment (mode AT_GLOBAL, affine gaps): a cell (i, j), 1 <= i <= l1, 1 <= j <= l2, whose diagonal
+ * j - i lies outside the band (clipped as above) is -inf in M, L and U and its pointer is never read.  Everything else
+ * is the reference's: row 0 and column 0 keep their border values, the end cell is (l1, l2) with max5's end state, and
+ * the traceback, then the flush of the rest of the target and of the read, follow trace_back_gla.  The band must hold
+ * the end diagonal, lo[p] <= l2 - l1 <= hi[p] (else AT_E_ARG; checked per pair after lo > hi): then every in-band cell
+ * is finite and a banded global result always exists.  Identity: when every cell (i >= 1, j >= 1) of the unbanded
+ * traceback path, end cell included, lies in the band, the banded result equals the unbanded one in every field.
+ * Banded global pairs all run on the wavefront kernel (K2), short ones included; at_timing.cells and ptr_bytes are as
+ * for overlap.  Local, fit and edit take no band. */
 typedef struct at_band {
 	const int32_t *lo;     /* [n_pairs] lowest diagonal d = j - i of the band  */
 	const int32_t *hi;     /* [n_pairs] highest diagonal                        */
