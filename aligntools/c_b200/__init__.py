@@ -21,6 +21,7 @@ LIB_PATH = os.environ.get("AT_LIB_PATH") or os.path.join(HERE, "libaligntools_b2
 
 MODES = {"global": 0, "local": 1, "fit": 2, "overlap": 3, "edit": 4}
 OUT_CIGAR, OUT_ALN = 1, 2
+OUT_EDIT_PATH = 4      # AT_OUT_EDIT_PATH: "edit" honours OUT_CIGAR / OUT_ALN (otherwise it is score-only)
 SEQ_BYTES, SEQ_2BIT = 0, 1
 RC_NAMES = {0: "AT_OK", -1: "AT_E_ARG", -2: "AT_E_CUDA", -3: "AT_E_NOMEM", -4: "AT_E_FITLEN",
             -5: "AT_E_NOSPACE", -6: "AT_E_RANGE", -7: "AT_E_UNDEF"}
@@ -186,6 +187,11 @@ def _mode(mode):
     return MODES[mode] if isinstance(mode, str) else int(mode)
 
 
+def _has_path(md, out_flags):
+    """Whether a run produces alignments: every mode but "edit", which needs OUT_EDIT_PATH as well."""
+    return md != 4 or bool(out_flags & OUT_EDIT_PATH)
+
+
 def pack_seqs(seqs):
     """list[bytes] -> (uint8 concat, uint64 offsets[n], uint32 lens[n])"""
     lens = np.fromiter((len(s) for s in seqs), dtype=np.uint32, count=len(seqs))
@@ -319,11 +325,12 @@ class Batch:
         out.score = res.score.ctypes.data
         out.end_i, out.end_j = res.end_i.ctypes.data, res.end_j.ctypes.data
         out.beg_i, out.beg_j = res.beg_i.ctypes.data, res.beg_j.ctypes.data
-        if self.out_flags & OUT_CIGAR and self.mode != 4:
+        path = _has_path(self.mode, self.out_flags)
+        if self.out_flags & OUT_CIGAR and path:
             res.cigar = np.zeros(no.value + 1, np.uint32)
             res.cigar_off = np.zeros(self.n + 1, np.uint64)
             out.cigar, out.cigar_cap, out.cigar_off = res.cigar.ctypes.data, no.value + 1, res.cigar_off.ctypes.data
-        if self.out_flags & OUT_ALN and self.mode != 4:
+        if self.out_flags & OUT_ALN and path:
             res.aln1 = np.zeros(nc.value + 1, np.uint8)
             res.aln2 = np.zeros(nc.value + 1, np.uint8)
             res.aln_off = np.zeros(self.n + 1, np.uint64)
@@ -384,7 +391,8 @@ class Aligner:
         o.score = res.score.ctypes.data
         o.end_i, o.end_j = res.end_i.ctypes.data, res.end_j.ctypes.data
         o.beg_i, o.beg_j = res.beg_i.ctypes.data, res.beg_j.ctypes.data
-        if out_flags & OUT_CIGAR and md != 4:
+        path = _has_path(md, out_flags)
+        if out_flags & OUT_CIGAR and path:
             if cigar_cap is None:
                 worst = int(q_len.astype(np.uint64).sum() + t_len.astype(np.uint64).sum())     # one op per column
                 cigar_cap = worst if worst <= (1 << 26) else 32 * n + 1024
@@ -393,7 +401,7 @@ class Aligner:
                 res.cigar = np.zeros(cap, np.uint32)
                 res.cigar_off = np.zeros(n + 1, np.uint64)
             o.cigar, o.cigar_cap, o.cigar_off = res.cigar.ctypes.data, res.cigar.size, res.cigar_off.ctypes.data
-        if out_flags & OUT_ALN and md != 4:
+        if out_flags & OUT_ALN and path:
             cap = int(aln_cap if aln_cap is not None else int(q_len.astype(np.uint64).sum() + t_len.astype(np.uint64).sum()) + 16)
             if res.aln1 is None or res.aln1.size < cap:
                 res.aln1 = np.zeros(cap, np.uint8)

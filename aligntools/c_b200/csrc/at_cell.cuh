@@ -299,4 +299,33 @@ AT_HD int lin_update(LinRow &st, const int d2, const int pw, const int a_up, con
 }
 AT_HD uint32_t lin_word(uint32_t x) { return AT_LIN_BIAS - x; }
 
+// ------------------------------------------------------------------------------------------------
+// Edit distance paths (AT_OUT_EDIT_PATH).  The pointer of a cell is min3's argmin (src/alignment.h:280-286) with the
+// first-strictly-smaller rule in argument order: LEFT 0, DIAGONAL 1, UP 2 -- the 2-bit code overlap's walker reads
+// (bit 1 UP, bit 0 DIAGONAL), so the cell-by-cell kernel stores it in overlap's layout.
+// Cell-by-cell: the candidates x4 with the code in the two low bits; one VIMNMX3 gives value (vt >> 2) and code (vt & 3).
+// ------------------------------------------------------------------------------------------------
+AT_HD int edit_min3_tagged(const int left, const int diag, const int up)      // M(i, j-1), M(i-1, j-1) + s, M(i-1, j)
+{
+	const int a = 4 * left + 4, b = 4 * diag + 1, c = 4 * up + 6;
+#ifdef __CUDA_ARCH__
+	return __vimin3_s32(a, b, c);
+#else
+	int v = a < b ? a : b; return v < c ? v : c;
+#endif
+}
+
+// Bit-parallel kernel (`edit -u 1`): the two pointer planes of one 32-row block column, from the vectors the column update
+// holds.  pv: vertical +1 deltas of column j-1 (before the update); ph / mh: horizontal +1 / -1 deltas of column j at the
+// block's rows (before the shift); eq: the PURE match vector of column j's symbol (without the carried-in hn).
+//   LEFT  iff M(i, j) = M(i, j-1) + 1, i.e. the horizontal delta is +1;
+//   DIAG  iff not LEFT and M(i, j) - M(i-1, j-1) = s(i, j).  That difference, d = dh(i, j) + dv(i, j-1), is 0 or 1;
+//         on a match s = 0 and d = 0 always, on a mismatch s = 1 and, with dh in {0, -1}, d = 1 iff dh = 0 and dv = +1.
+//   UP    otherwise.
+AT_HD void edit_bits_ptr(const uint32_t eq, const uint32_t pv, const uint32_t ph, const uint32_t mh, uint32_t &left, uint32_t &diag)
+{
+	left = ph;
+	diag = ~ph & (eq | (pv & ~mh));
+}
+
 }  // namespace atb2

@@ -188,7 +188,22 @@ struct RunWriter {
 // BANDED (overlap or global with a per-pair band): the pointer block has the banded layout (PtrView::seek_band / up_band)
 // and a walk that reaches a cell outside the band stops, as at row 0 -- cells on a finite path are in band.  Global's
 // flush after the walk is the unbanded one.
-template <bool BESIDE_FILL, bool BANDED = false>
+// EDIT (AT_OUT_EDIT_PATH; a.mode is ignored): the edit walk over the layout of the kernel that filled the shard --
+// EDIT_WALK_LIN: at_wave_linear<MODE_EDIT, .., PTR>, overlap's 2-bit codes (LEFT 0, DIAG 1, UP 2);
+// EDIT_WALK_BITS: at_wave_edit_bits<R, PTR>, a uint2 (LEFT, DIAG) of bit planes per block column (at_wavefront.cuh).
+// From (l1, l2) while i > 0 && j > 0: LEFT -> D, DIAG -> M, UP -> I; then global's flush.
+enum { EDIT_WALK_NONE = 0, EDIT_WALK_LIN = 1, EDIT_WALK_BITS = 2 };
+
+// word (uint2 index) of cell (i, j), i, j >= 1, in a bit-parallel edit block; `bit` receives the cell's bit
+__device__ __forceinline__ size_t edit_bits_index(uint32_t i, uint32_t j, uint32_t R, uint32_t G, uint32_t &bit)
+{
+	const uint32_t ri = i - 1, RPP = 1024u * R, s = ri / RPP, rem = ri - s * RPP;
+	const uint32_t lane = rem / (32u * R), r = (rem >> 5) - lane * R, t = j + 2u * lane + 1u;
+	bit = rem & 31u;
+	return ((((size_t)s * G + (t >> 4)) * R + r) * 16 + (t & 15u)) * 32 + lane;
+}
+
+template <bool BESIDE_FILL, bool BANDED = false, int EDIT = EDIT_WALK_NONE>
 __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 {
 	// Few long walks: ONE walker per warp (lane 0), so that a walk is not held back at every step by the
@@ -212,7 +227,33 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 	RunWriter w;
 	w.dst = a.scratch + a.scratch_off[k]; w.n_ops = w.n_cols = w.run = 0; w.op = 0;
 	uint32_t i = a.end_i[p], j = a.end_j[p], state = a.end_state[p], tick = 3;
-	if constexpr (BANDED) {
+	if constexpr (EDIT == EDIT_WALK_BITS) {
+		const uint32_t R = pv.R, G = (((l2 + 63u) | 15u) >> 4) + 1;
+		const uint2 *base = (const uint2 *)(a.ptr + a.ptr_off[k]);
+		while (i > 0 && j > 0) {
+			// the path mostly runs along the diagonal: pull the word AT_TB_PF_AHEAD cells up-left into L2
+			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u)) && i > AT_TB_PF_AHEAD && j > AT_TB_PF_AHEAD) {
+				uint32_t b2;
+				asm volatile("prefetch.global.L2 [%0];" :: "l"(base + edit_bits_index(i - AT_TB_PF_AHEAD, j - AT_TB_PF_AHEAD, R, G, b2)));
+			}
+			uint32_t b;
+			const uint2 pl = __ldg(base + edit_bits_index(i, j, R, G, b));
+			if ((pl.x >> b) & 1u)      { --j; w.col(CIG_D); }                 // LEFT
+			else if ((pl.y >> b) & 1u) { --i; --j; w.col(CIG_M); }            // DIAG
+			else                       { --i; w.col(CIG_I); }                 // UP
+		}
+	} else if constexpr (EDIT == EDIT_WALK_LIN) {
+		const uint32_t tl = steps_last(l2, 15);
+		pv.G = (tl >> 4) + 1; pv.GJ = 0;
+		if (i) pv.seek(i);
+		while (i > 0 && j > 0) {
+			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u))) pv.prefetch(i, j, 4);
+			const uint32_t c = pv.two(j);                                      // bit 1: UP, bit 0: DIAG, 0: LEFT
+			if (c & 2u)      { --i; pv.up(); w.col(CIG_I); }
+			else if (c & 1u) { --i; pv.up(); --j; w.col(CIG_M); }
+			else             { --j; w.col(CIG_D); }
+		}
+	} else if constexpr (BANDED) {
 		const bool ov = a.mode == MODE_OVERLAP;
 		pv.l1 = l1; pv.l2 = l2; pv.elo = a.band[p].x; pv.ehi = a.band[p].y; pv.wsh = ov ? 4u : 3u;
 		if (i && j) pv.seek_band(i);
@@ -272,7 +313,7 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 	}
 	}
 	a.beg_i[p] = i; a.beg_j[p] = j;
-	if (a.mode == MODE_GLOBAL) {                          // flush (:398-407): rest of the target, then rest of the read
+	if (EDIT || a.mode == MODE_GLOBAL) {                  // flush (:398-407): rest of the target, then rest of the read
 		while (j > 0) { --j; w.col(CIG_D); }
 		while (i > 0) { --i; w.col(CIG_I); }
 	}
@@ -282,6 +323,7 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 
 // One warp per pair: reverse the scratch ops into the dense CIGAR and, on request, replay them
 // forward over the two sequences to write the gapped strings r1 / r2 (coalesced).
+// Edit paths are launched with a.mode = MODE_GLOBAL: like global's, they start at (0, 0) after the flush.
 template <bool BESIDE_FILL>
 __global__ void __launch_bounds__(128) at_traceback_emit(const TraceArgs a)
 {

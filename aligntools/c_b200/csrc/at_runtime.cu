@@ -210,6 +210,7 @@ struct Shard {
 	DevBuf<uint8_t> d_symmap; DevBuf<uint32_t> d_symset;
 	bool prof = false; uint32_t syms = 0;      // query-profile variant of K1: the targets use <= 4 distinct bytes
 	bool bits = false;                         // bit-parallel edit distance: `-u 1` and reads of <= 8 distinct bytes
+	int bits_r = 1;                            // its 32-row blocks per lane (one launch per shard; fixes the edit-path pointer layout)
 	bool twobit = false;                       // the sequences stay 2-bit packed in HBM (AT_SEQ_2BIT input consumed directly by K1 / K2 / K3)
 	bool banded = false;                       // overlap / global with a per-pair band: h_band / d_band hold it clipped (at_band.h)
 	std::vector<int2> h_band;
@@ -260,16 +261,23 @@ struct at_batch {
 
 static inline uint32_t rclass_of(uint32_t l1) { uint32_t r = (l1 + 31) / 32; return r < 1 ? 1 : (r > (uint32_t)MAXR ? MAXR : r); }
 
+// pointer words of one pair's block; edit (AT_OUT_EDIT_PATH) on the cell-by-cell kernel stores overlap's layout
 static uint64_t ptr_words_of(int mode, bool jump, uint32_t l1, uint32_t l2)
 {
 	const uint32_t R = rclass_of(l1), RPP = 32 * R;
 	const uint64_t stripes = (l1 + RPP - 1) / RPP;
-	if (mode == AT_EDIT) return 0;
-	if (mode == AT_OVERLAP) { const uint32_t tl = (l2 + 31u) | 15u; return stripes * ((tl >> 4) + 1) * RPP; }
+	if (mode == AT_OVERLAP || mode == AT_EDIT) { const uint32_t tl = (l2 + 31u) | 15u; return stripes * ((tl >> 4) + 1) * RPP; }
 	const uint32_t tl = (l2 + 31u) | (jump ? 31u : 7u);
 	uint64_t w = stripes * ((tl >> 3) + 1) * RPP;
 	if (jump) w += stripes * ((tl >> 5) + 1) * RPP;
 	return w;
+}
+
+// the same for at_wave_edit_bits<R, true>: a uint2 per (32-row block, step), stripes of 1024 R rows, steps 0 .. (l2 + 63) | 15
+static uint64_t edit_bits_words(uint32_t R, uint32_t l1, uint32_t l2)
+{
+	const uint64_t stripes = (l1 + 1024u * R - 1) / (1024u * R), G = (((l2 + 63u) | 15u) >> 4) + 1;
+	return stripes * G * R * 1024u;
 }
 
 __global__ void at_unpack_2bit(const uint8_t *src, const uint64_t *src_off, const uint64_t *dst_off,
@@ -586,13 +594,28 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 	// banded pairs: the in-band cells, the pointer words of their stripe windows (at_band.h).  Banded global pairs all run
 	// on K2's affine kernel, short ones included: R = 8 rows per lane, 8-step pointer groups
 	const bool band_affine = s.banded && b->mode == AT_GLOBAL;
-	auto rclass = [&](uint32_t l1) -> uint32_t { return band_affine ? (uint32_t)MAXR : rclass_of(l1); };
-	auto pair_cells = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t { return s.banded ? band_cells(l1, l2, s.h_band[k].x, s.h_band[k].y) : (uint64_t)l1 * l2; };
-	auto pair_ptr_words = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t {
-		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass(l1), band_affine ? 3u : 4u) : ptr_words_of(b->mode, jump, l1, l2);
-	};
 	if ((rc = choose_variants(b, s, in, q_span))) return rc;
 	if (jump && (rc = build_jump_mask(b, s, in))) return rc;
+	// bit-parallel edit distance: r = 32-row blocks per lane, 1024*r rows per stripe.  One column step of a
+	// lane is a serial chain through its r blocks, so few long pairs want r = 1 (more stripes in flight);
+	// 4 blocks per lane amortise the per-step overhead once there are tasks for every resident warp.
+	// Decided for the whole shard before the arena is sized: an edit path's pointer layout depends on it.
+	s.bits_r = 1;
+	if (s.bits) {
+		const uint64_t warp_slots = (uint64_t)s.dev->sm_count * 8 * AT_WAVE_WARPS;
+		for (int r : {4, 2}) {
+			uint64_t tasks = 0;
+			for (uint32_t k = 0; k < n; ++k) tasks += (in->q_len[s.p0 + k] + 1024u * r - 1) / (1024u * r);
+			if (tasks >= 2 * warp_slots) { s.bits_r = r; break; }
+		}
+	}
+	const bool bits_path = s.bits && b->traceback;      // edit paths on at_wave_edit_bits: K3 reads R from the pair's class
+	auto rclass = [&](uint32_t l1) -> uint32_t { return band_affine ? (uint32_t)MAXR : bits_path ? (uint32_t)s.bits_r : rclass_of(l1); };
+	auto pair_cells = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t { return s.banded ? band_cells(l1, l2, s.h_band[k].x, s.h_band[k].y) : (uint64_t)l1 * l2; };
+	auto pair_ptr_words = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t {
+		if (bits_path) return edit_bits_words((uint32_t)s.bits_r, l1, l2);
+		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass(l1), band_affine ? 3u : 4u) : ptr_words_of(b->mode, jump, l1, l2);
+	};
 	mark("alphabet+jmask");
 	// a UNIFORM shard (every pair of the same shape, all on K1) needs no per-pair work on the host at all: see below
 	const uint32_t l1u = in->q_len[s.p0], l2u = in->t_len[s.p0];
@@ -759,18 +782,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		by_cells(wave_pairs);
 		c.h_bnd_off.assign(nc, 0);
 		c.bnd_elems = 0; c.prog_words = 0;
-		// bit-parallel edit distance: r = 32-row blocks per lane, 1024*r rows per stripe.  One column step of a
-		// lane is a serial chain through its r blocks, so few long pairs want r = 1 (more stripes in flight);
-		// 4 blocks per lane amortise the per-step overhead once there are tasks for every resident warp.
-		int bits_r = 1;
-		if (s.bits) {
-			const uint64_t warp_slots = (uint64_t)s.dev->sm_count * 8 * AT_WAVE_WARPS;
-			for (int r : {4, 2}) {
-				uint64_t tasks = 0;
-				for (uint32_t k : wave_pairs) tasks += (in->q_len[s.p0 + k] + 1024u * r - 1) / (1024u * r);
-				if (tasks >= 2 * warp_slots) { bits_r = r; break; }
-			}
-		}
+		const int bits_r = s.bits_r;
 		for (uint32_t k : wave_pairs) {
 			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
 			const int r = s.bits ? bits_r : (s.h_rclass[k] & 15);
@@ -1005,11 +1017,19 @@ extern "C" int at_plan_slices(const uint32_t *q_len, const uint32_t *t_len, uint
 	return AT_OK;
 }
 
+// whether a run walks the pointers: any output beyond the score; edit only when the path is asked for as well
+// (AT_OUT_EDIT_PATH: without it edit stays score-only, whatever else the flags say)
+static bool wants_traceback(int mode, uint32_t out_flags)
+{
+	if (!(out_flags & (AT_OUT_CIGAR | AT_OUT_ALN))) return false;
+	return mode != AT_EDIT || (out_flags & AT_OUT_EDIT_PATH);
+}
+
 static at_batch *new_batch(at_handle *h, int mode, const at_params *p, uint32_t out_flags, uint64_t n)
 {
 	at_batch *b = new at_batch();
 	b->h = h; b->mode = mode; b->prm = *p; b->out_flags = out_flags; b->n = n;
-	b->traceback = mode != AT_EDIT && (out_flags & (AT_OUT_CIGAR | AT_OUT_ALN));
+	b->traceback = wants_traceback(mode, out_flags);
 	return b;
 }
 
@@ -1106,12 +1126,12 @@ template <bool PROF> static fill2_fn affine_kernel_r(int kind, int R)
 	}
 }
 static fill2_fn affine_kernel(int kind, int R, bool prof) { return prof ? affine_kernel_r<true>(kind, R) : affine_kernel_r<false>(kind, R); }
-template <int MODE, bool PROF, bool BANDED = false> static wave_fn wave_linear_fn(int R)
+template <int MODE, bool PROF, bool BANDED = false, bool PTR = false> static wave_fn wave_linear_fn(int R)
 {
 	switch (R) {
-	case 1: return at_wave_linear<MODE, 1, PROF, BANDED>; case 2: return at_wave_linear<MODE, 2, PROF, BANDED>; case 3: return at_wave_linear<MODE, 3, PROF, BANDED>;
-	case 4: return at_wave_linear<MODE, 4, PROF, BANDED>; case 5: return at_wave_linear<MODE, 5, PROF, BANDED>; case 6: return at_wave_linear<MODE, 6, PROF, BANDED>;
-	case 7: return at_wave_linear<MODE, 7, PROF, BANDED>; default: return at_wave_linear<MODE, 8, PROF, BANDED>;
+	case 1: return at_wave_linear<MODE, 1, PROF, BANDED, PTR>; case 2: return at_wave_linear<MODE, 2, PROF, BANDED, PTR>; case 3: return at_wave_linear<MODE, 3, PROF, BANDED, PTR>;
+	case 4: return at_wave_linear<MODE, 4, PROF, BANDED, PTR>; case 5: return at_wave_linear<MODE, 5, PROF, BANDED, PTR>; case 6: return at_wave_linear<MODE, 6, PROF, BANDED, PTR>;
+	case 7: return at_wave_linear<MODE, 7, PROF, BANDED, PTR>; default: return at_wave_linear<MODE, 8, PROF, BANDED, PTR>;
 	}
 }
 // banded overlap / global (validate_band admits a band with AT_OVERLAP and AT_GLOBAL only)
@@ -1120,9 +1140,15 @@ static wave_fn wave_banded_kernel(int mode, int R, bool prof)
 	if (mode == AT_GLOBAL) return prof ? at_wave_affine<MODE_GLOBAL, false, true, true> : at_wave_affine<MODE_GLOBAL, false, false, true>;
 	return prof ? wave_linear_fn<MODE_OVERLAP, true, true>(R) : wave_linear_fn<MODE_OVERLAP, false, true>(R);
 }
-static wave_fn bits_kernel(int R) { return R == 1 ? at_wave_edit_bits<1> : (R == 2 ? at_wave_edit_bits<2> : at_wave_edit_bits<4>); }
-static wave_fn wave_kernel(int mode, bool jump, int R, bool prof)
+// edit paths (AT_OUT_EDIT_PATH): the PTR instantiations, which also store the pointers
+static wave_fn bits_kernel(int R, bool path)
 {
+	if (path) return R == 1 ? at_wave_edit_bits<1, true> : (R == 2 ? at_wave_edit_bits<2, true> : at_wave_edit_bits<4, true>);
+	return R == 1 ? at_wave_edit_bits<1> : (R == 2 ? at_wave_edit_bits<2> : at_wave_edit_bits<4>);
+}
+static wave_fn wave_kernel(int mode, bool jump, int R, bool prof, bool path)
+{
+	if (mode == AT_EDIT && path) return prof ? wave_linear_fn<MODE_EDIT, true, false, true>(R) : wave_linear_fn<MODE_EDIT, false, false, true>(R);
 	switch (mode) {
 	case AT_GLOBAL: return prof ? at_wave_affine<MODE_GLOBAL, false, true> : at_wave_affine<MODE_GLOBAL, false, false>;
 	case AT_LOCAL: return prof ? at_wave_affine<MODE_LOCAL, false, true> : at_wave_affine<MODE_LOCAL, false, false>;
@@ -1169,7 +1195,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 		if (first) { CU(h, cudaEventRecord(e_first, st)); first = false; }
 		for (size_t li = 0; li < c.launches.size(); ++li) {
 			Launch &l = c.launches[li];
-			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r) : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(b->mode, l.r, s.prof) : (const void *)wave_kernel(b->mode, jump, l.r, s.prof))
+			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r, b->traceback) : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(b->mode, l.r, s.prof) : (const void *)wave_kernel(b->mode, jump, l.r, s.prof, b->traceback))
 			                                   : (const void *)affine_kernel(l.kind == LK_PACKED ? (b->mode == AT_LOCAL ? 4 : b->mode == AT_GLOBAL ? 5 : 6) : (b->mode == AT_FIT ? (jump ? 3 : 2) : b->mode), l.r, s.prof);
 			const int warps = l.kind >= LK_WAVE ? AT_WAVE_WARPS : AT_FILL_WARPS;
 			const size_t dyn_smem = l.kind >= LK_WAVE ? 0 : fill_smem_bytes(l.r, l.kind == LK_PACKED, s.prof);
@@ -1235,13 +1261,16 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 			ta.ops_off = c.d_ops_off.p; ta.cols_off = c.d_cols_off.p;
 			ta.scratch = s.d_scratch.p; ta.scratch_off = c.d_scratch_off.p;
 			ta.cigar = nullptr; ta.aln1 = nullptr; ta.aln2 = nullptr;
-			ta.mode = b->mode; ta.jump = jump ? 1 : 0; ta.twobit = s.twobit ? 1 : 0;
+			ta.mode = b->mode == AT_EDIT ? MODE_GLOBAL : b->mode;      // an edit path is emitted as global's: from (0, 0)
+			ta.jump = jump ? 1 : 0; ta.twobit = s.twobit ? 1 : 0;
 			ta.band = s.banded ? s.d_band.p : nullptr;
 			// few long walks: one walker per warp, prefetching ahead; with many walks, or short ones (a few hundred
 			// steps: nothing to prefetch far ahead of), the chase is throughput-bound and the prefetches only add traffic
 			ta.lookahead = nc < 32768u && c.scratch_words / nc >= 2048 ? 1 : 0;
 			const int walk_blocks = ta.lookahead ? (int)(((uint64_t)nc * 32 + 127) / 128) : (int)((nc + 127) / 128);   // one walker per warp | per thread
-			if (s.banded) at_traceback_walk<false, true><<<walk_blocks, 128, 0, st>>>(ta);
+			if (b->mode == AT_EDIT && s.bits) at_traceback_walk<false, false, EDIT_WALK_BITS><<<walk_blocks, 128, 0, st>>>(ta);
+			else if (b->mode == AT_EDIT) at_traceback_walk<false, false, EDIT_WALK_LIN><<<walk_blocks, 128, 0, st>>>(ta);
+			else if (s.banded) at_traceback_walk<false, true><<<walk_blocks, 128, 0, st>>>(ta);
 			else if (s.workspace && tb_overlap) at_traceback_walk<true><<<walk_blocks, 128, 0, st>>>(ta);
 			else at_traceback_walk<false><<<walk_blocks, 128, 0, st>>>(ta);
 			CU(h, cudaGetLastError());

@@ -557,7 +557,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 
 // =====================================================================================
 // Single-plane kernel: overlap (max-plus, linear gap, 2-bit pointers) and edit distance
-// (min-plus, unit gaps, score only), int32 lanes, R = 1..8 rows per lane.
+// (min-plus, unit gaps; score only unless PTR, below), int32 lanes, R = 1..8 rows per lane.
 //
 // Overlap runs lin_update() of at_cell.cuh: scores x4, every cell carries A = 4*M + 4*o, the argmax of the one
 // VIMNMX3 rides in the two spare bits (LEFT 2, DIAGONAL 1, RIGHT 0: the reference's order with
@@ -579,11 +579,17 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 // predecessor when it has a window; otherwise the row above is -inf, as row 0 is.  Pointer words are stored relative to
 // t0 at the stripe's offset in the pair's block.  A queued stripe without a window is the pair's last one: it only
 // writes the end cell M[l1][0] = 0.
-template <int MODE, int R, bool PROF, bool BANDED = false>
+//
+// PTR (edit only, AT_OUT_EDIT_PATH): the cell is edit_min3_tagged() of at_cell.cuh -- the three candidates x4 with min3's
+// argmin code in the low bits (LEFT 0, DIAGONAL 1, UP 2), one VIMNMX3 -- and the codes are stored in overlap's layout
+// (2 bits, 16 steps per word, code = the tag itself), so K3 walks them with overlap's reader.
+template <int MODE, int R, bool PROF, bool BANDED = false, bool PTR = false>
 __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveArgs a)
 {
+	static_assert(!PTR || (MODE == MODE_EDIT && !BANDED), "PTR: the edit kernel's pointers (overlap stores its own)");
 	constexpr int RPP = 32 * R;
 	constexpr bool OV = MODE == MODE_OVERLAP;
+	constexpr bool STORE = OV || PTR;      // the kernel writes 2-bit pointer words
 	constexpr int UNR = OV ? AT_WAVE_UNROLL_OVERLAP : AT_WAVE_UNROLL_EDIT;
 	constexpr int LS = prof_lane_stride(R);
 	struct __align__(16) Smem { int prof[PROF ? 4 : 1][PROF ? 32 : 1][PROF ? LS : 2]; WaveRing<false> rg; int cring[64]; int stage[64]; };
@@ -602,7 +608,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 	const int pw_match = OV ? S * (a.m - a.o) - 1 : 0;               // substitution term of a match (overlap: carried value -> tagged diagonal candidate)
 	const uint32_t pen = OV ? (uint32_t)(S * (a.m >= a.u ? a.m - a.u : a.u - a.m)) : (uint32_t)(a.u >= 0 ? a.u : -a.u);
 	const int nsg = OV ? (a.m >= a.u ? -1 : 1) : (a.u >= 0 ? 1 : -1);
-	const bool want_ptr = OV && a.want_ptr != 0;
+	const bool want_ptr = STORE && a.want_ptr != 0;
 	int nz = lane ? 1 : 0;                                            // lane 0 takes the row above the stripe instead of a neighbour
 	asm volatile("" : "+r"(nz));                                      // opaque: keep x * nz + b a multiply-add (FMA pipe), not a SEL
 
@@ -622,7 +628,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 		const uint32_t sh = twobit ? 4u * sh16 : sh16;                        // ring position of target index 0
 		const uint32_t tile_wait = twobit ? 192u : 224u;                      // step (mod 256) at which the next tile must have landed: lane 0 is up to sh + 1 columns ahead of the step counter
 		uint32_t n_tiles = (l2 + sh + 255u) >> 8;
-		uint32_t *__restrict__ ptr = OV ? a.ptr + a.ptr_off[p - a.pair_base] : nullptr;
+		uint32_t *__restrict__ ptr = STORE ? a.ptr + a.ptr_off[p - a.pair_base] : nullptr;
 		const uint32_t G = (((l2 + 31u) | 15u) >> 4) + 1;                 // pointer-block geometry shared with K3
 		uint32_t t_last = (l2 + 31u) | 31u;
 		const uint32_t n_stripes = (l1 + RPP - 1) / RPP;
@@ -742,6 +748,12 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 						v = lin_update(stl[r], D, sub, Vup, gap, dn);
 						D = dn;
 						if (MSK && (uint32_t)(j - (int)row0 - 1 - r - elo) > (uint32_t)(ehi - elo)) { v = AT_NEGL; stl[r].a2 = AT_NEGL + 2; }   // d = j - i out of band
+					} else if (PTR) {
+						const int vt = edit_min3_tagged(Vl[r], D + sub, Vup);     // min3 (:280-286) + its argmin code
+						D = Vl[r];
+						v = vt >> 2;
+						stl[r].x = stl[r].x * 4u + (uint32_t)(vt & 3);
+						Vl[r] = v;
 					} else {
 						const int diag = D + sub;
 						D = Vl[r];
@@ -757,7 +769,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 					if (OV) { if (j < (int)l2 && rowV > capV) { capV = rowV; capJ = j; } }   // column l2 excluded (:955)
 					else if (j == (int)l2) capV = rowV;
 				}
-			} else if (OV) {
+			} else if (STORE) {
 #pragma unroll
 				for (int r = 0; r < R; ++r) stl[r].x *= 4u;
 			}
@@ -823,7 +835,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 			} else if (want_ptr && (tb >> 4) < G) {
 				uint32_t *w = ptr + ((size_t)(stripe * G + (tb >> 4)) * 32 + lane) * R;
 #pragma unroll
-				for (int r = 0; r < R; ++r) w[r] = lin_word(stl[r].x);
+				for (int r = 0; r < R; ++r) w[r] = PTR ? stl[r].x : lin_word(stl[r].x);      // edit: the code is the tag
 			}
 		}
 		__syncwarp();
@@ -858,8 +870,15 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 // zeroed by the host before every run.  (The release/acquire protocol of the other kernels cost a
 // membar per 32 columns -- 22 % of this kernel's stall samples when it was first written that way.)
 //   score = M[l1][l2] = l1 + sum over j of the horizontal difference at row l1.     SURVEY.md 8(f) #4.
+//
+// PTR (AT_OUT_EDIT_PATH): every block column also yields min3's argmin for its 32 cells as two bit planes (edit_bits_ptr,
+// at_cell.cuh: LEFT = Ph, DIAG = ~Ph & (Eq | (Pv & ~Mh)), UP = neither), stored as one uint2 (LEFT, DIAG) per
+// (block, column) in SKEWED coordinates -- step t = j + 2 lane + 1, as the lanes run:
+//     uint2 index = (((stripe * G + t / 16) * R + r) * 16 + t % 16) * 32 + lane,    G = ((l2 + 63) | 15) / 16 + 1,
+// so one store per block column writes 256 contiguous bytes across the warp (full sectors, no staging) and a pair's block
+// is 2 bits per cell of its stripes (rows rounded up to 1024 R).  K3's bit-parallel walker reads it.
 // =====================================================================================
-template <int R>
+template <int R, bool PTR = false>
 __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const WaveArgs a)
 {
 	constexpr int RPP = 1024 * R;                 // rows per stripe
@@ -899,6 +918,8 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 		const uint64_t tag_in = (uint64_t)stripe << 32;                    // the predecessor's tag: (stripe - 1) + 1
 		const uint64_t tag_out = (uint64_t)(stripe + 1u) << 32;
 		const uint32_t row0 = stripe * RPP + lane * 32u * R;
+		uint2 *__restrict__ pp = nullptr;                                  // PTR: this lane's words of the stripe
+		if constexpr (PTR) pp = (uint2 *)(a.ptr + a.ptr_off[p - a.pair_base]) + (size_t)stripe * ((((l2 + 63u) | 15u) >> 4) + 1) * R * 512 + lane;
 
 		__syncwarp();
 		if (n_tiles > 0) ring_issue<false>(sm.rg, tbase16, nullptr, 0, lane, twobit);
@@ -953,6 +974,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 		// critical path -- the chain per step is the column update alone.  inA / inB: the neighbour's outputs
 		// received at the end of the previous two steps (inA is the one due now).
 		uint32_t sP = 0, sN = 0, inA_p = 0, inA_n = 0, inB_p = 0, inB_n = 0;
+		uint32_t lft[R], dg[R];                                            // PTR: pointer planes of the column just computed
 		// one column of the lane's R blocks; eq[] = match vectors of the column's symbol, (hp, hn) = horizontal
 		// difference entering the first block, replaced by the one leaving the last block
 		auto column = [&](const uint32_t (&eq)[R], uint32_t &hp, uint32_t &hn) {
@@ -964,6 +986,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 				const uint32_t Xh = (((Eq & Pv[r]) + Pv[r]) ^ Pv[r]) | Eq;
 				uint32_t Ph = Mv[r] | ~(Xh | Pv[r]);
 				uint32_t Mh = Pv[r] & Xh;
+				if constexpr (PTR) edit_bits_ptr(eq[r], Pv[r], Ph, Mh, lft[r], dg[r]);
 				if (r == own_r) dist += (int)((Ph >> own_b) & 1u) - (int)((Mh >> own_b) & 1u);
 				const uint32_t op = Ph >> 31, on = Mh >> 31;
 				Ph = (Ph << 1) | hp;
@@ -976,6 +999,11 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 		auto pass_on = [&]() {                                             // end of a step: send this step's output down, age the queue
 			inA_p = inB_p; inA_n = inB_n;
 			inB_p = __shfl_up_sync(0xffffffffu, sP, 1); inB_n = __shfl_up_sync(0xffffffffu, sN, 1);
+		};
+		auto store_ptr = [&](const uint32_t t) {                          // PTR: the planes of step t's column
+			uint2 *w = pp + ((size_t)(t >> 4) * R * 16 + (t & 15u)) * 32;
+#pragma unroll
+			for (int r = 0; r < R; ++r) w[r * 512] = make_uint2(lft[r], dg[r]);
 		};
 		auto step = [&](const uint32_t t) {                                // any step: range-checked
 			const int j = (int)t - 2 * lane - 1;
@@ -992,6 +1020,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 #pragma unroll
 				for (int r = 0; r < R; ++r) eq[r] = sm.eq[c][lane][r];
 				column(eq, hp, hn);
+				if constexpr (PTR) store_ptr(t);
 				sP = hp; sN = hn;
 				if (lane == 31 && !last_stripe) {
 					out_bits |= (hp | (hn << 1)) << (2u * (((uint32_t)j - 1u) & 15u));
@@ -1029,6 +1058,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 				uint32_t hp = inA_p, hn = inA_n;
 				if (first) { hp = (tops >> (2 * k)) & 1u; hn = (tops >> (2 * k + 1)) & 1u; }
 				column(eq[k], hp, hn);
+				if constexpr (PTR) store_ptr(tb + k);
 				sP = hp; sN = hn;
 				packed |= (hp | (hn << 1)) << (2 * k);
 				pass_on();

@@ -134,8 +134,27 @@ typedef struct at_batch_input {
 enum at_out_flags {
 	AT_OUT_SCORE = 0,        /* score, end cell and end state are always produced           */
 	AT_OUT_CIGAR = 1u << 0,  /* run traceback, emit run-length ops                          */
-	AT_OUT_ALN   = 1u << 1   /* run traceback, emit the two gapped strings (r1, r2)         */
+	AT_OUT_ALN   = 1u << 1,  /* run traceback, emit the two gapped strings (r1, r2)         */
+	AT_OUT_EDIT_PATH = 1u << 2   /* AT_EDIT: honour AT_OUT_CIGAR / AT_OUT_ALN (below); other
+	                                modes ignore it                                           */
 };
+
+/* Edit paths.  AT_EDIT runs its traceback only when AT_OUT_EDIT_PATH is set together with AT_OUT_CIGAR and/or AT_OUT_ALN,
+ * which then select the outputs as for the other modes.  Without AT_OUT_EDIT_PATH an edit batch is score-only whatever the
+ * other flags say: no pointers are stored (at_timing.ptr_bytes 0) and cigar_off / aln_off come back all zero -- so callers
+ * that pass CIGAR | ALN for every mode do not start writing 2 bits per cell (2.5 GB for a 100 kbp x 100 kbp pair).
+ * The path is the traceback edit_dist (src/alignment.h:291-315) would have, with the conventions of the other modes:
+ *   - the recurrence and borders are unchanged: M[i][0] = i, M[0][j] = j,
+ *     M[i][j] = min3(M[i][j-1] + 1, M[i-1][j-1] + (s1[i-1] == s2[j-1] ? 0 : u), M[i-1][j] + 1);
+ *   - a cell's pointer is min3's argmin, first strictly smaller in argument order: LEFT wins ties, then DIAG, then UP;
+ *   - the walk starts at (l1, l2) and, reading the pointer of the cell before each move, runs while i > 0 && j > 0:
+ *     LEFT emits (-, s2[--j]) as AT_CIG_D, DIAG (s1[--i], s2[--j]) as AT_CIG_M, UP (s1[--i], -) as AT_CIG_I;
+ *   - then the rest of the target (AT_CIG_D) and the rest of the read (AT_CIG_I) are flushed, as global's traceback does.
+ * end = (l1, l2), end state MID; beg_i / beg_j = the cell where the walk stopped, before the flush; the score is unchanged.
+ * The path's cost -- 0 per equal M column, u per unequal one, 1 per I or D column -- equals the score for every u.
+ * The bit-parallel kernel (u = 1, reads of <= 8 distinct bytes) and the cell-by-cell one give identical results.
+ * at_timing.ptr_bytes reports the pointers (about l1 * l2 / 4 bytes per pair); they are chunked by the pointer arena as
+ * for the other modes. */
 
 /* CIGAR op = (run_length << 4) | code; columns left to right (SURVEY.md A.8) */
 enum at_cigar_op { AT_CIG_M = 0 /* (x,y) */, AT_CIG_I = 1 /* (x,-) LOW */,
