@@ -18,7 +18,7 @@
 //     Jk = Jt & ~1); these CLEAN values are what the next cells consume;
 //   * the pointer nibble of a cell is a LINEAR function of (tagged - clean):
 //         nibble = 13 + (Mk + Lk + 4 Uk) - (Mt + Lt + 4 Ut)
-//       = (3 - tag of M) + 4 [L opened] + 8 [U extended]      (K3's layout, at_kernels.cuh header)
+//       = (3 - tag of M) + 4 [L opened] + 8 [U extended]      (K3's layout, at_ptr_layout.h)
 //     so the kernels keep one accumulator per row, X = 16 X + (Mk + Lk + 4 Uk) - (Mt + Lt + 4 Ut) -- six
 //     adds / multiply-adds on the FMA pipe, no shifts / masks / selects on the ALU pipe -- and store
 //     X + 0xDDDDDDDD once per pointer word.  All of it is arithmetic mod 2^32, also for packed s16x2 lanes:

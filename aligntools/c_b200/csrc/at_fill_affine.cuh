@@ -84,7 +84,8 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 	static_assert(!PACKED || !JUMP, "packed lanes: no jump state");
 	constexpr bool LOCAL = MODE == MODE_LOCAL;
 	constexpr uint32_t SPW = V::STEPS_PER_WORD;
-	constexpr int RPP = 32 * R;
+	constexpr uint32_t SH = PACKED ? PTR_SH_PACKED : PTR_SH_NIB;           // pointer layout (at_ptr_layout.h)
+	static_assert(SPW == 1u << SH, "a lane assembles one pointer word per SPW steps");
 	constexpr int LS = k1_lane_stride(R), NC = prof_combs(PACKED);
 	constexpr uint32_t COMB_BYTES = 32u * LS * 4u;             // one comb's slice of the profile
 	constexpr size_t WARP_BYTES = fill_smem_bytes(R, PACKED, PROF) / AT_FILL_WARPS;
@@ -123,9 +124,9 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 		const uint8_t *__restrict__ tA = a.t + a.t_off[pA], *__restrict__ tB = a.t + a.t_off[pB];
 		const uint8_t *__restrict__ jm = JUMP ? a.jmask + a.j_off[pA] : nullptr;
 		uint32_t *__restrict__ ptr = a.ptr + a.ptr_off[pA - a.pair_base];
-		const uint32_t t_last = (l2 + 31u) | (JUMP ? 31u : (SPW - 1u));
-		const uint32_t G = t_last / SPW + 1;
-		uint32_t *__restrict__ ptrJ = ptr + (size_t)G * RPP;
+		const uint32_t t_last = ptr_last_step(l2, SH, JUMP);                  // also the last step the warp runs
+		const uint32_t G = ptr_groups(t_last, SH);
+		uint32_t *__restrict__ ptrJ = ptr_plane(ptr, 1u, G, R);
 
 		// ring[(j-1) & 511]: packed (tA << 8) | (tB << 24); int32 (tA << 16) | blacklist bit;
 		// PROF: byte offset of the column's comb in the profile | blacklist bit
@@ -381,12 +382,12 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 				for (uint32_t k = 0; k < SPW; ++k) step(tb + k, true, nullptr, (PACKED && k == 0) ? 0u : 16u, 2u, false);
 			}
 			if (want_ptr) {
-				uint32_t *w = ptr + ((size_t)(tb / SPW) * 32 + lane) * R;
+				uint32_t *w = ptr_at(ptr, 0u, 0u, tb >> SH, lane, R);          // one stripe
 #pragma unroll
 				for (int r = 0; r < R; ++r) w[r] = ptr_word(st[r].x);
 			}
 			if (JUMP && want_ptr && ((tb + SPW - 1u) & 31u) == 31u) {
-				uint32_t *w = ptrJ + ((size_t)(tb >> 5) * 32 + lane) * R;
+				uint32_t *w = ptr_at(ptrJ, 0u, 0u, tb >> PTR_SH_JUMP, lane, R);
 #pragma unroll
 				for (int r = 0; r < R; ++r) w[r] = jump_word(st[r].xj);
 			}

@@ -24,19 +24,12 @@
 // parks it in a boundary row that lane 0 reads back on the next stripe (reads longer than
 // 32*R rows).  Per-row state (M+o, U, H, code, J of column j-1) stays in registers.
 //
-// Traceback pointers: one nibble per cell, bits 0-1 = pointerM (0 LOW, 1 MID, 2 UPP,
-// 3 HOME|JUMP), bit 2 = pointerL is MID (gap opened), bit 3 = pointerU is UPP (gap
-// extended); fit+jump adds a 1-bit plane (pointerJ is JUMP).  Reference planes:
-// src/alignment.h:44-47, values :27-34.  Nibbles of 8 consecutive steps of one row are
-// packed into a 32-bit word (earliest step in the top nibble) and stored as
-//   word[((stripe*G + step/8)*32 + lane)*R + r]
-// i.e. in SKEWED coordinates (step = column + lane) with the R words of a lane's 8-step block
-// contiguous: a warp flush writes one dense 128*R-byte run, and a diagonal traceback move
-// (row-1, column-1) stays inside the same 32-byte sector most of the time.
+// Traceback pointers: at_ptr_layout.h defines every pointer-block layout the fills store and K3 reads.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "at_cell.cuh"      // Lanes<>, cell_update(), AT_NEG: the cell arithmetic shared by K1 and K2
+#include "at_ptr_layout.h"  // pointer-block layouts shared by the runtime, K1, K2 and K3
 #include "at_band.h"        // banded overlap / global: stripe windows and pointer layout shared by the runtime, K2 and K3
 
 // traceback walker's look-ahead: how far ahead (steps) and how often (every PERIOD-th step, a power of two) it prefetches
@@ -53,8 +46,6 @@ enum { MODE_GLOBAL = 0, MODE_LOCAL = 1, MODE_FIT = 2, MODE_OVERLAP = 3, MODE_EDI
 enum { ST_LOW = 0, ST_MID = 1, ST_UPP = 2, ST_JUMP = 3 };   // also the 2-bit pointerM codes
 enum { CIG_M = 0, CIG_I = 1, CIG_D = 2, CIG_N = 3 };
 
-__device__ __forceinline__ uint32_t steps_last(uint32_t l2, int align_mask) { return (l2 + 31u) | (uint32_t)align_mask; }
-
 }  // namespace atb2
 #include "at_fill_affine.cuh"
 #include "at_wavefront.cuh"
@@ -70,8 +61,7 @@ struct TraceArgs {
 	const uint8_t  *q;  const uint64_t *q_off;  const uint32_t *q_len;
 	const uint8_t  *t;  const uint64_t *t_off;  const uint32_t *t_len;
 	const uint32_t *ptr; const uint64_t *ptr_off;
-	const uint8_t  *rclass;    // [pair] bits 0-3: rows-per-lane R the fill used; bits 4-5: 0 = int32 layout,
-	                           //        1 / 2 = packed s16x2 layout, pair in the low / high half
+	const uint8_t  *rclass;    // [pair] layout class (at_ptr_layout.h: ptr_class): the fill's R and packed half
 	uint32_t        pair_base, n_pairs;   // chunk
 	const uint32_t *end_i, *end_j; const uint8_t *end_state;
 	uint32_t       *beg_i, *beg_j;
@@ -87,8 +77,8 @@ struct TraceArgs {
 	const int2     *band;                  // banded walker: [pair] clipped band (lo, hi) on j - i (at_band.h)
 };
 
-// Cursor over a pair's pointer block (layout: at_kernels.cuh header).  The word of cell (i, j) is
-//   ptr[rowA(i) + ((j + lane(i)) >> SH) * RPP],   rowA(i) = stripe * G * RPP + lane * R + r,
+// Cursor over a pair's pointer block (layout: at_ptr_layout.h).  The word of cell (i, j) is
+//   ptr[rowA(i) + ((j + lane(i)) >> SH) * RPP],   rowA(i) = PtrRow::base,
 // with stripe / lane / r the position of row i-1 in the fill's geometry.  A traceback only ever moves
 // to row i-1, so rowA is kept incrementally (it just decrements, except across a stripe) instead of
 // being re-derived with two integer divisions per visited cell.
@@ -98,10 +88,10 @@ struct PtrView {
 	uint32_t r, lane;            // position of row i-1: row within the lane, lane within the stripe
 	size_t rowA, rowJ;           // word offsets of row i-1 in the nibble / 2-bit block and in the jump-bit plane
 	__device__ __forceinline__ void seek(uint32_t i) {            // i >= 1
-		const uint32_t ri = i - 1, stripe = ri / RPP, rem = ri - stripe * RPP;
-		lane = rem / R; r = rem - lane * R;
-		rowA = (size_t)stripe * G * RPP + (size_t)lane * R + r;
-		rowJ = (size_t)stripe * GJ * RPP + (size_t)lane * R + r;
+		const PtrRow w = ptr_row(i, R);
+		lane = w.lane; r = w.r;
+		rowA = w.base(G, R);
+		rowJ = w.base(GJ, R);
 	}
 	__device__ __forceinline__ void up() {                        // row i-1 -> row i-2 (no-op bookkeeping when leaving row 0)
 		if (r) { --r; --rowA; --rowJ; return; }
@@ -126,16 +116,16 @@ struct PtrView {
 	__device__ __forceinline__ uint32_t nib(uint32_t j) const {
 		const uint32_t t = j + lane;
 		if (half) {   // packed s16x2: 4 steps x 2 pairs per word, single stripe
-			const uint32_t w = __ldg(ptr + rowA + (size_t)(t >> 2) * RPP);
-			return (w >> (16 * (half - 1) + 4 * (3 - (t & 3)))) & 15u;
+			const uint32_t w = __ldg(ptr + rowA + (size_t)(t >> PTR_SH_PACKED) * RPP);
+			return (w >> (16 * (half - 1) + ptr_shift(t, PTR_SH_PACKED, 4))) & 15u;
 		}
-		const uint32_t w = __ldg(ptr + rowA + (size_t)(t >> 3) * RPP);
-		return (w >> (4 * (7 - (t & 7)))) & 15u;
+		const uint32_t w = __ldg(ptr + rowA + (size_t)(t >> PTR_SH_NIB) * RPP);
+		return (w >> ptr_shift(t, PTR_SH_NIB, 4)) & 15u;
 	}
 	__device__ __forceinline__ uint32_t jbit(uint32_t j) const {
 		const uint32_t t = j + lane;
-		const uint32_t w = __ldg(ptrJ + rowJ + (size_t)(t >> 5) * RPP);
-		return (w >> (31 - (t & 31))) & 1u;
+		const uint32_t w = __ldg(ptrJ + rowJ + (size_t)(t >> PTR_SH_JUMP) * RPP);
+		return (w >> ptr_shift(t, PTR_SH_JUMP, 1)) & 1u;
 	}
 	// Banded pairs (at_band.h): stripe s's words start at off(s) and count groups of 2^wsh steps (overlap 16, global 8) from
 	// the stripe's first step t0, so rowA folds in - (t0 >> wsh) * RPP and two() / nib() stay as they are.  Crossing to the
@@ -169,8 +159,8 @@ struct PtrView {
 	}
 	__device__ __forceinline__ uint32_t two(uint32_t j) const {   // overlap: 2 bits, 16 steps per word
 		const uint32_t t = j + lane;
-		const uint32_t w = __ldg(ptr + rowA + (size_t)(t >> 4) * RPP);
-		return (w >> (2 * (15 - (t & 15)))) & 3u;
+		const uint32_t w = __ldg(ptr + rowA + (size_t)(t >> PTR_SH_2BIT) * RPP);
+		return (w >> ptr_shift(t, PTR_SH_2BIT, 2)) & 3u;
 	}
 };
 
@@ -190,18 +180,9 @@ struct RunWriter {
 // flush after the walk is the unbanded one.
 // EDIT (AT_OUT_EDIT_PATH; a.mode is ignored): the edit walk over the layout of the kernel that filled the shard --
 // EDIT_WALK_LIN: at_wave_linear<MODE_EDIT, .., PTR>, overlap's 2-bit codes (LEFT 0, DIAG 1, UP 2);
-// EDIT_WALK_BITS: at_wave_edit_bits<R, PTR>, a uint2 (LEFT, DIAG) of bit planes per block column (at_wavefront.cuh).
+// EDIT_WALK_BITS: at_wave_edit_bits<R, PTR>, a uint2 (LEFT, DIAG) of bit planes per block column (at_ptr_layout.h).
 // From (l1, l2) while i > 0 && j > 0: LEFT -> D, DIAG -> M, UP -> I; then global's flush.
 enum { EDIT_WALK_NONE = 0, EDIT_WALK_LIN = 1, EDIT_WALK_BITS = 2 };
-
-// word (uint2 index) of cell (i, j), i, j >= 1, in a bit-parallel edit block; `bit` receives the cell's bit
-__device__ __forceinline__ size_t edit_bits_index(uint32_t i, uint32_t j, uint32_t R, uint32_t G, uint32_t &bit)
-{
-	const uint32_t ri = i - 1, RPP = 1024u * R, s = ri / RPP, rem = ri - s * RPP;
-	const uint32_t lane = rem / (32u * R), r = (rem >> 5) - lane * R, t = j + 2u * lane + 1u;
-	bit = rem & 31u;
-	return ((((size_t)s * G + (t >> 4)) * R + r) * 16 + (t & 15u)) * 32 + lane;
-}
 
 template <bool BESIDE_FILL, bool BANDED = false, int EDIT = EDIT_WALK_NONE>
 __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
@@ -216,19 +197,19 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 	const uint32_t p = a.pair_base + k;
 	const uint32_t l1 = a.q_len[p], l2 = a.t_len[p];
 	PtrView pv;
-	pv.R = a.rclass[p] & 15u; pv.RPP = 32 * pv.R; pv.half = (a.rclass[p] >> 4) & 3u;
-	const uint32_t n_stripes = (l1 + pv.RPP - 1) / pv.RPP;
+	pv.R = ptr_class_r(a.rclass[p]); pv.RPP = 32 * pv.R; pv.half = ptr_class_half(a.rclass[p]);
+	const uint32_t n_stripes = ptr_stripes(l1, pv.R);
 	const bool jump = a.jump != 0;
-	if (a.mode == MODE_OVERLAP) { const uint32_t tl = steps_last(l2, 15); pv.G = (tl >> 4) + 1; pv.GJ = 0; }
-	else if (pv.half) { const uint32_t tl = steps_last(l2, 3); pv.G = (tl >> 2) + 1; pv.GJ = 0; }
-	else { const uint32_t tl = steps_last(l2, jump ? 31 : 7); pv.G = (tl >> 3) + 1; pv.GJ = (tl >> 5) + 1; }
+	if (a.mode == MODE_OVERLAP) { pv.G = ptr_groups(ptr_last_step(l2, PTR_SH_2BIT), PTR_SH_2BIT); pv.GJ = 0; }
+	else if (pv.half) { pv.G = ptr_groups(ptr_last_step(l2, PTR_SH_PACKED), PTR_SH_PACKED); pv.GJ = 0; }
+	else { const uint32_t tl = ptr_last_step(l2, PTR_SH_NIB, jump); pv.G = ptr_groups(tl, PTR_SH_NIB); pv.GJ = ptr_groups(tl, PTR_SH_JUMP); }
 	pv.ptr = a.ptr + a.ptr_off[k];
-	pv.ptrJ = pv.ptr + (size_t)n_stripes * pv.G * pv.RPP;
+	pv.ptrJ = ptr_plane(pv.ptr, n_stripes, pv.G, pv.R);
 	RunWriter w;
 	w.dst = a.scratch + a.scratch_off[k]; w.n_ops = w.n_cols = w.run = 0; w.op = 0;
 	uint32_t i = a.end_i[p], j = a.end_j[p], state = a.end_state[p], tick = 3;
 	if constexpr (EDIT == EDIT_WALK_BITS) {
-		const uint32_t R = pv.R, G = (((l2 + 63u) | 15u) >> 4) + 1;
+		const uint32_t R = pv.R, G = edit_bits_groups(l2);
 		const uint2 *base = (const uint2 *)(a.ptr + a.ptr_off[k]);
 		while (i > 0 && j > 0) {
 			// the path mostly runs along the diagonal: pull the word AT_TB_PF_AHEAD cells up-left into L2
@@ -243,11 +224,10 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 			else                       { --i; w.col(CIG_I); }                 // UP
 		}
 	} else if constexpr (EDIT == EDIT_WALK_LIN) {
-		const uint32_t tl = steps_last(l2, 15);
-		pv.G = (tl >> 4) + 1; pv.GJ = 0;
+		pv.G = ptr_groups(ptr_last_step(l2, PTR_SH_2BIT), PTR_SH_2BIT); pv.GJ = 0;
 		if (i) pv.seek(i);
 		while (i > 0 && j > 0) {
-			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u))) pv.prefetch(i, j, 4);
+			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u))) pv.prefetch(i, j, PTR_SH_2BIT);
 			const uint32_t c = pv.two(j);                                      // bit 1: UP, bit 0: DIAG, 0: LEFT
 			if (c & 2u)      { --i; pv.up(); w.col(CIG_I); }
 			else if (c & 1u) { --i; pv.up(); --j; w.col(CIG_M); }
@@ -255,7 +235,7 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 		}
 	} else if constexpr (BANDED) {
 		const bool ov = a.mode == MODE_OVERLAP;
-		pv.l1 = l1; pv.l2 = l2; pv.elo = a.band[p].x; pv.ehi = a.band[p].y; pv.wsh = ov ? 4u : 3u;
+		pv.l1 = l1; pv.l2 = l2; pv.elo = a.band[p].x; pv.ehi = a.band[p].y; pv.wsh = ov ? PTR_SH_2BIT : PTR_SH_NIB;
 		if (i && j) pv.seek_band(i);
 		while (j > 0) {
 			if (i == 0) break;
@@ -281,7 +261,7 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 	if (a.mode == MODE_OVERLAP) {
 		while (j > 0) {                                   // :899
 			if (i == 0) break;                            // row 0 is -inf (:937): unreachable on a finite path
-			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u))) pv.prefetch(i, j, 4);      // every AT_TB_PF_PERIOD-th step: a sector holds eight rows of a lane block
+			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u))) pv.prefetch(i, j, PTR_SH_2BIT);      // every AT_TB_PF_PERIOD-th step: a sector holds eight rows of a lane block
 			const uint32_t c = pv.two(j);                 // bit 1: RIGHT beat both; bit 0: DIAGONAL beat LEFT
 			if (c & 2u)      { --i; pv.up(); w.col(CIG_I); }                  // RIGHT
 			else if (c & 1u) { --i; pv.up(); --j; w.col(CIG_M); }             // DIAGONAL
@@ -294,11 +274,11 @@ __global__ void __launch_bounds__(128) at_traceback_walk(const TraceArgs a)
 			if (!go || home) break;
 			if (j == 0 && state != ST_LOW) break;         // only reachable with corrupt pointers: never index s2[-1]
 			if (state == ST_JUMP && jump) {               // a jump run reads only the 1-bit plane (32 columns per word)
-				if (a.lookahead && j > 160u) asm volatile("prefetch.global.L2 [%0];" :: "l"(pv.ptrJ + pv.rowJ + (size_t)((j - 128u + pv.lane) >> 5) * pv.RPP));
+				if (a.lookahead && j > 160u) asm volatile("prefetch.global.L2 [%0];" :: "l"(pv.ptrJ + pv.rowJ + (size_t)((j - 128u + pv.lane) >> PTR_SH_JUMP) * pv.RPP));
 				state = pv.jbit(j) ? ST_JUMP : ST_MID; --j; w.col(CIG_N);
 				continue;
 			}
-			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u))) pv.prefetch(i, j, pv.half ? 2 : 3);
+			if (a.lookahead && !(++tick & (AT_TB_PF_PERIOD - 1u))) pv.prefetch(i, j, pv.half ? PTR_SH_PACKED : PTR_SH_NIB);
 			const uint32_t nb = pv.nib(j);
 			if (state == ST_LOW)      { state = (nb & 4u) ? ST_MID : ST_LOW; --i; pv.up(); w.col(CIG_I); }
 			else if (state == ST_MID) {
@@ -435,7 +415,7 @@ __global__ void at_plan_uniform(uint32_t n, int packed, uint32_t R, uint64_t wor
 	ptr_off[k] = (uint64_t)job * words_per_job;
 	bnd_off[k] = 0;
 	if (scratch_off) scratch_off[k] = (uint64_t)k * scratch_per_pair;
-	rclass[k] = (uint8_t)(R | (packed ? ((k & 1u) ? 2u : 1u) << 4 : 0u));
+	rclass[k] = ptr_class(R, packed ? ((k & 1u) ? 2u : 1u) : 0u);
 	if (!packed) jobs[k] = FillJob{k, k};
 	else if (!(k & 1u)) jobs[job] = FillJob{k, has_partner ? k + 1u : k};
 }

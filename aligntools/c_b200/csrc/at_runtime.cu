@@ -261,25 +261,6 @@ struct at_batch {
 
 static inline uint32_t rclass_of(uint32_t l1) { uint32_t r = (l1 + 31) / 32; return r < 1 ? 1 : (r > (uint32_t)MAXR ? MAXR : r); }
 
-// pointer words of one pair's block; edit (AT_OUT_EDIT_PATH) on the cell-by-cell kernel stores overlap's layout
-static uint64_t ptr_words_of(int mode, bool jump, uint32_t l1, uint32_t l2)
-{
-	const uint32_t R = rclass_of(l1), RPP = 32 * R;
-	const uint64_t stripes = (l1 + RPP - 1) / RPP;
-	if (mode == AT_OVERLAP || mode == AT_EDIT) { const uint32_t tl = (l2 + 31u) | 15u; return stripes * ((tl >> 4) + 1) * RPP; }
-	const uint32_t tl = (l2 + 31u) | (jump ? 31u : 7u);
-	uint64_t w = stripes * ((tl >> 3) + 1) * RPP;
-	if (jump) w += stripes * ((tl >> 5) + 1) * RPP;
-	return w;
-}
-
-// the same for at_wave_edit_bits<R, true>: a uint2 per (32-row block, step), stripes of 1024 R rows, steps 0 .. (l2 + 63) | 15
-static uint64_t edit_bits_words(uint32_t R, uint32_t l1, uint32_t l2)
-{
-	const uint64_t stripes = (l1 + 1024u * R - 1) / (1024u * R), G = (((l2 + 63u) | 15u) >> 4) + 1;
-	return stripes * G * R * 1024u;
-}
-
 __global__ void at_unpack_2bit(const uint8_t *src, const uint64_t *src_off, const uint64_t *dst_off,
                                const uint32_t *len, uint32_t n_pairs, uint8_t *dst)
 {
@@ -605,16 +586,18 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		const uint64_t warp_slots = (uint64_t)s.dev->sm_count * 8 * AT_WAVE_WARPS;
 		for (int r : {4, 2}) {
 			uint64_t tasks = 0;
-			for (uint32_t k = 0; k < n; ++k) tasks += (in->q_len[s.p0 + k] + 1024u * r - 1) / (1024u * r);
+			for (uint32_t k = 0; k < n; ++k) tasks += (in->q_len[s.p0 + k] + edit_bits_rows(r) - 1) / edit_bits_rows(r);
 			if (tasks >= 2 * warp_slots) { s.bits_r = r; break; }
 		}
 	}
 	const bool bits_path = s.bits && b->traceback;      // edit paths on at_wave_edit_bits: K3 reads R from the pair's class
 	auto rclass = [&](uint32_t l1) -> uint32_t { return band_affine ? (uint32_t)MAXR : bits_path ? (uint32_t)s.bits_r : rclass_of(l1); };
 	auto pair_cells = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t { return s.banded ? band_cells(l1, l2, s.h_band[k].x, s.h_band[k].y) : (uint64_t)l1 * l2; };
+	// overlap and edit on the cell-by-cell kernel store 2-bit codes, the affine modes nibbles
+	const uint32_t code_sh = b->mode >= AT_OVERLAP ? PTR_SH_2BIT : PTR_SH_NIB;
 	auto pair_ptr_words = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t {
-		if (bits_path) return edit_bits_words((uint32_t)s.bits_r, l1, l2);
-		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass(l1), band_affine ? 3u : 4u) : ptr_words_of(b->mode, jump, l1, l2);
+		if (bits_path) return edit_bits_pair_words(l1, l2, (uint32_t)s.bits_r);
+		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass(l1), code_sh) : ptr_pair_words(l1, l2, rclass(l1), code_sh, jump);
 	};
 	mark("alphabet+jmask");
 	// a UNIFORM shard (every pair of the same shape, all on K1) needs no per-pair work on the host at all: see below
@@ -628,7 +611,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		s.h_rclass.resize(n);
 		for (uint32_t k = 0; k < n; ++k) {
 			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-			s.h_rclass[k] = (uint8_t)rclass(l1);
+			s.h_rclass[k] = ptr_class(rclass(l1), 0);
 			s.cells += pair_cells(k, l1, l2);
 		}
 	}
@@ -684,13 +667,12 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 	{
 		if (uniform && need_words && need_words > budget_words) {      // several chunks: the general plan (it needs the per-pair classes)
 			uniform = false;
-			s.h_rclass.assign(n, (uint8_t)rclass_of(l1u));
+			s.h_rclass.assign(n, ptr_class(rclass_of(l1u), 0));
 		}
 		if (uniform) {
 			const bool packed = p16_ok(l1u, l2u) && n >= 2;
 			const uint32_t R = rclass_of(l1u);
-			const uint32_t tl = (l2u + 31u) | (packed ? 3u : (jump ? 31u : 7u));
-			const uint64_t words_per_job = !b->traceback ? 0 : packed ? (uint64_t)((tl >> 2) + 1) * R * 32 : ptr_words_of(b->mode, jump, l1u, l2u);
+			const uint64_t words_per_job = !b->traceback ? 0 : packed ? ptr_packed_job_words(l2u, R) : pair_ptr_words(0, l1u, l2u);
 			const uint64_t n_jobs = packed ? (n + 1) / 2 : n;
 			s.chunks.emplace_back();
 			Chunk &c = s.chunks.back();
@@ -768,7 +750,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 			if (!sorted) std::stable_sort(cand.begin(), cand.end(), [&](uint32_t x, uint32_t y) { return key(x) > key(y); });
 			for (size_t x = 0; x < cand.size();) {
 				if (x + 1 < cand.size() && key(cand[x]) == key(cand[x + 1])) {
-					const int r = s.h_rclass[cand[x]] & 15;
+					const int r = ptr_class_r(s.h_rclass[cand[x]]);
 					l16[r].h_jobs.push_back(FillJob{cand[x], cand[x + 1]});
 					l16[r].cells += cells_of(cand[x]) + cells_of(cand[x + 1]);
 					x += 2;
@@ -777,7 +759,7 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		}
 		// ---- int32 jobs (K1) per R class ----
 		by_cells(scalar_pairs);
-		for (uint32_t k : scalar_pairs) { const int r = s.h_rclass[k] & 15; l32[r].h_jobs.push_back(FillJob{k, k}); l32[r].cells += cells_of(k); }
+		for (uint32_t k : scalar_pairs) { const int r = ptr_class_r(s.h_rclass[k]); l32[r].h_jobs.push_back(FillJob{k, k}); l32[r].cells += cells_of(k); }
 		// ---- wavefront tasks (K2): (pair, stripe), collected pair by pair, then put in queue order (order_wave_tasks) ----
 		by_cells(wave_pairs);
 		c.h_bnd_off.assign(nc, 0);
@@ -785,8 +767,8 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		const int bits_r = s.bits_r;
 		for (uint32_t k : wave_pairs) {
 			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-			const int r = s.bits ? bits_r : (s.h_rclass[k] & 15);
-			const uint32_t rows = s.bits ? 1024u * r : 32u * r;
+			const int r = s.bits ? bits_r : ptr_class_r(s.h_rclass[k]);
+			const uint32_t rows = s.bits ? edit_bits_rows(r) : 32u * r;
 			Launch &lw = s.bits ? lbit[r] : lwv[r];
 			const uint32_t n_stripes = (l1 + rows - 1) / rows;
 			uint32_t queued = 0;
@@ -823,13 +805,12 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 			for (const Launch &l : c.launches) {
 				if (l.kind == LK_PACKED) {
 					for (const FillJob &jb : l.h_jobs) {
-						const uint32_t tl = (in->t_len[s.p0 + jb.a] + 31u) | 3u;
 						c.h_ptr_off[jb.a - c.k0] = words; c.h_ptr_off[jb.b - c.k0] = words;
-						s.h_rclass[jb.a] = (uint8_t)(l.r | (1 << 4)); s.h_rclass[jb.b] = (uint8_t)(l.r | (2 << 4));
-						words += (uint64_t)((tl >> 2) + 1) * l.r * 32;
+						s.h_rclass[jb.a] = ptr_class(l.r, 1); s.h_rclass[jb.b] = ptr_class(l.r, 2);
+						words += ptr_packed_job_words(in->t_len[s.p0 + jb.a], l.r);
 					}
 				} else if (l.kind == LK_INT32) {
-					for (const FillJob &jb : l.h_jobs) { const uint32_t k = jb.a; c.h_ptr_off[k - c.k0] = words; words += ptr_words_of(b->mode, jump, in->q_len[s.p0 + k], in->t_len[s.p0 + k]); }
+					for (const FillJob &jb : l.h_jobs) { const uint32_t k = jb.a; c.h_ptr_off[k - c.k0] = words; words += pair_ptr_words(k, in->q_len[s.p0 + k], in->t_len[s.p0 + k]); }
 				} else {
 					// a pair's block goes where its first task is queued (stripe 0 unless the band leaves stripe 0 out)
 					std::vector<uint8_t> placed(nc, 0);
@@ -1061,7 +1042,7 @@ static uint64_t banded_global_tasks(const at_batch_input *in, const at_band *ban
 		int32_t elo, ehi;
 		band_clip(l1, l2, band->lo[k], band->hi[k], elo, ehi);
 		BandWin w;
-		for (uint32_t s = (l1 + RPP - 1) / RPP; s-- > 0 && band_stripe(l1, l2, elo, ehi, RPP, s, w, 3u);) ++n;      // the windows are the bottom run
+		for (uint32_t s = (l1 + RPP - 1) / RPP; s-- > 0 && band_stripe(l1, l2, elo, ehi, RPP, s, w, PTR_SH_NIB);) ++n;      // the windows are the bottom run
 	}
 	return n;
 }

@@ -203,7 +203,7 @@ __device__ __forceinline__ void wait_columns(const uint32_t *prog, uint32_t need
 // LDS from the boundary ring); it enters through a multiply-add with a 0/1 lane mask, not a branch.
 // Boundary element (int4 per column): x = M + o (tag 3), y = L (tag 3), z = H (tagged), w unused.
 //
-// BANDED (global only): the pair's band (at_band.h, 8-step pointer groups: wsh = 3) limits every stripe to its column
+// BANDED (global only): the pair's band (at_band.h, 8-step pointer groups: wsh = PTR_SH_NIB) limits every stripe to its column
 // window.  The band holds the end diagonal l2 - l1 (the host checks it), so the stripes without a window are a run at the
 // top of the pair and the host queues none of them.  The steps run from the window's t0 to (c1 + 31) | 31; 8-step blocks
 // whose cells may leave the band force M, L and U of those cells to -inf, blocks wholly inside the band run the plain body.
@@ -260,11 +260,11 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 		const uint8_t *jbase16 = JUMP ? a.jmask + a.j_off[p] - sh : nullptr;     // the host lays the masks out with the targets' ring alignment
 		uint32_t n_tiles = (l2 + sh + 255u) >> 8;
 		uint32_t *__restrict__ ptr = a.ptr + a.ptr_off[p - a.pair_base];
-		const uint32_t t_ptr_last = (l2 + 31u) | (JUMP ? 31u : 7u);       // pointer-block geometry shared with K1 / K3
-		const uint32_t G = (t_ptr_last >> 3) + 1, GJ = (t_ptr_last >> 5) + 1;
+		const uint32_t t_ptr_last = ptr_last_step(l2, PTR_SH_NIB, JUMP);
+		const uint32_t G = ptr_groups(t_ptr_last, PTR_SH_NIB), GJ = ptr_groups(t_ptr_last, PTR_SH_JUMP);
 		uint32_t t_last = (l2 + 31u) | 31u;
 		const uint32_t n_stripes = (l1 + RPP - 1) / RPP;
-		uint32_t *__restrict__ ptrJ = ptr + (size_t)n_stripes * G * RPP;
+		uint32_t *__restrict__ ptrJ = ptr_plane(ptr, n_stripes, G, R);
 		const bool last_stripe = stripe + 1 == n_stripes;
 		// banded: this stripe's window (bw), the one above (bwp), whether the stripe above takes part
 		BandWin bw = {1u, l2, 0u, G}, bwp = bw;
@@ -273,11 +273,11 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 		if constexpr (BANDED) {
 			const int2 bd = a.band[p];
 			elo = bd.x; ehi = bd.y;
-			band_stripe(l1, l2, elo, ehi, RPP, stripe, bw, 3u);             // queued stripes have a window
-			has_prev = stripe > 0 && band_stripe(l1, l2, elo, ehi, RPP, stripe - 1u, bwp, 3u);
+			band_stripe(l1, l2, elo, ehi, RPP, stripe, bw, PTR_SH_NIB);     // queued stripes have a window
+			has_prev = stripe > 0 && band_stripe(l1, l2, elo, ehi, RPP, stripe - 1u, bwp, PTR_SH_NIB);
 			t_last = band_t_last(bw);
 			n_tiles = min(n_tiles, ((bw.c1 - 1u + sh) >> 8) + 1u);         // tiles the window reads
-			if (want_ptr) ptr += band_stripe_off(l1, l2, elo, ehi, RPP, stripe, 3u);
+			if (want_ptr) ptr += band_stripe_off(l1, l2, elo, ehi, RPP, stripe, PTR_SH_NIB);
 		}
 		const uint32_t tile0 = bw.t0 >> 8;                                 // first tile the stripe reads (0 unbanded)
 		const uint32_t slab = (l2 + 4u) & ~3u;
@@ -490,18 +490,18 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 				for (uint32_t k = 0; k < 8; ++k) step(tb + k, true, std::true_type(), std::integral_constant<bool, BANDED>());
 			}
 			if constexpr (BANDED) {
-				if (want_ptr && ((tb - bw.t0) >> 3) < bw.groups) {
-					uint32_t *w = ptr + ((size_t)((tb - bw.t0) >> 3) * 32 + lane) * R;
+				if (want_ptr && ((tb - bw.t0) >> PTR_SH_NIB) < bw.groups) {
+					uint32_t *w = ptr_at(ptr, 0u, 0u, (tb - bw.t0) >> PTR_SH_NIB, lane, R);
 #pragma unroll
 					for (int r = 0; r < R; ++r) w[r] = ptr_word(st[r].x);
 				}
-			} else if (want_ptr && (tb >> 3) < G) {
-				uint32_t *w = ptr + ((size_t)(stripe * G + (tb >> 3)) * 32 + lane) * R;
+			} else if (want_ptr && (tb >> PTR_SH_NIB) < G) {
+				uint32_t *w = ptr_at(ptr, stripe, G, tb >> PTR_SH_NIB, lane, R);
 #pragma unroll
 				for (int r = 0; r < R; ++r) w[r] = ptr_word(st[r].x);
 			}
-			if (JUMP && want_ptr && (tb & 31u) == 24u && (tb >> 5) < GJ) {
-				uint32_t *w = ptrJ + ((size_t)(stripe * GJ + (tb >> 5)) * 32 + lane) * R;
+			if (JUMP && want_ptr && (tb & 31u) == 24u && (tb >> PTR_SH_JUMP) < GJ) {
+				uint32_t *w = ptr_at(ptrJ, stripe, GJ, tb >> PTR_SH_JUMP, lane, R);
 #pragma unroll
 				for (int r = 0; r < R; ++r) w[r] = jump_word(st[r].xj);
 			}
@@ -629,7 +629,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 		const uint32_t tile_wait = twobit ? 192u : 224u;                      // step (mod 256) at which the next tile must have landed: lane 0 is up to sh + 1 columns ahead of the step counter
 		uint32_t n_tiles = (l2 + sh + 255u) >> 8;
 		uint32_t *__restrict__ ptr = STORE ? a.ptr + a.ptr_off[p - a.pair_base] : nullptr;
-		const uint32_t G = (((l2 + 31u) | 15u) >> 4) + 1;                 // pointer-block geometry shared with K3
+		const uint32_t G = ptr_groups(ptr_last_step(l2, PTR_SH_2BIT), PTR_SH_2BIT);
 		uint32_t t_last = (l2 + 31u) | 31u;
 		const uint32_t n_stripes = (l1 + RPP - 1) / RPP;
 		const bool last_stripe = stripe + 1 == n_stripes;
@@ -640,16 +640,16 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 		if constexpr (BANDED) {
 			const int2 bd = a.band[p];
 			elo = bd.x; ehi = bd.y;
-			if (!band_stripe(l1, l2, elo, ehi, RPP, stripe, bw)) {
+			if (!band_stripe(l1, l2, elo, ehi, RPP, stripe, bw, PTR_SH_2BIT)) {
 				if (lane == 0) { a.score[p] = 0; a.end_i[p] = l1; a.end_j[p] = 0; a.end_state[p] = ST_MID; }      // M[l1][0] (:938)
 				__syncwarp();
 				continue;
 			}
-			has_prev = stripe > 0 && band_stripe(l1, l2, elo, ehi, RPP, stripe - 1u, bwp);
-			has_next = !last_stripe && band_stripe(l1, l2, elo, ehi, RPP, stripe + 1u, bwn);
+			has_prev = stripe > 0 && band_stripe(l1, l2, elo, ehi, RPP, stripe - 1u, bwp, PTR_SH_2BIT);
+			has_next = !last_stripe && band_stripe(l1, l2, elo, ehi, RPP, stripe + 1u, bwn, PTR_SH_2BIT);
 			t_last = band_t_last(bw);
 			n_tiles = min(n_tiles, ((bw.c1 - 1u + sh) >> 8) + 1u);         // tiles the window reads
-			if (want_ptr) ptr += band_stripe_off(l1, l2, elo, ehi, RPP, stripe);
+			if (want_ptr) ptr += band_stripe_off(l1, l2, elo, ehi, RPP, stripe, PTR_SH_2BIT);
 		}
 		const uint32_t tile0 = bw.t0 >> 8;                                 // first tile the stripe reads (0 unbanded)
 		const uint32_t slab = (l2 + 4u) & ~3u;
@@ -827,13 +827,13 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 				for (uint32_t k = 0; k < 16; ++k) step(tb + k, true, std::true_type(), std::integral_constant<bool, BANDED>());
 			}
 			if constexpr (BANDED) {
-				if (want_ptr && ((tb - bw.t0) >> 4) < bw.groups) {
-					uint32_t *w = ptr + ((size_t)((tb - bw.t0) >> 4) * 32 + lane) * R;
+				if (want_ptr && ((tb - bw.t0) >> PTR_SH_2BIT) < bw.groups) {
+					uint32_t *w = ptr_at(ptr, 0u, 0u, (tb - bw.t0) >> PTR_SH_2BIT, lane, R);
 #pragma unroll
 					for (int r = 0; r < R; ++r) w[r] = lin_word(stl[r].x);
 				}
-			} else if (want_ptr && (tb >> 4) < G) {
-				uint32_t *w = ptr + ((size_t)(stripe * G + (tb >> 4)) * 32 + lane) * R;
+			} else if (want_ptr && (tb >> PTR_SH_2BIT) < G) {
+				uint32_t *w = ptr_at(ptr, stripe, G, tb >> PTR_SH_2BIT, lane, R);
 #pragma unroll
 				for (int r = 0; r < R; ++r) w[r] = PTR ? stl[r].x : lin_word(stl[r].x);      // edit: the code is the tag
 			}
@@ -871,17 +871,13 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 // membar per 32 columns -- 22 % of this kernel's stall samples when it was first written that way.)
 //   score = M[l1][l2] = l1 + sum over j of the horizontal difference at row l1.     SURVEY.md 8(f) #4.
 //
-// PTR (AT_OUT_EDIT_PATH): every block column also yields min3's argmin for its 32 cells as two bit planes (edit_bits_ptr,
-// at_cell.cuh: LEFT = Ph, DIAG = ~Ph & (Eq | (Pv & ~Mh)), UP = neither), stored as one uint2 (LEFT, DIAG) per
-// (block, column) in SKEWED coordinates -- step t = j + 2 lane + 1, as the lanes run:
-//     uint2 index = (((stripe * G + t / 16) * R + r) * 16 + t % 16) * 32 + lane,    G = ((l2 + 63) | 15) / 16 + 1,
-// so one store per block column writes 256 contiguous bytes across the warp (full sectors, no staging) and a pair's block
-// is 2 bits per cell of its stripes (rows rounded up to 1024 R).  K3's bit-parallel walker reads it.
+// PTR (AT_OUT_EDIT_PATH): every block column also stores min3's argmin for its 32 cells in the bit-parallel edit layout of
+// at_ptr_layout.h.  K3's bit-parallel walker reads it.
 // =====================================================================================
 template <int R, bool PTR = false>
 __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const WaveArgs a)
 {
-	constexpr int RPP = 1024 * R;                 // rows per stripe
+	constexpr int RPP = edit_bits_rows(R);        // rows per stripe
 	constexpr int NSYM = 9;                       // 8 symbols + "matches nothing"
 	struct __align__(16) Smem { uint32_t eq[NSYM][32][R]; WaveRing<false> rg; };
 	__shared__ Smem sm_all[AT_WAVE_WARPS];
@@ -918,8 +914,10 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 		const uint64_t tag_in = (uint64_t)stripe << 32;                    // the predecessor's tag: (stripe - 1) + 1
 		const uint64_t tag_out = (uint64_t)(stripe + 1u) << 32;
 		const uint32_t row0 = stripe * RPP + lane * 32u * R;
-		uint2 *__restrict__ pp = nullptr;                                  // PTR: this lane's words of the stripe
-		if constexpr (PTR) pp = (uint2 *)(a.ptr + a.ptr_off[p - a.pair_base]) + (size_t)stripe * ((((l2 + 63u) | 15u) >> 4) + 1) * R * 512 + lane;
+		// PTR: this lane's words of the stripe, edit_bits_slot(stripe, G, 0, R, 0, lane); store_ptr adds (t, r)'s offset.
+		// Spelled out here: through the helper, nvcc orders this kernel's address arithmetic differently.
+		uint2 *__restrict__ pp = nullptr;
+		if constexpr (PTR) pp = (uint2 *)(a.ptr + a.ptr_off[p - a.pair_base]) + (size_t)stripe * edit_bits_groups(l2) * R * 512 + lane;
 
 		__syncwarp();
 		if (n_tiles > 0) ring_issue<false>(sm.rg, tbase16, nullptr, 0, lane, twobit);
@@ -1067,7 +1065,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_edit_bits(const Wa
 			if (pf) { pf_word = nw; pf_group = ng; }
 		};
 
-		const uint32_t t_end = (l2 + 63u) | 15u;                           // lane 31 reaches column l2 at step l2 + 63
+		const uint32_t t_end = edit_bits_last_step(l2);
 		for (uint32_t tb = 0; tb <= t_end; tb += 16) {
 			if ((tb & 255u) == 96u && tb > 96u) {                          // lane 31 has left tile tb/256 - 1: refill its slot two tiles ahead
 				const uint32_t c = (tb >> 8) + 1u;
