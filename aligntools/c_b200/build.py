@@ -16,7 +16,7 @@ HOST_HEADERS = ["at_fasta.h"]
 CLI = os.path.join(ROOT, "bin", "alignTools")
 FASTA_DUMP = os.path.join(ROOT, "bin", "at_fasta_dump")
 SOURCES = ["at_runtime.cu", "at_shim.cu"]
-HEADERS = ["at_kernels.cuh", "at_cell.cuh", "at_band.h", "at_ptr_layout.h", "at_fill_affine.cuh", "at_wavefront.cuh", "at_devmem.h", "at_pipeline.inl", os.path.join("..", "..", "..", "include", "aligntools_b200.h")]
+HEADERS = ["at_kernels.cuh", "at_cell.cuh", "at_band.h", "at_ptr_layout.h", "at_plan.h", "at_fill_affine.cuh", "at_wavefront.cuh", "at_devmem.h", "at_pipeline.inl", os.path.join("..", "..", "..", "include", "aligntools_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-O2,-Wall,-Wno-unused-function", "--threads", "0"]
 

@@ -34,6 +34,7 @@
 // tie rules SURVEY.md A.0:  M: first strictly greater in order L,M,U,(J|HOME);  L: extend wins
 // ties;  U: open wins ties;  J: enter wins ties, entering forbidden on listed target indices.
 #pragma once
+#include "at_plan.h"      // FillJob
 
 namespace atb2 {
 
@@ -53,8 +54,6 @@ __host__ __device__ constexpr size_t fill_smem_bytes(int R, bool packed, bool pr
 	return (size_t)AT_FILL_WARPS * (prof ? (size_t)(AT_RING + AT_RING_MIRROR) * 2 + (size_t)prof_combs(packed) * 32 * k1_lane_stride(R) * 4
 	                                     : (size_t)(AT_RING + AT_RING_MIRROR) * 4);
 }
-
-struct FillJob { uint32_t a, b; };     // pair indices; b == a for int32 lanes or a packed job without partner
 
 struct FillArgs2 {
 	const uint8_t  *q;       const uint64_t *q_off;  const uint32_t *q_len;

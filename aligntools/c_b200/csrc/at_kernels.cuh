@@ -403,21 +403,18 @@ __global__ void __launch_bounds__(256) at_symbol_set(const uint8_t *bytes, uint6
 
 // Plan arrays of a UNIFORM shard (every pair has the same l1 and the same l2, all on K1): what the host otherwise
 // builds pair by pair and uploads -- the job list, the pointer-block / scratch offsets, the layout class -- is
-// closed form, so the device writes it itself (no host loops, no pageable uploads on the set-up path).
-// packed: jobs are pairs (2k, 2k+1), a last odd pair runs alone.
-__global__ void at_plan_uniform(uint32_t n, int packed, uint32_t R, uint64_t words_per_job, uint64_t scratch_per_pair,
-                                FillJob *jobs, uint64_t *ptr_off, uint64_t *bnd_off, uint64_t *scratch_off, uint8_t *rclass)
+// closed form (uniform_pair, at_plan.h), so the device writes it itself (no host loops, no pageable uploads on the
+// set-up path).
+__global__ void at_plan_uniform(uint32_t n, const UniformPlan u, FillJob *jobs, uint64_t *ptr_off, uint64_t *bnd_off, uint64_t *scratch_off, uint8_t *rclass)
 {
 	const uint32_t k = blockIdx.x * blockDim.x + threadIdx.x;
 	if (k >= n) return;
-	const uint32_t job = packed ? k >> 1 : k;
-	const bool has_partner = packed && ((k | 1u) < n);
-	ptr_off[k] = (uint64_t)job * words_per_job;
+	const UniformPair p = uniform_pair(u, n, k);
+	ptr_off[k] = p.ptr_off;
 	bnd_off[k] = 0;
-	if (scratch_off) scratch_off[k] = (uint64_t)k * scratch_per_pair;
-	rclass[k] = ptr_class(R, packed ? ((k & 1u) ? 2u : 1u) : 0u);
-	if (!packed) jobs[k] = FillJob{k, k};
-	else if (!(k & 1u)) jobs[job] = FillJob{k, has_partner ? k + 1u : k};
+	if (scratch_off) scratch_off[k] = p.scratch_off;
+	rclass[k] = p.rclass;
+	if (p.writes_job) jobs[p.job] = p.fj;
 }
 
 // fit+jump: expand the per-pair blacklists into a byte mask aligned with the target bytes.

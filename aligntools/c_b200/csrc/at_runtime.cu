@@ -154,34 +154,14 @@ extern "C" int at_device_count(const at_handle *h) { return h ? (int)h->devs.siz
 extern "C" uint64_t at_launch_count(const at_handle *h) { return h ? h->launches.load() : 0; }
 
 // ------------------------------------------------------------------- batch ----
-static const int MAXR = 8;
 static const size_t AT_SEQ_SLACK = 1024;   // K2 stages 256-byte target tiles by TMA: the last tile may run past the last record
 
-// One kernel launch of a chunk: the jobs of one (kernel kind, rows-per-lane) class.
-enum { LK_INT32 = 0, LK_PACKED = 1, LK_WAVE = 2, LK_BITS = 3 };   // LK_BITS: bit-parallel edit distance (K2 task geometry, 1024*r rows per stripe)
-struct Launch {
-	int kind = LK_INT32, r = 1;
-	uint64_t cells = 0;
-	std::vector<FillJob> h_jobs;        // LK_INT32: one pair per warp (a == b); LK_PACKED: two pairs per warp
-	DevBuf<FillJob> d_jobs;
-	std::vector<WaveTask> h_tasks;      // LK_WAVE / LK_BITS: (pair, stripe) in queue order (order_wave_tasks)
-	DevBuf<WaveTask> d_tasks;
-	uint64_t prog_base = 0;             // first progress word of this launch in Shard::d_prog
-	size_t n_planned = 0;               // uniform shards: the job list exists on the device only (at_plan_uniform)
-	size_t n_jobs() const { return n_planned ? n_planned : (kind >= LK_WAVE ? h_tasks.size() : h_jobs.size()); }
-};
-
-struct Chunk {
-	uint32_t k0 = 0, k1 = 0;            // shard-local pair range
-	uint64_t ptr_words = 0;
-	std::vector<uint64_t> h_ptr_off;    // chunk-local
-	DevBuf<uint64_t> d_ptr_off;
-	std::vector<Launch> launches;
-	std::vector<uint64_t> h_bnd_off;    // chunk-local: element offset of the pair's two boundary slabs (K2)
-	DevBuf<uint64_t> d_bnd_off;
-	uint64_t bnd_elems = 0, prog_words = 0;
-	DevBuf<uint64_t> d_ops_off, d_cols_off, d_scratch_off;
-	std::vector<uint64_t> h_scratch_off; uint64_t scratch_words = 0;
+// A chunk of the shard's plan (at_plan.h) and its device buffers
+struct Chunk : PlanChunk {
+	explicit Chunk(PlanChunk &&p) : PlanChunk(std::move(p)) {}
+	std::vector<DevBuf<FillJob>> d_jobs;       // [launch] K1 jobs ...
+	std::vector<DevBuf<WaveTask>> d_tasks;     // ... or K2 tasks
+	DevBuf<uint64_t> d_ptr_off, d_bnd_off, d_ops_off, d_cols_off, d_scratch_off;
 	DevBuf<uint32_t> d_cigar; DevBuf<uint8_t> d_aln1, d_aln2;   // exact-size outputs of this chunk ...
 	uint32_t *cigar = nullptr; uint8_t *aln1 = nullptr, *aln2 = nullptr;   // ... or the workspace's grow-only buffers (pipelined path); what fetch reads
 	uint64_t tot_ops = 0, tot_cols = 0;
@@ -212,15 +192,13 @@ struct Shard {
 	bool bits = false;                         // bit-parallel edit distance: `-u 1` and reads of <= 8 distinct bytes
 	int bits_r = 1;                            // its 32-row blocks per lane (one launch per shard; fixes the edit-path pointer layout)
 	bool twobit = false;                       // the sequences stay 2-bit packed in HBM (AT_SEQ_2BIT input consumed directly by K1 / K2 / K3)
-	bool banded = false;                       // overlap / global with a per-pair band: h_band / d_band hold it clipped (at_band.h)
-	std::vector<int2> h_band;
+	bool banded = false;                       // overlap / global with a per-pair band: d_band holds it clipped (at_band.h)
 	DevBuf<int2> d_band;
 	std::vector<uint64_t> h_t_rel;             // twobit + jump: device offsets of the packed targets (the jump masks copy their alignment)
 	DevBuf<uint64_t> d_j_off;                  // twobit + jump: per-pair offsets into d_jmask (byte-encoded targets use d_t_off)
 	BufCache cache;                            // released device blocks, reused by this shard's next allocations
 	struct UploadGate *gate = nullptr; uint64_t gate_turn = 0;   // pipelined path: sub-slices upload their sequences one at a time, in pair order
 	bool workspace = false;                    // pipeline workspace: reused for many sub-slices, buffers get head-room
-	std::vector<uint8_t> h_rclass;
 	std::vector<Chunk> chunks;
 	uint64_t cells = 0, ptr_bytes = 0, t_span = 0;   // t_span: bytes of d_t that hold the caller's target span
 	cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -258,8 +236,6 @@ struct at_batch {
 	std::vector<Shard> shards;
 	bool ran = false;
 };
-
-static inline uint32_t rclass_of(uint32_t l1) { uint32_t r = (l1 + 31) / 32; return r < 1 ? 1 : (r > (uint32_t)MAXR ? MAXR : r); }
 
 __global__ void at_unpack_2bit(const uint8_t *src, const uint64_t *src_off, const uint64_t *dst_off,
                                const uint32_t *len, uint32_t n_pairs, uint8_t *dst)
@@ -338,7 +314,7 @@ static int upload_side(at_handle *h, Shard &s, uint32_t encoding, const uint8_t 
 static void release_chunks(Shard &s)
 {
 	for (auto &c : s.chunks) {
-		c.d_ptr_off.release(); c.d_bnd_off.release(); for (auto &l : c.launches) { l.d_jobs.release(); l.d_tasks.release(); }
+		c.d_ptr_off.release(); c.d_bnd_off.release(); for (auto &d : c.d_jobs) d.release(); for (auto &d : c.d_tasks) d.release();
 		c.d_ops_off.release(); c.d_cols_off.release(); c.d_scratch_off.release(); c.d_cigar.release(); c.d_aln1.release(); c.d_aln2.release();
 	}
 	s.chunks.clear();
@@ -474,45 +450,8 @@ static int build_jump_mask(at_batch *b, Shard &s, const at_batch_input *in)
 }
 
 
-// Queue order of the K2 tasks of one launch.  The persistent warps claim tasks in queue order, and a stripe can only run
-// as far as the stripe above it has got.  Pair after pair (round 1) puts a pair's stripes next to each other in the
-// queue: they are claimed within microseconds of each other and run as ONE tightly coupled chain, each stripe 64 columns
-// behind the one above -- the chain advances at the pace of its momentarily slowest warp and the others poll (ncu on
-// C3, 2 048 pairs: 21 % of all warp samples in the progress poll and its warp-sync).  Stripe after stripe ACROSS the
-// launch's pairs -- all stripes 0, then all stripes 1, ... -- puts as many other tasks between a stripe and its
-// predecessor as the launch has pairs: with more pairs than resident warps the predecessor has finished (or is far
-// ahead) when the stripe is claimed and nothing ever polls; with fewer pairs the chains are as long as they have to be
-// to fill the GPU and no longer.  A task's predecessor still precedes it in the queue, so a claimed task only ever
-// waits for a running one (deadlock freedom as before).  In: tasks collected pair by pair, stripes ascending.
-// AT_WAVE_ORDER=pair keeps the old order (A/B runs).
 // AT_WAVE_START_LAG (columns, default 0): a K2 stripe starts only once the stripe above it is this far ahead (A/B knob)
 static uint32_t wave_start_lag() { static const uint32_t v = [] { const char *e = getenv("AT_WAVE_START_LAG"); return e && *e ? (uint32_t)strtoul(e, nullptr, 10) : 0u; }(); return v; }
-
-static void order_wave_tasks(std::vector<WaveTask> &t)
-{
-	static const bool pair_major = [] { const char *e = getenv("AT_WAVE_ORDER"); return e && !strcmp(e, "pair"); }();
-	const size_t n = t.size();
-	if (pair_major || n == 0) {
-		for (size_t x = 0; x < n; ++x) t[x].prev = (uint32_t)(t[x].stripe ? x - 1 : x);
-		return;
-	}
-	struct Run { uint32_t pair, n, last; size_t x0; };      // x0: the pair's first task in `t` (its stripes need not start at 0: banded pairs)
-	std::vector<Run> active;
-	for (size_t x = 0; x < n;) { size_t y = x; while (y < n && t[y].pair == t[x].pair) ++y; active.push_back(Run{t[x].pair, (uint32_t)(y - x), 0, x}); x = y; }
-	std::vector<WaveTask> out;
-	out.reserve(n);
-	for (uint32_t s = 0; !active.empty(); ++s) {
-		size_t keep = 0;
-		for (Run &r : active) {
-			const uint32_t idx = (uint32_t)out.size();
-			out.push_back(WaveTask{r.pair, t[r.x0 + s].stripe, s ? r.last : idx, 0});
-			r.last = idx;
-			if (s + 1 < r.n) active[keep++] = r;
-		}
-		active.resize(keep);
-	}
-	t.swap(out);
-}
 
 // `band` (NULL: unbanded): the caller's band arrays, indexed like `in` (band->lo[s.p0 + k] is the shard's pair k)
 static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at_band *band)
@@ -562,83 +501,35 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 	mark("upload");
 	const bool jump = b->mode == AT_FIT && b->prm.jump;
 	s.banded = band != nullptr;
+	std::vector<PairBand> bands;
 	if (s.banded) {
-		s.h_band.resize(n);
-		for (uint32_t k = 0; k < n; ++k) {
-			int32_t elo, ehi;
-			band_clip(in->q_len[s.p0 + k], in->t_len[s.p0 + k], band->lo[s.p0 + k], band->hi[s.p0 + k], elo, ehi);
-			s.h_band[k] = make_int2(elo, ehi);
-		}
+		bands.resize(n);
+		for (uint32_t k = 0; k < n; ++k) band_clip(in->q_len[s.p0 + k], in->t_len[s.p0 + k], band->lo[s.p0 + k], band->hi[s.p0 + k], bands[k].lo, bands[k].hi);
 		CU(h, s.d_band.alloc(n));
-		CU(h, cudaMemcpyAsync(s.d_band.p, s.h_band.data(), n * sizeof(int2), cudaMemcpyHostToDevice, st));      // staged before the set-up's synchronisation
+		CU(h, cudaMemcpyAsync(s.d_band.p, bands.data(), n * sizeof(int2), cudaMemcpyHostToDevice, st));      // staged before the set-up's synchronisation
 	}
-	// banded pairs: the in-band cells, the pointer words of their stripe windows (at_band.h).  Banded global pairs all run
-	// on K2's affine kernel, short ones included: R = 8 rows per lane, 8-step pointer groups
-	const bool band_affine = s.banded && b->mode == AT_GLOBAL;
 	if ((rc = choose_variants(b, s, in, q_span))) return rc;
 	if (jump && (rc = build_jump_mask(b, s, in))) return rc;
-	// bit-parallel edit distance: r = 32-row blocks per lane, 1024*r rows per stripe.  One column step of a
-	// lane is a serial chain through its r blocks, so few long pairs want r = 1 (more stripes in flight);
-	// 4 blocks per lane amortise the per-step overhead once there are tasks for every resident warp.
-	// Decided for the whole shard before the arena is sized: an edit path's pointer layout depends on it.
-	s.bits_r = 1;
-	if (s.bits) {
-		const uint64_t warp_slots = (uint64_t)s.dev->sm_count * 8 * AT_WAVE_WARPS;
-		for (int r : {4, 2}) {
-			uint64_t tasks = 0;
-			for (uint32_t k = 0; k < n; ++k) tasks += (in->q_len[s.p0 + k] + edit_bits_rows(r) - 1) / edit_bits_rows(r);
-			if (tasks >= 2 * warp_slots) { s.bits_r = r; break; }
-		}
-	}
-	const bool bits_path = s.bits && b->traceback;      // edit paths on at_wave_edit_bits: K3 reads R from the pair's class
-	auto rclass = [&](uint32_t l1) -> uint32_t { return band_affine ? (uint32_t)MAXR : bits_path ? (uint32_t)s.bits_r : rclass_of(l1); };
-	auto pair_cells = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t { return s.banded ? band_cells(l1, l2, s.h_band[k].x, s.h_band[k].y) : (uint64_t)l1 * l2; };
-	// overlap and edit on the cell-by-cell kernel store 2-bit codes, the affine modes nibbles
-	const uint32_t code_sh = b->mode >= AT_OVERLAP ? PTR_SH_2BIT : PTR_SH_NIB;
-	auto pair_ptr_words = [&](uint32_t k, uint32_t l1, uint32_t l2) -> uint64_t {
-		if (bits_path) return edit_bits_pair_words(l1, l2, (uint32_t)s.bits_r);
-		return s.banded ? band_pair_words(l1, l2, s.h_band[k].x, s.h_band[k].y, 32u * rclass(l1), code_sh) : ptr_pair_words(l1, l2, rclass(l1), code_sh, jump);
-	};
+	s.bits_r = s.bits ? (int)choose_bits_r(in->q_len + s.p0, n, (uint64_t)s.dev->sm_count * 8 * AT_WAVE_WARPS) : 1;
 	mark("alphabet+jmask");
-	// a UNIFORM shard (every pair of the same shape, all on K1) needs no per-pair work on the host at all: see below
-	const uint32_t l1u = in->q_len[s.p0], l2u = in->t_len[s.p0];
-	bool uniform = b->mode <= AT_FIT && l1u <= 32u * MAXR && !band_affine && !getenv("AT_NO_UNIFORM_PLAN");
-	for (uint32_t k = 1; k < n && uniform; ++k) uniform = in->q_len[s.p0 + k] == l1u && in->t_len[s.p0 + k] == l2u;
-	// per-pair class, result arrays
-	s.cells = 0;
-	if (uniform) s.cells = (uint64_t)n * l1u * l2u;
-	else {
-		s.h_rclass.resize(n);
-		for (uint32_t k = 0; k < n; ++k) {
-			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-			s.h_rclass[k] = ptr_class(rclass(l1), 0);
-			s.cells += pair_cells(k, l1, l2);
-		}
-	}
-	CU(h, s.d_score.alloc(n)); CU(h, s.d_end_i.alloc(n)); CU(h, s.d_end_j.alloc(n)); CU(h, s.d_end_state.alloc(n));
-	CU(h, s.d_beg_i.alloc(n)); CU(h, s.d_beg_j.alloc(n)); CU(h, s.d_n_ops.alloc(n + 1)); CU(h, s.d_n_cols.alloc(n + 1));
-	CU(h, cudaMemsetAsync(s.d_n_ops.p, 0, (n + 1) * sizeof(uint32_t), st));
-	CU(h, cudaMemsetAsync(s.d_n_cols.p, 0, (n + 1) * sizeof(uint32_t), st));
-	CU(h, cudaMemsetAsync(s.d_beg_i.p, 0, n * sizeof(uint32_t), st));
-	CU(h, cudaMemsetAsync(s.d_beg_j.p, 0, n * sizeof(uint32_t), st));
-	CU(h, s.d_counter.alloc(64));
-
-	mark("results");
-	// ---- chunking by pointer-arena budget ----
+	PlanIn pin;
+	pin.n = n; pin.l1 = in->q_len + s.p0; pin.l2 = in->t_len + s.p0;
+	pin.mode = b->mode; pin.traceback = b->traceback; pin.jump = jump;
+	pin.band = s.banded ? bands.data() : nullptr;
+	pin.bits = s.bits; pin.bits_r = (uint32_t)s.bits_r;
+	pin.p16 = p16_rule(b->mode, b->prm, jump, getenv("AT_NO_P16") != nullptr);
+	pin.allow_uniform = !getenv("AT_NO_UNIFORM_PLAN");
+	static const bool pair_major = [] { const char *e = getenv("AT_WAVE_ORDER"); return e && !strcmp(e, "pair"); }();
+	pin.pair_major = pair_major;
+	// ---- pointer-arena budget ----
 	// The whole shard's pointer blocks in one chunk if they fit the arena this shard already owns (a
 	// pipeline workspace after its first sub-slice); otherwise ask the driver what is free.
 	// cudaMemGetInfo is kept off the steady-state path: with other threads driving the device it was
 	// seen to block for tens of milliseconds.
-	uint64_t need_words = 0;
-	auto pair_words = [&](uint32_t k) -> uint64_t {
-		const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-		return b->traceback ? pair_ptr_words(k, l1, l2) + 64ull * rclass(l1) : 0;   // + rounding slack of the packed layout
-	};
-	if (uniform) need_words = (uint64_t)n * pair_words(0);
-	else for (uint32_t k = 0; k < n; ++k) need_words += pair_words(k);
+	const uint64_t need = need_words(pin);
 	size_t free_b = 0, total_b = 0;
-	const bool owned = need_words <= s.d_ptr.n && !getenv("AT_PTR_BUDGET_MB");
-	if (!owned && need_words) {
+	const bool owned = need <= s.d_ptr.n && !getenv("AT_PTR_BUDGET_MB");
+	if (!owned && need) {
 		CU(h, cudaMemGetInfo(&free_b, &total_b));
 		// blocks cached in the stream-ordered pool are reusable by this batch: count them as free
 		cudaMemPool_t pool; uint64_t reserved = 0, used = 0;
@@ -649,230 +540,73 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 		free_b += s.d_ptr.bytes;      // the arena this shard holds is re-sized, not added to
 		free_b += s.dev->big->cached_bytes();      // arena-sized blocks cached in the handle are dropped on demand
 	}
-	uint64_t budget_words = owned ? std::max<uint64_t>(s.d_ptr.n, 1) : (uint64_t)(free_b * 0.45) / 4;
-	if (!need_words) budget_words = UINT64_MAX;
-	if (const char *env = getenv("AT_PTR_BUDGET_MB")) budget_words = (uint64_t)atoll(env) * (1ull << 20) / 4;
-	// packed s16x2 lanes (two pairs per warp): local mode, scores x8 must fit int16, 8|m-u| < 256 (symbols are << 8)
-	const int64_t maxabs = std::max<int64_t>({llabs((long long)b->prm.m), llabs((long long)b->prm.u), llabs((long long)b->prm.o), llabs((long long)b->prm.e), 1});
-	// global / fit (without jump state) also carry -inf inside the 16 bits (AT_NEG16 = -30000, at_cell.cuh): finite values must
-	// stay above -24000 and a -inf value may drift by a few steps' worth of the largest parameter
-	const bool p16_local = b->mode == AT_LOCAL;
-	const bool p16_mode = (p16_local || b->mode == AT_GLOBAL || (b->mode == AT_FIT && !jump)) && llabs((long long)b->prm.m - b->prm.u) <= 31 &&
-	                      (p16_local || maxabs <= 31) && !getenv("AT_NO_P16");
-	auto p16_ok = [&](uint32_t l1, uint32_t l2) {
-		return p16_mode && l1 <= 32u * MAXR && l2 <= 60000u && 8 * (int64_t)(l1 + l2 + 42) * maxabs < (p16_local ? 32000 : 24000);      // + 40: K1 also computes up to 34 columns past l2
-	};
+	pin.budget_words = owned ? std::max<uint64_t>(s.d_ptr.n, 1) : (uint64_t)(free_b * 0.45) / 4;
+	if (!need) pin.budget_words = UINT64_MAX;
+	if (const char *env = getenv("AT_PTR_BUDGET_MB")) pin.budget_words = (uint64_t)atoll(env) * (1ull << 20) / 4;
+	mark("meminfo");
+	Plan plan = make_plan(pin);
+	if (plan.fail_pair != UINT32_MAX) {
+		set_err(h, "pair %llu needs %llu MB of traceback pointers; arena budget is %llu MB", (unsigned long long)(s.p0 + plan.fail_pair),
+		        (unsigned long long)(plan.fail_words >> 18), (unsigned long long)(pin.budget_words >> 18));
+		return AT_E_NOMEM;
+	}
+	mark("plan");
+	// ---- device buffers: results, then what the plan says ----
+	CU(h, s.d_score.alloc(n)); CU(h, s.d_end_i.alloc(n)); CU(h, s.d_end_j.alloc(n)); CU(h, s.d_end_state.alloc(n));
+	CU(h, s.d_beg_i.alloc(n)); CU(h, s.d_beg_j.alloc(n)); CU(h, s.d_n_ops.alloc(n + 1)); CU(h, s.d_n_cols.alloc(n + 1));
+	CU(h, cudaMemsetAsync(s.d_n_ops.p, 0, (n + 1) * sizeof(uint32_t), st));
+	CU(h, cudaMemsetAsync(s.d_n_cols.p, 0, (n + 1) * sizeof(uint32_t), st));
+	CU(h, cudaMemsetAsync(s.d_beg_i.p, 0, n * sizeof(uint32_t), st));
+	CU(h, cudaMemsetAsync(s.d_beg_j.p, 0, n * sizeof(uint32_t), st));
+	CU(h, s.d_counter.alloc(64));
+	CU(h, s.d_rclass.alloc(n));
 	release_chunks(s);      // a pipeline worker reuses its shard (and the shard-level buffers) for every sub-slice
-	// ---- uniform shard: every pair has the same shape and runs on K1 in one chunk -> the plan is closed form ----
-	{
-		if (uniform && need_words && need_words > budget_words) {      // several chunks: the general plan (it needs the per-pair classes)
-			uniform = false;
-			s.h_rclass.assign(n, ptr_class(rclass_of(l1u), 0));
-		}
-		if (uniform) {
-			const bool packed = p16_ok(l1u, l2u) && n >= 2;
-			const uint32_t R = rclass_of(l1u);
-			const uint64_t words_per_job = !b->traceback ? 0 : packed ? ptr_packed_job_words(l2u, R) : pair_ptr_words(0, l1u, l2u);
-			const uint64_t n_jobs = packed ? (n + 1) / 2 : n;
-			s.chunks.emplace_back();
-			Chunk &c = s.chunks.back();
-			c.k0 = 0; c.k1 = n;
-			c.ptr_words = words_per_job * n_jobs;
-			c.scratch_words = b->traceback ? (uint64_t)n * (l1u + l2u) : 0;
-			c.launches.emplace_back();
-			Launch &l = c.launches.back();
-			l.kind = packed ? LK_PACKED : LK_INT32; l.r = (int)R; l.cells = (uint64_t)n * l1u * l2u; l.n_planned = n_jobs;
-			CU(h, l.d_jobs.alloc(n_jobs)); CU(h, c.d_ptr_off.alloc(n)); CU(h, c.d_bnd_off.alloc(n)); CU(h, s.d_rclass.alloc(n));
-			if (b->traceback) { CU(h, c.d_ops_off.alloc(n + 1)); CU(h, c.d_cols_off.alloc(n + 1)); CU(h, c.d_scratch_off.alloc(n)); }
-			// on this stream, behind the uploads; the host does not wait for it (it may sit behind another sub-slice's fill)
-			at_plan_uniform<<<(n + 255) / 256, 256, 0, st>>>(n, packed ? 1 : 0, R, words_per_job, (uint64_t)l1u + l2u, l.d_jobs.p, c.d_ptr_off.p, c.d_bnd_off.p,
-			                                                 b->traceback ? c.d_scratch_off.p : nullptr, s.d_rclass.p);
-			CU(h, cudaGetLastError());
-			h->launches++;
-			s.ptr_bytes = c.ptr_words * 4;
-			CU(h, s.d_bnd.alloc(64)); CU(h, s.d_prog.alloc(1)); CU(h, s.d_chain.alloc(4ull * n + 4));
-			if (c.scratch_words && s.d_scratch.alloc(c.scratch_words) != cudaSuccess) { set_err(h, "traceback scratch of %llu MB", (unsigned long long)(c.scratch_words >> 18)); return AT_E_NOMEM; }
-			if (c.ptr_words) {
-				cudaError_t e = s.d_ptr.alloc(c.ptr_words + (s.workspace && c.ptr_words > s.d_ptr.n ? c.ptr_words / 16 : 0));
-				if (e != cudaSuccess) { set_err(h, "pointer arena of %llu MB: %s", (unsigned long long)(c.ptr_words >> 18), cudaGetErrorString(e)); return AT_E_NOMEM; }
-			}
-			for (auto &e : s.ev) if (!e) CU(h, event_create_timed(&e));
-			for (auto &e : s.evk) if (!e) CU(h, event_create_timed(&e));
-			mark("uniform plan");
-			CU(h, cudaEventSynchronize(s.ev_up));      // the caller's buffers have been read; the plan kernel may still be queued
-			mark("sync");
-			if (trace_setup) fprintf(stderr, "[at setup] pairs %u:%s\n", n, tl_.c_str());
-			return AT_OK;
-		}
-	}
-	uint64_t max_chunk_words = 0, max_scratch_words = 0;
-	{
-		Chunk cur; cur.k0 = 0;
-		uint64_t words = 0;
-		for (uint32_t k = 0; k < n; ++k) {
-			const uint64_t w = pair_words(k);
-			if (w > budget_words) { set_err(h, "pair %llu needs %llu MB of traceback pointers; arena budget is %llu MB",
-			                                (unsigned long long)(s.p0 + k), (unsigned long long)(w >> 18), (unsigned long long)(budget_words >> 18)); return AT_E_NOMEM; }
-			if (words + w > budget_words && k > cur.k0) {
-				cur.k1 = k; s.chunks.push_back(std::move(cur));
-				cur = Chunk(); cur.k0 = k; words = 0;
-			}
-			words += w;
-		}
-		cur.k1 = n; s.chunks.push_back(std::move(cur));
-	}
-	mark("meminfo+chunks");
-	s.ptr_bytes = 0;
-	const bool linear = b->mode >= AT_OVERLAP;          // single-plane modes run on K2 at every length
-	uint64_t max_bnd_elems = 0, max_prog_words = 0;
-	for (auto &c : s.chunks) {
+	s.cells = plan.cells; s.ptr_bytes = 0;
+	// pageable host vectors: each copy is staged before cudaMemcpyAsync returns
+	auto upload = [&](auto &d, const auto &v) -> cudaError_t { return v.empty() ? cudaSuccess : cudaMemcpyAsync(d.p, v.data(), v.size() * sizeof(v[0]), cudaMemcpyHostToDevice, st); };
+	for (PlanChunk &pc : plan.chunks) {
+		s.chunks.emplace_back(std::move(pc));
+		Chunk &c = s.chunks.back();
 		const uint32_t nc = c.k1 - c.k0;
-		auto cells_of = [&](uint32_t k) { return (uint64_t)in->q_len[s.p0 + k] * in->t_len[s.p0 + k]; };
-		auto by_cells = [&](std::vector<uint32_t> &v) {   // largest pairs first (dynamic queue => good tail balance)
-			bool ragged = false;
-			for (size_t x = 1; x < v.size() && !ragged; ++x) ragged = cells_of(v[x]) != cells_of(v[0]);
-			if (ragged) std::stable_sort(v.begin(), v.end(), [&](uint32_t x, uint32_t y) { return cells_of(x) > cells_of(y); });
-		};
-		Launch l32[MAXR + 1], l16[MAXR + 1], lwv[MAXR + 1], lbit[MAXR + 1];
-		std::vector<uint32_t> scalar_pairs, wave_pairs, cand;
-		for (uint32_t k = c.k0; k < c.k1; ++k) {
-			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-			if (linear || band_affine || l1 > 32u * MAXR) wave_pairs.push_back(k);
-			else if (p16_ok(l1, l2)) cand.push_back(k);
-			else scalar_pairs.push_back(k);
+		c.d_jobs.resize(c.launches.size()); c.d_tasks.resize(c.launches.size());
+		for (size_t li = 0; li < c.launches.size(); ++li) {
+			const PlanLaunch &l = c.launches[li];
+			if (l.kind >= LK_WAVE) { CU(h, c.d_tasks[li].alloc(l.n)); CU(h, upload(c.d_tasks[li], l.tasks)); }
+			else { CU(h, c.d_jobs[li].alloc(l.n)); CU(h, upload(c.d_jobs[li], l.jobs)); }
 		}
-		// ---- packed jobs (K1, s16x2): partners must share the rows-per-lane class and l2 ----
-		{
-			// local: the partners share the rows-per-lane class and l2; global / fit: l1 as well (one lane holds the last row of both)
-			auto key = [&](uint32_t k) { return ((uint64_t)(p16_local ? s.h_rclass[k] : in->q_len[s.p0 + k]) << 32) | in->t_len[s.p0 + k]; };
-			bool sorted = true;
-			for (size_t x = 1; x < cand.size() && sorted; ++x) sorted = key(cand[x - 1]) >= key(cand[x]);
-			if (!sorted) std::stable_sort(cand.begin(), cand.end(), [&](uint32_t x, uint32_t y) { return key(x) > key(y); });
-			for (size_t x = 0; x < cand.size();) {
-				if (x + 1 < cand.size() && key(cand[x]) == key(cand[x + 1])) {
-					const int r = ptr_class_r(s.h_rclass[cand[x]]);
-					l16[r].h_jobs.push_back(FillJob{cand[x], cand[x + 1]});
-					l16[r].cells += cells_of(cand[x]) + cells_of(cand[x + 1]);
-					x += 2;
-				} else { scalar_pairs.push_back(cand[x]); x += 1; }
-			}
-		}
-		// ---- int32 jobs (K1) per R class ----
-		by_cells(scalar_pairs);
-		for (uint32_t k : scalar_pairs) { const int r = ptr_class_r(s.h_rclass[k]); l32[r].h_jobs.push_back(FillJob{k, k}); l32[r].cells += cells_of(k); }
-		// ---- wavefront tasks (K2): (pair, stripe), collected pair by pair, then put in queue order (order_wave_tasks) ----
-		by_cells(wave_pairs);
-		c.h_bnd_off.assign(nc, 0);
-		c.bnd_elems = 0; c.prog_words = 0;
-		const int bits_r = s.bits_r;
-		for (uint32_t k : wave_pairs) {
-			const uint32_t l1 = in->q_len[s.p0 + k], l2 = in->t_len[s.p0 + k];
-			const int r = s.bits ? bits_r : ptr_class_r(s.h_rclass[k]);
-			const uint32_t rows = s.bits ? edit_bits_rows(r) : 32u * r;
-			Launch &lw = s.bits ? lbit[r] : lwv[r];
-			const uint32_t n_stripes = (l1 + rows - 1) / rows;
-			uint32_t queued = 0;
-			for (uint32_t st2 = 0; st2 < n_stripes; ++st2) {
-				// banded: only stripes with a window run; the last stripe always does (it writes the end cell; banded global:
-				// the end diagonal is in band, so the last stripe has a window)
-				BandWin w;
-				if (s.banded && st2 + 1 < n_stripes && !band_stripe(l1, l2, s.h_band[k].x, s.h_band[k].y, rows, st2, w)) continue;
-				lw.h_tasks.push_back(WaveTask{k, st2, 0, 0});
-				++queued;
-			}
-			lw.cells += s.banded ? pair_cells(k, l1, l2) : cells_of(k);
-			if (queued > 1) { c.h_bnd_off[k - c.k0] = c.bnd_elems; c.bnd_elems += 2ull * ((l2 + 4u) & ~3u); }
-		}
-		for (int r = 1; r <= MAXR; ++r) {
-			if (!l32[r].h_jobs.empty()) { l32[r].kind = LK_INT32; l32[r].r = r; c.launches.push_back(std::move(l32[r])); }
-			if (!l16[r].h_jobs.empty()) { l16[r].kind = LK_PACKED; l16[r].r = r; c.launches.push_back(std::move(l16[r])); }
-			order_wave_tasks(lwv[r].h_tasks); order_wave_tasks(lbit[r].h_tasks);
-			if (!lwv[r].h_tasks.empty()) {
-				lwv[r].kind = LK_WAVE; lwv[r].r = r; lwv[r].prog_base = c.prog_words; c.prog_words += lwv[r].h_tasks.size();
-				c.launches.push_back(std::move(lwv[r]));
-			}
-			if (!lbit[r].h_tasks.empty()) {
-				lbit[r].kind = LK_BITS; lbit[r].r = r; lbit[r].prog_base = c.prog_words; c.prog_words += lbit[r].h_tasks.size();
-				c.launches.push_back(std::move(lbit[r]));
-			}
-		}
-		max_bnd_elems = std::max(max_bnd_elems, c.bnd_elems);
-		max_prog_words = std::max(max_prog_words, c.prog_words);
-		// ---- pointer blocks: one per int32 / wavefront pair, one per packed job (shared by its two pairs) ----
-		c.h_ptr_off.assign(nc, 0);
-		uint64_t words = 0;
-		if (b->traceback) {
-			for (const Launch &l : c.launches) {
-				if (l.kind == LK_PACKED) {
-					for (const FillJob &jb : l.h_jobs) {
-						c.h_ptr_off[jb.a - c.k0] = words; c.h_ptr_off[jb.b - c.k0] = words;
-						s.h_rclass[jb.a] = ptr_class(l.r, 1); s.h_rclass[jb.b] = ptr_class(l.r, 2);
-						words += ptr_packed_job_words(in->t_len[s.p0 + jb.a], l.r);
-					}
-				} else if (l.kind == LK_INT32) {
-					for (const FillJob &jb : l.h_jobs) { const uint32_t k = jb.a; c.h_ptr_off[k - c.k0] = words; words += pair_ptr_words(k, in->q_len[s.p0 + k], in->t_len[s.p0 + k]); }
-				} else {
-					// a pair's block goes where its first task is queued (stripe 0 unless the band leaves stripe 0 out)
-					std::vector<uint8_t> placed(nc, 0);
-					for (const WaveTask &tk : l.h_tasks) {
-						const uint32_t k = tk.pair;
-						if (placed[k - c.k0]) continue;
-						placed[k - c.k0] = 1;
-						c.h_ptr_off[k - c.k0] = words; words += pair_ptr_words(k, in->q_len[s.p0 + k], in->t_len[s.p0 + k]);
-					}
-				}
-			}
-		}
-		c.ptr_words = words;
-		max_chunk_words = std::max(max_chunk_words, c.ptr_words);
-		s.ptr_bytes += c.ptr_words * 4;
-		for (Launch &l : c.launches) {
-			if (l.kind >= LK_WAVE) {
-				CU(h, l.d_tasks.alloc(l.h_tasks.size()));
-				CU(h, cudaMemcpyAsync(l.d_tasks.p, l.h_tasks.data(), l.h_tasks.size() * sizeof(WaveTask), cudaMemcpyHostToDevice, st));
-			} else {
-				CU(h, l.d_jobs.alloc(l.h_jobs.size()));
-				CU(h, cudaMemcpyAsync(l.d_jobs.p, l.h_jobs.data(), l.h_jobs.size() * sizeof(FillJob), cudaMemcpyHostToDevice, st));
-			}
-		}
-		CU(h, c.d_ptr_off.alloc(nc));
-		CU(h, cudaMemcpyAsync(c.d_ptr_off.p, c.h_ptr_off.data(), nc * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-		CU(h, c.d_bnd_off.alloc(nc));
-		CU(h, cudaMemcpyAsync(c.d_bnd_off.p, c.h_bnd_off.data(), nc * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+		CU(h, c.d_ptr_off.alloc(nc)); CU(h, upload(c.d_ptr_off, c.ptr_off));
+		CU(h, c.d_bnd_off.alloc(nc)); CU(h, upload(c.d_bnd_off, c.bnd_off));
 		if (b->traceback) {
 			CU(h, c.d_ops_off.alloc(nc + 1)); CU(h, c.d_cols_off.alloc(nc + 1));
-			// traceback scratch: a slot of l1+l2 run-length ops per pair (an alignment has at most l1+l2 columns)
-			c.h_scratch_off.resize(nc);
-			uint64_t sw = 0;
-			for (uint32_t k = 0; k < nc; ++k) { c.h_scratch_off[k] = sw; sw += (uint64_t)in->q_len[s.p0 + c.k0 + k] + in->t_len[s.p0 + c.k0 + k]; }
-			c.scratch_words = sw;
-			max_scratch_words = std::max(max_scratch_words, sw);
-			CU(h, c.d_scratch_off.alloc(nc));
-			CU(h, cudaMemcpyAsync(c.d_scratch_off.p, c.h_scratch_off.data(), nc * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
+			CU(h, c.d_scratch_off.alloc(nc)); CU(h, upload(c.d_scratch_off, c.scratch_off));
 		}
+		s.ptr_bytes += c.ptr_words * 4;
 	}
-	mark("plan+jobs");
-	if (max_bnd_elems && s.d_bnd.alloc(max_bnd_elems * (linear ? sizeof(uint64_t) : sizeof(int4)) + 64) != cudaSuccess) { set_err(h, "stripe boundary slabs of %llu MB", (unsigned long long)((max_bnd_elems * (linear ? 8 : 16)) >> 20)); return AT_E_NOMEM; }
-	if (!max_bnd_elems) CU(h, s.d_bnd.alloc(64));
-	CU(h, s.d_prog.alloc(max_prog_words + 1));
-	{
-		uint32_t max_nc = 0;
-		for (auto &c : s.chunks) max_nc = std::max(max_nc, c.k1 - c.k0);
-		CU(h, s.d_chain.alloc(4ull * max_nc + 4));
-	}
-	if (max_scratch_words && s.d_scratch.alloc(max_scratch_words) != cudaSuccess) { set_err(h, "traceback scratch of %llu MB", (unsigned long long)(max_scratch_words >> 18)); return AT_E_NOMEM; }
-	CU(h, s.d_rclass.alloc(n));
-	CU(h, cudaMemcpyAsync(s.d_rclass.p, s.h_rclass.data(), n, cudaMemcpyHostToDevice, st));
-	if (max_chunk_words) {
-		cudaError_t e = s.d_ptr.alloc(max_chunk_words + (s.workspace && max_chunk_words > s.d_ptr.n ? max_chunk_words / 16 : 0));
-		if (e != cudaSuccess) { set_err(h, "pointer arena of %llu MB: %s", (unsigned long long)(max_chunk_words >> 18), cudaGetErrorString(e)); return AT_E_NOMEM; }
+	if (plan.uniform) {
+		// on this stream, behind the uploads; the host does not wait for it (it may sit behind another sub-slice's fill)
+		Chunk &c = s.chunks[0];
+		at_plan_uniform<<<(n + 255) / 256, 256, 0, st>>>(n, plan.u, c.d_jobs[0].p, c.d_ptr_off.p, c.d_bnd_off.p, b->traceback ? c.d_scratch_off.p : nullptr, s.d_rclass.p);
+		CU(h, cudaGetLastError());
+		h->launches++;
+	} else CU(h, upload(s.d_rclass, plan.rclass));
+	mark("jobs");
+	const bool linear = b->mode >= AT_OVERLAP;      // the single-plane kernels' boundary slabs hold 8-byte elements
+	if (plan.max_bnd_elems && s.d_bnd.alloc(plan.max_bnd_elems * (linear ? sizeof(uint64_t) : sizeof(int4)) + 64) != cudaSuccess) { set_err(h, "stripe boundary slabs of %llu MB", (unsigned long long)((plan.max_bnd_elems * (linear ? 8 : 16)) >> 20)); return AT_E_NOMEM; }
+	if (!plan.max_bnd_elems) CU(h, s.d_bnd.alloc(64));
+	CU(h, s.d_prog.alloc(plan.max_prog_words + 1));
+	CU(h, s.d_chain.alloc(4ull * plan.max_pairs + 4));
+	if (plan.max_scratch_words && s.d_scratch.alloc(plan.max_scratch_words) != cudaSuccess) { set_err(h, "traceback scratch of %llu MB", (unsigned long long)(plan.max_scratch_words >> 18)); return AT_E_NOMEM; }
+	if (plan.max_chunk_words) {
+		cudaError_t e = s.d_ptr.alloc(plan.max_chunk_words + (s.workspace && plan.max_chunk_words > s.d_ptr.n ? plan.max_chunk_words / 16 : 0));
+		if (e != cudaSuccess) { set_err(h, "pointer arena of %llu MB: %s", (unsigned long long)(plan.max_chunk_words >> 18), cudaGetErrorString(e)); return AT_E_NOMEM; }
 	}
 	for (auto &e : s.ev) if (!e) CU(h, event_create_timed(&e));
 	for (auto &e : s.evk) if (!e) CU(h, event_create_timed(&e));
 	mark("arena");
 	// the ONE synchronisation of the set-up: every upload has left the caller's buffers (they may be reused or freed once
-	// at_batch_create / the sub-slice's set-up returns) and the shard's own host vectors
-	CU(h, shard_sync(s));
+	// at_batch_create / the sub-slice's set-up returns) and the plan's host vectors.  A uniform plan uploads nothing from
+	// the host: the sequence copies are all it waits for, not the plan kernel (which may be queued behind another fill).
+	CU(h, plan.uniform ? cudaEventSynchronize(s.ev_up) : shard_sync(s));
 	mark("sync");
 	if (trace_setup) fprintf(stderr, "[at setup] pairs %u:%s\n", n, tl_.c_str());
 	return AT_OK;
@@ -950,50 +684,12 @@ static int validate_batch(at_handle *h, int mode, const at_params *p, const at_b
 	return AT_OK;
 }
 
-// the same slicing rule as cut_by_cells, from running cell counts (binary searches instead of passes over the pairs)
-static void cut_by_prefix(const std::vector<uint64_t> &prefix, uint64_t lo, uint64_t hi, size_t parts, std::vector<uint64_t> &cut)
-{
-	cut.assign(parts + 1, lo);
-	cut[parts] = hi;
-	if (parts <= 1) return;
-	const uint64_t base = prefix[lo], total = prefix[hi] - base;
-	for (size_t d = 1; d < parts; ++d) {
-		// smallest k in [lo, hi) with (prefix[k+1] - base) * parts >= total * d; the slice ends after it
-		uint64_t a = lo, b = hi;
-		while (a < b) {
-			const uint64_t mid = a + (b - a) / 2;
-			if ((unsigned __int128)(prefix[mid + 1] - base) * parts >= (unsigned __int128)total * d) b = mid; else a = mid + 1;
-		}
-		cut[d] = a < hi ? a + 1 : hi;
-	}
-	for (size_t d = 1; d <= parts; ++d) cut[d] = std::max(cut[d], cut[d - 1]);
-}
-
-// contiguous slices of [lo, hi) with (nearly) equal numbers of cells; cut has parts + 1 entries
-static void cut_by_cells(const at_batch_input *in, uint64_t lo, uint64_t hi, size_t parts, std::vector<uint64_t> &cut)
-{
-	cut.assign(parts + 1, lo);
-	cut[parts] = hi;
-	if (parts <= 1) return;
-	uint64_t total = 0;                       // sum of l1*l2 <= 2^31 pairs x 2^54 would overflow; validate_batch bounds l1+l2 < 2^27
-	for (uint64_t k = lo; k < hi; ++k) total += (uint64_t)in->q_len[k] * in->t_len[k];
-	uint64_t acc = 0; size_t d = 1;
-	for (uint64_t k = lo; k < hi && d < parts; ++k) {
-		acc += (uint64_t)in->q_len[k] * in->t_len[k];
-		while (d < parts && (unsigned __int128)acc * parts >= (unsigned __int128)total * d) { cut[d++] = k + 1; }
-	}
-	for (; d < parts; ++d) cut[d] = hi;
-	cut[parts] = hi;
-}
-
 extern "C" int at_plan_slices(const uint32_t *q_len, const uint32_t *t_len, uint64_t n_pairs, uint32_t parts, uint64_t *cut)
 {
 	if (!q_len || !t_len || !cut || parts == 0) return AT_E_ARG;
-	at_batch_input in;
-	memset(&in, 0, sizeof in);
-	in.n_pairs = n_pairs; in.q_len = q_len; in.t_len = t_len;
-	std::vector<uint64_t> c;
-	cut_by_cells(&in, 0, n_pairs, parts, c);
+	std::vector<uint64_t> prefix(n_pairs + 1, 0), c;
+	for (uint64_t k = 0; k < n_pairs; ++k) prefix[k + 1] = prefix[k] + (uint64_t)q_len[k] * t_len[k];
+	cut_by_prefix(prefix, 0, n_pairs, parts, c);
 	for (uint32_t k = 0; k <= parts; ++k) cut[k] = c[k];
 	return AT_OK;
 }
@@ -1033,16 +729,15 @@ static int validate_band(at_handle *h, int mode, const at_batch_input *in, const
 	return AT_OK;
 }
 
-// K2 tasks of a banded global batch: every pair runs on K2, one task per stripe of 256 rows with a window (at_band.h)
+// K2 tasks of a banded global batch: every pair runs on K2, one task per queued stripe of 256 rows (at_plan.h)
 static uint64_t banded_global_tasks(const at_batch_input *in, const at_band *band)
 {
 	uint64_t n = 0;
 	for (uint64_t k = 0; k < in->n_pairs; ++k) {
 		const uint32_t l1 = in->q_len[k], l2 = in->t_len[k], RPP = 32u * MAXR;
-		int32_t elo, ehi;
-		band_clip(l1, l2, band->lo[k], band->hi[k], elo, ehi);
-		BandWin w;
-		for (uint32_t s = (l1 + RPP - 1) / RPP; s-- > 0 && band_stripe(l1, l2, elo, ehi, RPP, s, w, PTR_SH_NIB);) ++n;      // the windows are the bottom run
+		PairBand bd;
+		band_clip(l1, l2, band->lo[k], band->hi[k], bd.lo, bd.hi);
+		for (uint32_t s = 0; s < (l1 + RPP - 1) / RPP; ++s) n += band_stripe_queued(l1, l2, bd, RPP, s);
 	}
 	return n;
 }
@@ -1058,13 +753,13 @@ extern "C" int at_batch_create_banded(at_handle *h, int mode, const at_params *p
 {
 	if (!h || !p || !in || !out) return AT_E_ARG;
 	*out = nullptr;
-	if (int rc = validate_batch(h, mode, p, in)) return rc;
+	// contiguous slices balanced by cells (one device: no running cell counts needed)
+	const size_t nd = h->devs.size();
+	std::vector<uint64_t> prefix, cut;
+	if (int rc = validate_batch(h, mode, p, in, nd > 1 ? &prefix : nullptr)) return rc;
 	if (int rc = validate_band(h, mode, in, band)) return rc;
 	at_batch *b = new_batch(h, mode, p, out_flags, in->n_pairs);
-	// contiguous slices balanced by cells
-	const size_t nd = h->devs.size();
-	std::vector<uint64_t> cut;
-	cut_by_cells(in, 0, b->n, nd, cut);
+	cut_by_prefix(prefix, 0, b->n, nd, cut);
 	b->shards.resize(nd);
 	std::vector<std::thread> th;
 	for (size_t d = 0; d < nd; ++d) {
@@ -1175,7 +870,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 		CU(h, cudaEventRecord(e_begin, st));
 		if (first) { CU(h, cudaEventRecord(e_first, st)); first = false; }
 		for (size_t li = 0; li < c.launches.size(); ++li) {
-			Launch &l = c.launches[li];
+			const PlanLaunch &l = c.launches[li];
 			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r, b->traceback) : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(b->mode, l.r, s.prof) : (const void *)wave_kernel(b->mode, jump, l.r, s.prof, b->traceback))
 			                                   : (const void *)affine_kernel(l.kind == LK_PACKED ? (b->mode == AT_LOCAL ? 4 : b->mode == AT_GLOBAL ? 5 : 6) : (b->mode == AT_FIT ? (jump ? 3 : 2) : b->mode), l.r, s.prof);
 			const int warps = l.kind >= LK_WAVE ? AT_WAVE_WARPS : AT_FILL_WARPS;
@@ -1187,7 +882,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 			// AT_PIPE_TB_OVERLAP (older scheme, kept for A/B runs): traceback kernels run beside the next sub-slice's
 			// fill, which must then leave them shared memory and registers (a K1 grid at full occupancy fills an SM)
 			if (tb_overlap && s.workspace && l.kind != LK_WAVE && l.kind != LK_BITS && occ > 4) occ = 4;
-			int blocks = (int)std::min<uint64_t>((uint64_t)s.dev->sm_count * occ, (l.n_jobs() + warps - 1) / warps);
+			int blocks = (int)std::min<uint64_t>((uint64_t)s.dev->sm_count * occ, (l.n + warps - 1) / warps);
 			if (blocks < 1) blocks = 1;
 			const bool dom = (int)ci == dom_chunk && (int)li == dom_launch;
 			if (dom) CU(h, cudaEventRecord(s.evk[0], st));
@@ -1196,7 +891,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 				wa.symmap = s.d_symmap.p; wa.syms = s.syms;
 				wa.q = s.d_q.p; wa.q_off = s.d_q_off.p; wa.q_len = s.d_q_len.p;
 				wa.t = s.d_t.p; wa.t_off = s.d_t_off.p; wa.t_len = s.d_t_len.p;
-				wa.jmask = s.d_jmask.p; wa.j_off = s.twobit && jump ? s.d_j_off.p : s.d_t_off.p; wa.twobit = s.twobit ? 1 : 0; wa.start_lag = wave_start_lag(); wa.tasks = l.d_tasks.p; wa.n_tasks = (uint32_t)l.h_tasks.size();
+				wa.jmask = s.d_jmask.p; wa.j_off = s.twobit && jump ? s.d_j_off.p : s.d_t_off.p; wa.twobit = s.twobit ? 1 : 0; wa.start_lag = wave_start_lag(); wa.tasks = c.d_tasks[li].p; wa.n_tasks = l.n;
 				wa.counter = s.d_counter.p + (l.kind == LK_BITS ? 48 : 32) + l.r; wa.prog = s.d_prog.p + l.prog_base;
 				wa.ptr = s.d_ptr.p; wa.ptr_off = c.d_ptr_off.p; wa.pair_base = c.k0;
 				wa.bnd = s.d_bnd.p; wa.bnd_off = c.d_bnd_off.p; wa.chain = s.d_chain.p;
@@ -1212,7 +907,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 				fa.q = s.d_q.p; fa.q_off = s.d_q_off.p; fa.q_len = s.d_q_len.p;
 				fa.t = s.d_t.p; fa.t_off = s.d_t_off.p; fa.t_len = s.d_t_len.p;
 				fa.jmask = s.d_jmask.p; fa.j_off = s.twobit && jump ? s.d_j_off.p : s.d_t_off.p; fa.symmap = s.d_symmap.p; fa.syms = s.syms;
-				fa.jobs = l.d_jobs.p; fa.n_jobs = (uint32_t)l.n_jobs();
+				fa.jobs = c.d_jobs[li].p; fa.n_jobs = l.n;
 				fa.counter = s.d_counter.p + (l.kind == LK_PACKED ? 16 : 0) + l.r; fa.ptr = s.d_ptr.p; fa.ptr_off = c.d_ptr_off.p; fa.pair_base = c.k0;
 				fa.score = s.d_score.p; fa.end_i = s.d_end_i.p; fa.end_j = s.d_end_j.p; fa.end_state = s.d_end_state.p;
 				fa.m = b->prm.m; fa.u = b->prm.u; fa.o = b->prm.o; fa.e = b->prm.e; fa.jp = b->prm.j;
@@ -1320,7 +1015,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 		CU(h, cudaEventElapsedTime(&ms, e_fill, e_tb)); s.tb_ms += ms;
 		if ((int)ci == dom_chunk) {
 			CU(h, cudaEventElapsedTime(&ms, s.evk[0], s.evk[1])); s.domk_ms = ms; s.domk_cells = dom_cells;
-			const Launch &dl = c.launches[dom_launch];
+			const PlanLaunch &dl = c.launches[dom_launch];
 			s.domk_kind = (uint32_t)dl.kind; s.domk_r = (uint32_t)dl.r; s.domk_flags = (s.prof ? 1u : 0u) | (jump ? 2u : 0u) | (s.twobit ? 4u : 0u);
 		}
 		if (ci + 1 == s.chunks.size()) { CU(h, cudaEventElapsedTime(&ms, e_first, e_tb)); s.dev_ms = ms; }

@@ -3,7 +3,7 @@
 //
 // A pair is cut into STRIPES of 32*R rows.  Every (pair, stripe) is a task; the persistent grid
 // claims tasks IN ORDER from an atomic queue, one warp per task.  The queue lists stripe after stripe
-// across the launch's pairs (order_wave_tasks, at_runtime.cu): stripes of one pair that happen to be
+// across the launch's pairs (order_wave_tasks, at_plan.h): stripes of one pair that happen to be
 // resident together run concurrently on different warps / CTAs / SMs, each at least two 32-column blocks
 // behind the one above; stripes claimed later find their predecessor finished.  Inside a
 // stripe the warp is the same systolic array as K1 (lane k owns R rows, column j = t - k).
@@ -28,6 +28,7 @@
 // :940-949 (overlap), :303-311 (edit); tie rules SURVEY.md A.0.
 #pragma once
 #include <type_traits>
+#include "at_plan.h"      // WaveTask
 
 namespace atb2 {
 
@@ -45,16 +46,12 @@ constexpr int AT_WAVE_UNROLL_AFFINE = AT_WAVE_UNROLL_AFFINE_N;     // steps per 
 constexpr int AT_WAVE_UNROLL_OVERLAP = 4, AT_WAVE_UNROLL_EDIT = 8;
 #define AT_PROG_DONE 0xffffffffu
 
-// One unit of K2 work: stripe `stripe` of pair `pair`.  `prev` is the queue index of the same pair's stripe above it (its
-// own index for stripe 0): the affine kernel waits on that task's progress word.
-struct __align__(16) WaveTask { uint32_t pair, stripe, prev, reserved; };
-
 struct WaveArgs {
 	const uint8_t  *q;       const uint64_t *q_off;  const uint32_t *q_len;
 	const uint8_t  *t;       const uint64_t *t_off;  const uint32_t *t_len;
 	const uint8_t  *jmask;   // fit+jump: 1 where entering J is forbidden, one byte per target symbol
 	const uint64_t *j_off;   // [pair] offset of the pair's mask (byte-encoded targets: the same array as t_off)
-	const WaveTask *tasks;   // the queue: a pair's stripes in ascending order (the host interleaves the pairs, at_runtime.cu)
+	const WaveTask *tasks;   // the queue: a pair's stripes in ascending order (the host interleaves the pairs, at_plan.h)
 	uint32_t        n_tasks;
 	uint32_t       *counter; // task queue head
 	uint32_t       *prog;    // [n_tasks] columns of the task's last row that are visible in its slab
