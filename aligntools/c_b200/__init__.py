@@ -32,7 +32,7 @@ EXPORTS = ["at_default_params", "at_strerror", "at_version", "at_create", "at_de
            "at_align_fit_affine_jump", "at_align_overlap", "at_edit_dist", "at_batch_create",
            "at_batch_run", "at_batch_sizes", "at_batch_fetch", "at_batch_free", "at_batch_align",
            "at_pack_2bit", "at_cigar_to_string", "at_plan_slices", "at_host_alloc", "at_host_free", "at_host_register", "at_host_unregister",
-           "at_batch_create_banded", "at_batch_align_banded"]
+           "at_batch_create_banded", "at_batch_align_banded", "at_batch_create_scored", "at_batch_align_scored"]
 
 
 class AtError(RuntimeError):
@@ -63,6 +63,48 @@ def _band_arrays(band, n):
         return None
     lo, hi = (np.ascontiguousarray(np.broadcast_to(np.asarray(x, dtype=np.int32), (n,))) for x in band)
     return lo, hi
+
+
+class _Scoring(C.Structure):
+    _fields_ = [("matrix", C.c_void_p)]
+
+
+def _scoring_matrix(scoring):
+    """scoring: None, or a 256 x 256 int8 substitution table, s(a, b) = scoring[a, b] for read byte a and target byte b."""
+    if scoring is None:
+        return None
+    m = np.asarray(scoring)
+    if m.shape != (256, 256):
+        raise ValueError("scoring: a 256 x 256 table of int8 scores is expected")
+    if m.dtype != np.int8:
+        if m.min(initial=0) < -128 or m.max(initial=0) > 127:
+            raise ValueError("scoring: entries must fit int8")
+        m = m.astype(np.int8)
+    return np.ascontiguousarray(m)
+
+
+def scoring_matrix(alphabet, scores, default=0):
+    """A 256 x 256 int8 substitution table from a K-letter alphabet (bytes or str) and a K x K table of scores:
+    s(alphabet[a], alphabet[b]) = scores[a][b]; every pair with a byte outside the alphabet scores `default`.
+    Example, DNA with transitions scored above transversions and N neutral:
+        scoring_matrix("ACGTN", [[2, -3, -1, -3, 0], [-3, 2, -3, -1, 0], [-1, -3, 2, -3, 0], [-3, -1, -3, 2, 0], [0] * 5])"""
+    ab = alphabet.encode() if isinstance(alphabet, str) else bytes(alphabet)
+    sc = np.asarray(scores, dtype=np.int64)
+    if len(set(ab)) != len(ab) or sc.shape != (len(ab), len(ab)):
+        raise ValueError("scoring_matrix: distinct letters and a K x K score table are expected")
+    if sc.min(initial=0) < -128 or sc.max(initial=0) > 127 or not -128 <= default <= 127:
+        raise ValueError("scoring_matrix: scores must fit int8")
+    m = np.full((256, 256), default, dtype=np.int8)
+    idx = np.frombuffer(ab, dtype=np.uint8)
+    m[np.ix_(idx, idx)] = sc.astype(np.int8)
+    return m
+
+
+def identity_scoring(m, u):
+    """The table that scores like match / mismatch: m on equal bytes, u otherwise (at_batch_align's scoring)."""
+    t = np.full((256, 256), u, dtype=np.int8)
+    np.fill_diagonal(t, m)
+    return t
 
 
 class _Output(C.Structure):
@@ -123,6 +165,10 @@ def load_library():
     lib.at_batch_create_banded.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Params), C.POINTER(_Input), C.POINTER(_Band),
                                            C.c_uint32, C.POINTER(C.c_void_p)]
     lib.at_batch_align_banded.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Params), C.POINTER(_Input), C.POINTER(_Band),
+                                          C.c_uint32, C.POINTER(_Output), C.POINTER(_Timing)]
+    lib.at_batch_create_scored.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Params), C.POINTER(_Input), C.POINTER(_Scoring),
+                                           C.c_uint32, C.POINTER(C.c_void_p)]
+    lib.at_batch_align_scored.argtypes = [C.c_void_p, C.c_int, C.POINTER(_Params), C.POINTER(_Input), C.POINTER(_Scoring),
                                           C.c_uint32, C.POINTER(_Output), C.POINTER(_Timing)]
     lib.at_pack_2bit.restype = C.c_int64
     lib.at_pack_2bit.argtypes = [C.c_char_p, C.c_uint64, C.c_void_p]
@@ -274,10 +320,11 @@ class Batch:
     """A batch resident on the device(s): create (H2D) -> run (kernels) -> fetch (D2H)."""
 
     def __init__(self, aligner, mode, opt, q, q_off, q_len, t, t_off, t_len, sites=None, site_off=None,
-                 out_flags=OUT_CIGAR | OUT_ALN, encoding=SEQ_BYTES, band=None):
+                 out_flags=OUT_CIGAR | OUT_ALN, encoding=SEQ_BYTES, band=None, scoring=None):
         """band: None, or (lo, hi) -- per-pair int32 diagonals (d = j - i) of a banded "overlap" or "global" alignment
         (at_batch_create_banded; a global pair's band must hold its end diagonal l2 - l1); a scalar applies to every
-        pair."""
+        pair.  scoring: None, or a 256 x 256 int8 substitution table (at_batch_create_scored; see scoring_matrix) for
+        "global", "local", "fit" or "overlap"; it takes no band."""
         self.al = aligner
         self.lib = aligner.lib
         self.n = int(len(q_len))
@@ -298,7 +345,14 @@ class Batch:
         self.h = C.c_void_p()
         prm = opt.c()
         self._band = _band_arrays(band, self.n)
-        if self._band is None:
+        self._scoring = _scoring_matrix(scoring)
+        if self._scoring is not None:
+            if self._band is not None:
+                raise ValueError("scoring: a substitution matrix takes no band")
+            sc = _Scoring(self._scoring.ctypes.data)
+            rc = self.lib.at_batch_create_scored(aligner.h, self.mode, C.byref(prm), C.byref(inp), C.byref(sc), out_flags,
+                                                 C.byref(self.h))
+        elif self._band is None:
             rc = self.lib.at_batch_create(aligner.h, self.mode, C.byref(prm), C.byref(inp), out_flags, C.byref(self.h))
         else:
             bd = _Band(self._band[0].ctypes.data, self._band[1].ctypes.data)
@@ -377,13 +431,14 @@ class Aligner:
 
     def align_arrays(self, mode, opt, q, q_off, q_len, t, t_off, t_len, sites=None, site_off=None,
                      out_flags=OUT_CIGAR, encoding=SEQ_BYTES, out: BatchResult = None,
-                     cigar_cap=None, aln_cap=None, band=None) -> BatchResult:
+                     cigar_cap=None, aln_cap=None, band=None, scoring=None) -> BatchResult:
         """One-shot at_batch_align (host arrays in, host arrays out; large batches are pipelined
         H2D / kernels / D2H inside the library).  `out` may be a BatchResult from a previous call
         whose buffers are reused; capacities default to the worst case (l1 + l2 per pair) for
         the alignment strings and for the CIGARs (32 ops per pair once that exceeds 64 Mi ops;
         AT_E_NOSPACE tells when to pass a larger cigar_cap).  band: (lo, hi) per-pair diagonals of a banded "overlap" or
-        "global" alignment (at_batch_align_banded), or None."""
+        "global" alignment (at_batch_align_banded), or None.  scoring: a 256 x 256 int8 substitution table
+        (at_batch_align_scored), or None."""
         md = _mode(mode)
         n = int(len(q_len))
         res = out if out is not None else BatchResult(n)
@@ -415,7 +470,13 @@ class Aligner:
         prm = opt.c()
         tm = _Timing()
         bnd = _band_arrays(band, n)
-        if bnd is None:
+        mat = _scoring_matrix(scoring)
+        if mat is not None:
+            if bnd is not None:
+                raise ValueError("scoring: a substitution matrix takes no band")
+            rc = self.lib.at_batch_align_scored(self.h, md, C.byref(prm), C.byref(inp), C.byref(_Scoring(mat.ctypes.data)), out_flags,
+                                                C.byref(o), C.byref(tm))
+        elif bnd is None:
             rc = self.lib.at_batch_align(self.h, md, C.byref(prm), C.byref(inp), out_flags, C.byref(o), C.byref(tm))
         else:
             bd = _Band(bnd[0].ctypes.data, bnd[1].ctypes.data)
@@ -426,8 +487,10 @@ class Aligner:
                             tm.fill_kernel_ms, tm.fill_kernel_cells, tm.fill_kernel_kind, tm.fill_kernel_rows, tm.fill_kernel_flags)
         return res
 
-    def align(self, mode, reads, targets, opt: Opt = None, sites=None, out_flags=OUT_CIGAR | OUT_ALN, band=None) -> BatchResult:
-        """Lists of bytes in, BatchResult out (create + run + fetch).  band: (lo, hi) diagonals, "overlap" or "global"."""
+    def align(self, mode, reads, targets, opt: Opt = None, sites=None, out_flags=OUT_CIGAR | OUT_ALN, band=None,
+              scoring=None) -> BatchResult:
+        """Lists of bytes in, BatchResult out (create + run + fetch).  band: (lo, hi) diagonals, "overlap" or "global".
+        scoring: a 256 x 256 int8 substitution table (see scoring_matrix), or None."""
         opt = opt or Opt()
         q, qo, ql = pack_seqs(reads)
         t, to, tl = pack_seqs(targets)
@@ -438,7 +501,7 @@ class Aligner:
             sa = np.array(flat + [0], dtype=np.int32)
             so = np.zeros(len(reads) + 1, np.uint64)
             np.cumsum([len(s or []) for s in sites], out=so[1:])
-        b = Batch(self, mode, opt, q, qo, ql, t, to, tl, sites=sa, site_off=so, out_flags=out_flags, band=band)
+        b = Batch(self, mode, opt, q, qo, ql, t, to, tl, sites=sa, site_off=so, out_flags=out_flags, band=band, scoring=scoring)
         try:
             tm = b.run()
             res = b.fetch()

@@ -54,6 +54,8 @@ __host__ __device__ constexpr size_t fill_smem_bytes(int R, bool packed, bool pr
 	return (size_t)AT_FILL_WARPS * (prof ? (size_t)(AT_RING + AT_RING_MIRROR) * 2 + (size_t)prof_combs(packed) * 32 * k1_lane_stride(R) * 4
 	                                     : (size_t)(AT_RING + AT_RING_MIRROR) * 4);
 }
+// ... and of at_fill_affine<.., R, false, false, false, true> (table variant): the same, then the shard's compact table
+__host__ __device__ constexpr size_t fill_smem_bytes_table(int R, uint32_t table_bytes) { return fill_smem_bytes(R, false, false) + table_bytes; }
 
 struct FillArgs2 {
 	const uint8_t  *q;       const uint64_t *q_off;  const uint32_t *q_len;
@@ -71,13 +73,20 @@ struct FillArgs2 {
 	int             want_ptr;
 	uint32_t        k_and, k_or;   // cell_k_and / cell_k_or of the lane type (at_cell.cuh: constants that must stay in registers)
 	int             twobit;  // PROF: q / t hold 2-bit codes (AT_SEQ_2BIT, four symbols per byte, byte-aligned records; *_off are byte offsets)
+	SubstArgs       sub;     // SCORED: the substitution matrix (at_kernels.cuh)
 };
 
 // packed lanes with up to five rows per lane (the 150-row reads of BASELINE config 2 are R = 5): hold ptxas to the 96 registers
 // that let five CTAs share an SM -- the shared-memory profile allows exactly five; the other variants to 128 / 168 / 255
-template <int MODE, int R, bool JUMP, bool PACKED, bool PROF>
+// SCORED (substitution matrix, at_batch_*_scored): with PROF the profile words come from the matrix row of the read symbol
+// (the cell is unchanged); without PROF (int32 lanes only) the TABLE variant: ac[r] holds the byte offset of the row's read
+// code in the shard's compact table (shared memory, after the warps' rings), the ring holds 2 x the column's target code
+// (| blacklist bit), and 8 s(i, j) is one LDS.S16 from their sum.
+template <int MODE, int R, bool JUMP, bool PACKED, bool PROF, bool SCORED = false>
 __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (JUMP && R > 5) ? 2 : (JUMP || R > 6) ? 3 : 4) at_fill_affine(const FillArgs2 a)
 {
+	static_assert(!SCORED || PROF || !PACKED, "the table variant runs on int32 lanes");
+	constexpr bool TABLE = SCORED && !PROF;
 	typedef Lanes<PACKED> V;
 	typedef typename V::T T;
 	static_assert(!PACKED || !JUMP, "packed lanes: no jump state");
@@ -97,6 +106,12 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 	uint16_t *ring16 = (uint16_t *)warp_smem;                                 // PROF: byte offset of the column's comb (| blacklist bit)
 	uint32_t *prof = (uint32_t *)(warp_smem + (AT_RING + AT_RING_MIRROR) * 2);   // PROF: [NC][32][LS]
 	const unsigned char *prof_lane = (const unsigned char *)(prof + lane * LS);
+	const unsigned char *tab = fill_smem + (TABLE ? fill_smem_bytes(R, false, false) : 0);      // TABLE: [read code][target code] of 8 s
+	if constexpr (TABLE) {
+		for (uint32_t x = threadIdx.x; x < a.sub.table_bytes / 16u; x += blockDim.x)
+			((uint4 *)tab)[x] = __ldg((const uint4 *)a.sub.table + x);
+		__syncthreads();
+	}
 
 	const int m = a.m, u = a.u, o = a.o, e = a.e;
 	CellConst<PACKED> cc;
@@ -182,10 +197,13 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 					ring16[slot] = (uint16_t)v;
 					if (slot < AT_RING_MIRROR) ring16[AT_RING + slot] = (uint16_t)v;
 				} else {
-					uint32_t v = PACKED ? 0x00010001u : 0x2u;      // past the end: never equals a symbol
+					uint32_t v = PACKED ? 0x00010001u : TABLE ? 0u : 0x2u;      // past the end: never equals a symbol (TABLE: target code 0)
 					if (idx < l2) {
 						if (PACKED) v = ((uint32_t)__ldg(tA + idx) << 8) | ((uint32_t)__ldg(tB + idx) << 24);
-						else { v = (uint32_t)__ldg(tA + idx) << 16; if (JUMP) v |= __ldg(jm + idx) ? 1u : 0u; }
+						else {
+							v = TABLE ? (uint32_t)__ldg(a.sub.tcol + __ldg(tA + idx)) : (uint32_t)__ldg(tA + idx) << 16;
+							if (JUMP) v |= __ldg(jm + idx) ? 1u : 0u;
+						}
 					}
 					ring[slot] = v;
 					if (slot < AT_RING_MIRROR) ring[AT_RING + slot] = v;
@@ -217,7 +235,8 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 				const uint32_t ka = ri < l1A ? (uint32_t)(5 - r) : 0x8000u, kb = ri < l1B ? (uint32_t)(5 - r) : 0x8000u;
 				crow[r] = (T)((ka & 0xffffu) | ((kb & 0xffffu) << 16));
 			} else {
-				if (!PROF) ac[r] = ri < l1A ? ((uint32_t)qA[ri] << SHIFT) : 0x4u;
+				if (TABLE) ac[r] = ri < l1A ? __ldg(a.sub.qrow + qA[ri]) : 0u;      // padded rows: any row of the table
+				else if (!PROF) ac[r] = ri < l1A ? ((uint32_t)qA[ri] << SHIFT) : 0x4u;
 				crow[r] = (T)(ri < l1A ? 5 - r : -(1 << 28));
 			}
 			// column 0 (left border), tags as cell_update leaves them: mo 3, u 1, h = the winner's
@@ -233,7 +252,12 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 #pragma unroll
 				for (int c = 0; c < 4; ++c) {
 					const uint32_t sy = twobit ? (uint32_t)c : (a.syms >> (8 * c)) & 255u;
-					sa[c] = 8 * (qa == sy ? m : u); sb[c] = 8 * (qb == sy ? m : u);
+					if constexpr (SCORED) {      // the matrix entries of the read and target BYTES (2-bit codes stand for A C G T)
+						const uint32_t ty = twobit ? (0x54474341u >> (8 * c)) & 255u : sy;
+						const uint32_t ya = twobit ? (0x54474341u >> (8 * (qa & 3u))) & 255u : qa & 255u, yb = twobit ? (0x54474341u >> (8 * (qb & 3u))) & 255u : qb & 255u;
+						sa[c] = qa < 0x100u ? 8 * (int)__ldg(a.sub.matrix + ya * 256u + ty) : 0;
+						sb[c] = qb < 0x100u ? 8 * (int)__ldg(a.sub.matrix + yb * 256u + ty) : 0;
+					} else { sa[c] = 8 * (qa == sy ? m : u); sb[c] = 8 * (qb == sy ? m : u); }
 				}
 #pragma unroll
 				for (int c = 0; c < NC; ++c)
@@ -318,6 +342,7 @@ __global__ void __launch_bounds__(32 * AT_FILL_WARPS, (PACKED && R <= 5) ? 5 : (
 				for (int r = 0; r < R; ++r) {
 					T s8;                                      // 8 s(i, j)
 					if (PROF) s8 = (T)pw[r];
+					else if (TABLE) s8 = (T)*(const int16_t *)(tab + ac[r] + c);
 					else {                                     // tt: 0 on a match, 8|m-u| otherwise (per half); plain-add form
 						const T tt = PACKED ? (T)__vminu2(ac[r] ^ c, mu8) : (T)min(ac[r] ^ c, mu8);
 						s8 = tt * (T)nsg + m8;

@@ -9,6 +9,8 @@
 //                                    every length;
 //     at_wave_edit_bits<R>         : bit-parallel (Myers) unit-cost edit distance in the same stripe
 //                                    pipeline                                   (at_wavefront.cuh)
+//     SCORED (last template flag of K1 / K2's affine and linear kernels): substitution-matrix scoring -- the profile
+//                                    from the matrix (PROF), or a compact byte table in shared memory (SubstArgs)
 // K3  at_traceback_walk            : device traceback, one thread per pair chases the pointers
 //                                    once and leaves the reversed run-length ops in scratch;
 //     at_traceback_emit            : one warp per pair writes the dense CIGAR and replays it over
@@ -45,6 +47,17 @@ namespace atb2 {
 enum { MODE_GLOBAL = 0, MODE_LOCAL = 1, MODE_FIT = 2, MODE_OVERLAP = 3, MODE_EDIT = 4 };
 enum { ST_LOW = 0, ST_MID = 1, ST_UPP = 2, ST_JUMP = 3 };   // also the 2-bit pointerM codes
 enum { CIG_M = 0, CIG_I = 1, CIG_D = 2, CIG_N = 3 };
+
+// Substitution-matrix scoring (at_batch_*_scored), read by the SCORED instantiations of K1 and K2 only.  Profile variants
+// read `matrix` when they build their profile; the table variants copy `table` into shared memory and index it with
+// qrow[read byte] + tcol[target byte] (byte offsets: the shard's alphabets compacted to codes, rows of int16 values).
+struct SubstArgs {
+	const int8_t   *matrix;       // the caller's 256 x 256 table, s(a, b) = matrix[a * 256 + b]
+	const int16_t  *table;        // [read code][target code]: 8 s (affine kernels) or 4 s (overlap)
+	const uint32_t *qrow;         // read byte -> byte offset of its row in `table`
+	const uint16_t *tcol;         // target byte -> byte offset of its column within a row (2 x code)
+	uint32_t        table_bytes;  // size of `table`, a multiple of 16
+};
 
 }  // namespace atb2
 #include "at_fill_affine.cuh"

@@ -50,6 +50,17 @@ inline P16Rule p16_rule(int mode, const at_params &p, bool jump, bool no_p16)
 	r.on = (r.local || mode == AT_GLOBAL || (mode == AT_FIT && !jump)) && iabs((int64_t)p.m - p.u) <= 31 && (r.local || r.maxabs <= 31) && !no_p16;
 	return r;
 }
+// Substitution-matrix scoring (at_batch_*_scored): `mat_maxabs` = max |s(a, b)| stands for m and u.  Packed lanes then run only
+// the profile variant, whose words hold the matrix values themselves, so the symbol-shift limit on |m - u| does not apply.
+inline P16Rule p16_rule(int mode, const at_params &p, bool jump, bool no_p16, int64_t mat_maxabs)
+{
+	auto iabs = [](int64_t x) { return x < 0 ? -x : x; };
+	P16Rule r;
+	r.local = mode == AT_LOCAL;
+	r.maxabs = std::max<int64_t>({mat_maxabs, iabs(p.o), iabs(p.e), 1});
+	r.on = (r.local || mode == AT_GLOBAL || (mode == AT_FIT && !jump)) && (r.local || r.maxabs <= 31) && !no_p16;
+	return r;
+}
 
 // Bit-parallel edit distance: r = 32-row blocks per lane, 1024 r rows per stripe.  One column step of a lane is a serial
 // chain through its r blocks, so few long pairs want r = 1 (more stripes in flight); 4 blocks per lane amortise the

@@ -194,6 +194,13 @@ struct Shard {
 	bool twobit = false;                       // the sequences stay 2-bit packed in HBM (AT_SEQ_2BIT input consumed directly by K1 / K2 / K3)
 	bool banded = false;                       // overlap / global with a per-pair band: d_band holds it clipped (at_band.h)
 	DevBuf<int2> d_band;
+	bool table = false;                        // substitution matrix, target alphabet of > 4 bytes: the TABLE variants of K1 / K2
+	DevBuf<int8_t> d_subst;                    // substitution matrix, profile variants: the caller's 256 x 256 table
+	DevBuf<int16_t> d_stab; DevBuf<uint32_t> d_qrow; DevBuf<uint16_t> d_tcol;      // ... table variants: SubstArgs
+	uint32_t stab_bytes = 0;
+	// what the substitution buffers above hold (a pipeline workspace keeps them from one sub-slice to the next): the matrix
+	// the profile variants read, and the (scale, read set, target set, matrix) the table was built from
+	std::vector<int8_t> up_matrix, up_table_matrix; std::vector<uint32_t> up_table_key;
 	std::vector<uint64_t> h_t_rel;             // twobit + jump: device offsets of the packed targets (the jump masks copy their alignment)
 	DevBuf<uint64_t> d_j_off;                  // twobit + jump: per-pair offsets into d_jmask (byte-encoded targets use d_t_off)
 	BufCache cache;                            // released device blocks, reused by this shard's next allocations
@@ -231,6 +238,7 @@ static cudaError_t shard_sync(Shard &s)
 struct at_batch {
 	at_handle *h = nullptr;
 	int mode = 0; at_params prm; uint32_t out_flags = 0;
+	std::vector<int8_t> subst;                 // substitution matrix (at_batch_*_scored): 256 x 256, empty = match / mismatch scoring
 	uint64_t n = 0;
 	bool traceback = false;
 	std::vector<Shard> shards;
@@ -332,6 +340,8 @@ static void free_shard(Shard &s)
 	s.ws_cigar.release(); s.ws_aln1.release(); s.ws_aln2.release();
 	s.d_score.release(); s.d_sites.release(); s.d_ptr.release(); s.d_scratch.release(); s.d_bnd.release(); s.d_scan_tmp.release();
 	s.d_prog.release(); s.d_chain.release(); s.d_symmap.release(); s.d_symset.release(); s.d_band.release();
+	s.d_subst.release(); s.d_stab.release(); s.d_qrow.release(); s.d_tcol.release();
+	s.up_matrix.clear(); s.up_table_matrix.clear(); s.up_table_key.clear();
 	release_chunks(s);
 	for (auto &e : s.ev) if (e) cudaEventDestroy(e);
 	for (auto &e : s.evk) if (e) cudaEventDestroy(e);
@@ -373,11 +383,13 @@ static int upload_symmap(at_handle *h, Shard &s, const uint8_t map[256])
 //   s.prof  query-profile variant of K1 / K2 -- the TARGETS use at most 4 distinct bytes (symmap: target byte -> 0..3);
 //   s.bits  bit-parallel kernel for `edit -u 1` -- the READS use at most 8 distinct bytes (symmap: read byte -> 0..7,
 //           anything else -> 8).  The two are exclusive: symmap describes one side.
+//   s.table substitution matrix with more than 4 target bytes: the table variants (upload_subst_table).
+static int upload_subst_table(at_batch *b, Shard &s, uint64_t q_span, const uint32_t *tset);
 static int choose_variants(at_batch *b, Shard &s, const at_batch_input *in, uint64_t q_span)
 {
 	at_handle *h = b->h;
 	int rc;
-	s.prof = false; s.bits = false; s.syms = 0;
+	s.prof = false; s.bits = false; s.syms = 0; s.table = false;
 	const bool two_bit = in->encoding == AT_SEQ_2BIT;                  // the alphabet is ACGT by construction
 	uint32_t set8[8];
 	uint8_t map[256];
@@ -393,7 +405,10 @@ static int choose_variants(at_batch *b, Shard &s, const at_batch_input *in, uint
 		if (nsym >= 1 && nsym <= 8) { s.bits = true; return upload_symmap(h, s, map); }
 		return AT_OK;                                                  // large read alphabet: cell-by-cell kernel, xor/min variant
 	}
-	if (getenv("AT_NO_PROFILE")) return AT_OK;
+	const bool scored = !b->subst.empty();
+	// AT_NO_PROFILE: a scored batch takes the table variants whatever its alphabet.  They read byte-encoded sequences, which
+	// setup_shard guarantees: AT_NO_PROFILE also turns 2-bit residency off (2-bit input is expanded to bytes on upload).
+	if (getenv("AT_NO_PROFILE")) return scored ? upload_subst_table(b, s, q_span, nullptr) : AT_OK;
 	memset(map, 0, sizeof map);
 	int nsym = 0; uint32_t syms = 0;
 	if (two_bit) { map['C'] = 1; map['G'] = 2; map['T'] = 3; nsym = 4; syms = (uint32_t)'A' | ((uint32_t)'C' << 8) | ((uint32_t)'G' << 16) | ((uint32_t)'T' << 24); }
@@ -403,10 +418,64 @@ static int choose_variants(at_batch *b, Shard &s, const at_batch_input *in, uint
 		for (int c = 0; c < 256; ++c)
 			if (set8[c >> 5] >> (c & 31) & 1u) { if (nsym < 4) { map[c] = (uint8_t)nsym; syms |= (uint32_t)c << (8 * nsym); } ++nsym; }
 	}
-	if (nsym < 1 || nsym > 4) return AT_OK;
+	if (nsym < 1 || nsym > 4) return scored ? upload_subst_table(b, s, q_span, set8) : AT_OK;      // (2-bit input has nsym = 4: set8 is the scan's)
 	for (int c = nsym; c < 4; ++c) syms |= (syms & 255u) << (8 * c);   // unused codes repeat a used symbol (they are never looked up)
 	s.syms = syms; s.prof = true;
+	if (scored && !(s.d_subst.p && s.up_matrix == b->subst)) {      // the profile variants build their profiles from the matrix itself
+		CU(h, s.d_subst.alloc(65536));
+		CU(h, cudaMemcpyAsync(s.d_subst.p, b->subst.data(), 65536, cudaMemcpyHostToDevice, s.stream));      // pageable: staged before the call returns
+		s.up_matrix = b->subst;
+	}
 	return upload_symmap(h, s, map);
+}
+
+// Substitution matrix, target alphabet of more than 4 bytes: the shard's read and target alphabets compacted to codes (in
+// byte order) and one int16 table [read code][target code] of what the kernels add per cell -- 8 s for the affine kernels, 4 s
+// for overlap's -- with the byte offsets of every read byte's row and every target byte's column.  The kernels copy the table
+// into shared memory (up to 128 KB for 256 x 256 symbols; a few hundred bytes for protein).  `tset`: the target alphabet when the
+// caller has scanned it already (NULL: scanned here).  A shard that already holds the table of the same alphabets and matrix
+// (the next sub-slice of a pipeline workspace) keeps it.
+static int upload_subst_table(at_batch *b, Shard &s, uint64_t q_span, const uint32_t *tset)
+{
+	at_handle *h = b->h;
+	int rc;
+	const int scale = b->mode == AT_OVERLAP ? 4 : 8;
+	std::vector<uint32_t> key(17);      // scale, read set, target set
+	key[0] = (uint32_t)scale;
+	if ((rc = scan_alphabet(h, s, s.d_q.p, q_span, key.data() + 1))) return rc;
+	if (tset) std::copy(tset, tset + 8, key.begin() + 9);
+	else if ((rc = scan_alphabet(h, s, s.d_t.p, s.t_span, key.data() + 9))) return rc;
+	s.table = true;
+	if (s.d_stab.p && key == s.up_table_key && b->subst == s.up_table_matrix) return AT_OK;
+	const uint32_t *qset = key.data() + 1, *tst = key.data() + 9;
+	std::vector<int> qb, tb;      // the bytes of each code
+	for (int c = 0; c < 256; ++c) { if (qset[c >> 5] >> (c & 31) & 1u) qb.push_back(c); if (tst[c >> 5] >> (c & 31) & 1u) tb.push_back(c); }
+	if (qb.empty()) qb.push_back(0);
+	if (tb.empty()) tb.push_back(0);
+	const size_t nq = qb.size(), nt = tb.size();
+	std::vector<int16_t> tab(((nq * nt * 2 + 15) & ~(size_t)15) / 2, 0);
+	for (size_t x = 0; x < nq; ++x)
+		for (size_t y = 0; y < nt; ++y) tab[x * nt + y] = (int16_t)(scale * b->subst[qb[x] * 256 + tb[y]]);
+	std::vector<uint32_t> qrow(256, 0);      // bytes outside the alphabet never occur: row 0
+	std::vector<uint16_t> tcol(256, 0);
+	for (size_t x = 0; x < nq; ++x) qrow[qb[x]] = (uint32_t)(x * nt * 2);
+	for (size_t y = 0; y < nt; ++y) tcol[tb[y]] = (uint16_t)(y * 2);
+	s.stab_bytes = (uint32_t)(tab.size() * 2);
+	CU(h, s.d_stab.alloc(tab.size())); CU(h, s.d_qrow.alloc(256)); CU(h, s.d_tcol.alloc(256));
+	cudaStream_t st = s.stream;      // pageable host vectors: each copy is staged before cudaMemcpyAsync returns
+	CU(h, cudaMemcpyAsync(s.d_stab.p, tab.data(), s.stab_bytes, cudaMemcpyHostToDevice, st));
+	CU(h, cudaMemcpyAsync(s.d_qrow.p, qrow.data(), 256 * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+	CU(h, cudaMemcpyAsync(s.d_tcol.p, tcol.data(), 256 * sizeof(uint16_t), cudaMemcpyHostToDevice, st));
+	s.up_table_key.swap(key); s.up_table_matrix = b->subst;
+	return AT_OK;
+}
+
+// max |s(a, b)| of a substitution matrix (256 x 256)
+static int64_t subst_maxabs(const int8_t *mat)
+{
+	int64_t v = 0;
+	for (int k = 0; k < 65536; ++k) v = std::max<int64_t>(v, mat[k] < 0 ? -(int64_t)mat[k] : mat[k]);
+	return v;
 }
 
 // fit+jump: the per-pair blacklists as a byte mask aligned with the target bytes (at_build_jmask)
@@ -517,7 +586,9 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 	pin.mode = b->mode; pin.traceback = b->traceback; pin.jump = jump;
 	pin.band = s.banded ? bands.data() : nullptr;
 	pin.bits = s.bits; pin.bits_r = (uint32_t)s.bits_r;
-	pin.p16 = p16_rule(b->mode, b->prm, jump, getenv("AT_NO_P16") != nullptr);
+	// substitution matrix: packed lanes only with the profile variant (the table variant runs on int32 lanes)
+	if (b->subst.empty()) pin.p16 = p16_rule(b->mode, b->prm, jump, getenv("AT_NO_P16") != nullptr);
+	else if (s.prof) pin.p16 = p16_rule(b->mode, b->prm, jump, getenv("AT_NO_P16") != nullptr, subst_maxabs(b->subst.data()));
 	pin.allow_uniform = !getenv("AT_NO_UNIFORM_PLAN");
 	static const bool pair_major = [] { const char *e = getenv("AT_WAVE_ORDER"); return e && !strcmp(e, "pair"); }();
 	pin.pair_major = pair_major;
@@ -617,8 +688,9 @@ static int setup_shard(at_batch *b, Shard &s, const at_batch_input *in, const at
 // so that the one-shot path validates, counts and slices a million-pair batch in one pass
 // `wave_tasks` (optional): number of K2 tasks -- (pair, stripe of 256 rows) -- the batch will run as, 0 for pairs that go to K1:
 // the one-shot path sizes its sub-slices so that each still fills the GPU several times over
+// `sc` (optional): a substitution matrix, whose largest entry stands for m and u in the score-range bound
 static int validate_batch(at_handle *h, int mode, const at_params *p, const at_batch_input *in, std::vector<uint64_t> *prefix = nullptr,
-                          uint64_t *wave_tasks = nullptr)
+                          uint64_t *wave_tasks = nullptr, const at_scoring *sc = nullptr)
 {
 	if (mode < AT_GLOBAL || mode > AT_EDIT) { set_err(h, "bad mode %d", mode); return AT_E_ARG; }
 	if (!in->n_pairs || !in->q || !in->q_off || !in->q_len || !in->t || !in->t_off || !in->t_len) { set_err(h, "align: parameter error"); return AT_E_ARG; }
@@ -630,6 +702,7 @@ static int validate_batch(at_handle *h, int mode, const at_params *p, const at_b
 			if (in->site_off[k + 1] < in->site_off[k] || in->site_off[k + 1] - in->site_off[0] > (1ull << 40)) { set_err(h, "site_off is not ascending at pair %llu", (unsigned long long)k); return AT_E_ARG; }
 	}
 	int64_t maxabs = std::max<int64_t>({llabs((long long)p->m), llabs((long long)p->u), llabs((long long)p->o), llabs((long long)p->e), llabs((long long)p->j), 1});
+	if (sc) maxabs = std::max<int64_t>({subst_maxabs(sc->matrix), llabs((long long)p->o), llabs((long long)p->e), llabs((long long)p->j), 1});
 	// Score lanes hold values x8.  With B = 8 (l1 + l2 + 2) maxabs bounding every finite value, a -inf stand-in
 	// (AT_NEG = -2^29, at_kernels.cuh) that has drifted by up to B must still lose against every finite value:
 	// AT_NEG + B < -B  <=>  (l1 + l2 + 2) * maxabs < 2^25.  (AT_NEG_INIT - B stays above INT32_MIN with room to spare.)
@@ -702,12 +775,22 @@ static bool wants_traceback(int mode, uint32_t out_flags)
 	return mode != AT_EDIT || (out_flags & AT_OUT_EDIT_PATH);
 }
 
-static at_batch *new_batch(at_handle *h, int mode, const at_params *p, uint32_t out_flags, uint64_t n)
+static at_batch *new_batch(at_handle *h, int mode, const at_params *p, uint32_t out_flags, uint64_t n, const at_scoring *sc = nullptr)
 {
 	at_batch *b = new at_batch();
 	b->h = h; b->mode = mode; b->prm = *p; b->out_flags = out_flags; b->n = n;
 	b->traceback = wants_traceback(mode, out_flags);
+	if (sc) b->subst.assign(sc->matrix, sc->matrix + 65536);
 	return b;
+}
+
+// a substitution matrix is for global, local, fit and overlap, and must be there
+static int validate_scoring(at_handle *h, int mode, const at_scoring *sc)
+{
+	if (!sc) return AT_OK;
+	if (mode == AT_EDIT) { set_err(h, "scoring: edit distance takes no substitution matrix"); return AT_E_ARG; }
+	if (!sc->matrix) { set_err(h, "scoring: matrix is NULL"); return AT_E_ARG; }
+	return AT_OK;
 }
 
 // a band is for AT_OVERLAP and AT_GLOBAL, with both arrays and lo[p] <= hi[p] for every pair; a global pair's band must
@@ -748,17 +831,36 @@ extern "C" int at_batch_create(at_handle *h, int mode, const at_params *p, const
 	return at_batch_create_banded(h, mode, p, in, nullptr, out_flags, out);
 }
 
+static int create_batch(at_handle *h, int mode, const at_params *p, const at_batch_input *in, const at_band *band, const at_scoring *sc,
+                        uint32_t out_flags, at_batch **out);
+
 extern "C" int at_batch_create_banded(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
                                       const at_band *band, uint32_t out_flags, at_batch **out)
+{
+	return create_batch(h, mode, p, in, band, nullptr, out_flags, out);
+}
+
+extern "C" int at_batch_create_scored(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
+                                      const at_scoring *sc, uint32_t out_flags, at_batch **out)
+{
+	if (!h || !p || !in || !out) return AT_E_ARG;
+	*out = nullptr;
+	if (int rc = validate_scoring(h, mode, sc)) return rc;
+	return create_batch(h, mode, p, in, nullptr, sc, out_flags, out);
+}
+
+// `band` / `sc` (NULL: none): at most one of the two is given
+static int create_batch(at_handle *h, int mode, const at_params *p, const at_batch_input *in, const at_band *band, const at_scoring *sc,
+                        uint32_t out_flags, at_batch **out)
 {
 	if (!h || !p || !in || !out) return AT_E_ARG;
 	*out = nullptr;
 	// contiguous slices balanced by cells (one device: no running cell counts needed)
 	const size_t nd = h->devs.size();
 	std::vector<uint64_t> prefix, cut;
-	if (int rc = validate_batch(h, mode, p, in, nd > 1 ? &prefix : nullptr)) return rc;
+	if (int rc = validate_batch(h, mode, p, in, nd > 1 ? &prefix : nullptr, nullptr, sc)) return rc;
 	if (int rc = validate_band(h, mode, in, band)) return rc;
-	at_batch *b = new_batch(h, mode, p, out_flags, in->n_pairs);
+	at_batch *b = new_batch(h, mode, p, out_flags, in->n_pairs, sc);
 	cut_by_prefix(prefix, 0, b->n, nd, cut);
 	b->shards.resize(nd);
 	std::vector<std::thread> th;
@@ -781,33 +883,39 @@ extern "C" int at_batch_create_banded(at_handle *h, int mode, const at_params *p
 typedef void (*fill2_fn)(const FillArgs2);
 typedef void (*wave_fn)(const WaveArgs);
 
-template <int R, bool PROF> static fill2_fn affine_fn(int kind)
+// SCORED: substitution-matrix scoring (the table variant, !PROF, has no packed kinds: p16 is off for it)
+template <int R, bool PROF, bool SCORED = false> static fill2_fn affine_fn(int kind)
 {
+	constexpr bool PK = !SCORED || PROF;      // packed kinds exist
 	switch (kind) {
-	case 0: return at_fill_affine<MODE_GLOBAL, R, false, false, PROF>;
-	case 1: return at_fill_affine<MODE_LOCAL, R, false, false, PROF>;
-	case 2: return at_fill_affine<MODE_FIT, R, false, false, PROF>;
-	case 3: return at_fill_affine<MODE_FIT, R, true, false, PROF>;
-	case 4: return at_fill_affine<MODE_LOCAL, R, false, true, PROF>;
-	case 5: return at_fill_affine<MODE_GLOBAL, R, false, true, PROF>;
-	default: return at_fill_affine<MODE_FIT, R, false, true, PROF>;
+	case 0: return at_fill_affine<MODE_GLOBAL, R, false, false, PROF, SCORED>;
+	case 1: return at_fill_affine<MODE_LOCAL, R, false, false, PROF, SCORED>;
+	case 2: return at_fill_affine<MODE_FIT, R, false, false, PROF, SCORED>;
+	case 3: return at_fill_affine<MODE_FIT, R, true, false, PROF, SCORED>;
+	case 4: return at_fill_affine<MODE_LOCAL, R, false, PK, PROF, SCORED>;
+	case 5: return at_fill_affine<MODE_GLOBAL, R, false, PK, PROF, SCORED>;
+	default: return at_fill_affine<MODE_FIT, R, false, PK, PROF, SCORED>;
 	}
 }
-template <bool PROF> static fill2_fn affine_kernel_r(int kind, int R)
+template <bool PROF, bool SCORED = false> static fill2_fn affine_kernel_r(int kind, int R)
 {
 	switch (R) {
-	case 1: return affine_fn<1, PROF>(kind); case 2: return affine_fn<2, PROF>(kind); case 3: return affine_fn<3, PROF>(kind);
-	case 4: return affine_fn<4, PROF>(kind); case 5: return affine_fn<5, PROF>(kind); case 6: return affine_fn<6, PROF>(kind);
-	case 7: return affine_fn<7, PROF>(kind); default: return affine_fn<8, PROF>(kind);
+	case 1: return affine_fn<1, PROF, SCORED>(kind); case 2: return affine_fn<2, PROF, SCORED>(kind); case 3: return affine_fn<3, PROF, SCORED>(kind);
+	case 4: return affine_fn<4, PROF, SCORED>(kind); case 5: return affine_fn<5, PROF, SCORED>(kind); case 6: return affine_fn<6, PROF, SCORED>(kind);
+	case 7: return affine_fn<7, PROF, SCORED>(kind); default: return affine_fn<8, PROF, SCORED>(kind);
 	}
 }
-static fill2_fn affine_kernel(int kind, int R, bool prof) { return prof ? affine_kernel_r<true>(kind, R) : affine_kernel_r<false>(kind, R); }
-template <int MODE, bool PROF, bool BANDED = false, bool PTR = false> static wave_fn wave_linear_fn(int R)
+static fill2_fn affine_kernel(int kind, int R, bool prof, bool scored)
+{
+	if (scored) return prof ? affine_kernel_r<true, true>(kind, R) : affine_kernel_r<false, true>(kind, R);
+	return prof ? affine_kernel_r<true>(kind, R) : affine_kernel_r<false>(kind, R);
+}
+template <int MODE, bool PROF, bool BANDED = false, bool PTR = false, bool SCORED = false> static wave_fn wave_linear_fn(int R)
 {
 	switch (R) {
-	case 1: return at_wave_linear<MODE, 1, PROF, BANDED, PTR>; case 2: return at_wave_linear<MODE, 2, PROF, BANDED, PTR>; case 3: return at_wave_linear<MODE, 3, PROF, BANDED, PTR>;
-	case 4: return at_wave_linear<MODE, 4, PROF, BANDED, PTR>; case 5: return at_wave_linear<MODE, 5, PROF, BANDED, PTR>; case 6: return at_wave_linear<MODE, 6, PROF, BANDED, PTR>;
-	case 7: return at_wave_linear<MODE, 7, PROF, BANDED, PTR>; default: return at_wave_linear<MODE, 8, PROF, BANDED, PTR>;
+	case 1: return at_wave_linear<MODE, 1, PROF, BANDED, PTR, SCORED>; case 2: return at_wave_linear<MODE, 2, PROF, BANDED, PTR, SCORED>; case 3: return at_wave_linear<MODE, 3, PROF, BANDED, PTR, SCORED>;
+	case 4: return at_wave_linear<MODE, 4, PROF, BANDED, PTR, SCORED>; case 5: return at_wave_linear<MODE, 5, PROF, BANDED, PTR, SCORED>; case 6: return at_wave_linear<MODE, 6, PROF, BANDED, PTR, SCORED>;
+	case 7: return at_wave_linear<MODE, 7, PROF, BANDED, PTR, SCORED>; default: return at_wave_linear<MODE, 8, PROF, BANDED, PTR, SCORED>;
 	}
 }
 // banded overlap / global (validate_band admits a band with AT_OVERLAP and AT_GLOBAL only)
@@ -835,7 +943,26 @@ static wave_fn wave_kernel(int mode, bool jump, int R, bool prof, bool path)
 	}
 }
 
+// substitution-matrix scoring (global, local, fit, overlap; validate_scoring): the SCORED instantiations
+static wave_fn wave_scored_kernel(int mode, bool jump, int R, bool prof)
+{
+	switch (mode) {
+	case AT_GLOBAL: return prof ? at_wave_affine<MODE_GLOBAL, false, true, false, true> : at_wave_affine<MODE_GLOBAL, false, false, false, true>;
+	case AT_LOCAL: return prof ? at_wave_affine<MODE_LOCAL, false, true, false, true> : at_wave_affine<MODE_LOCAL, false, false, false, true>;
+	case AT_FIT: return jump ? (prof ? at_wave_affine<MODE_FIT, true, true, false, true> : at_wave_affine<MODE_FIT, true, false, false, true>)
+	                         : (prof ? at_wave_affine<MODE_FIT, false, true, false, true> : at_wave_affine<MODE_FIT, false, false, false, true>);
+	default: return prof ? wave_linear_fn<MODE_OVERLAP, true, false, false, true>(R) : wave_linear_fn<MODE_OVERLAP, false, false, false, true>(R);
+	}
+}
+
 struct CastU64 { __host__ __device__ uint64_t operator()(const uint32_t &x) const { return (uint64_t)x; } };
+
+static SubstArgs subst_args(const Shard &s)
+{
+	SubstArgs a;
+	a.matrix = s.d_subst.p; a.table = s.d_stab.p; a.qrow = s.d_qrow.p; a.tcol = s.d_tcol.p; a.table_bytes = s.table ? s.stab_bytes : 0;
+	return a;
+}
 
 // `fills_done` (optional) is called once, when the next sub-slice of the pipelined one-shot path may
 // launch its fill: after this shard's last traceback kernel has been enqueued (score-only: after its
@@ -871,11 +998,18 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 		if (first) { CU(h, cudaEventRecord(e_first, st)); first = false; }
 		for (size_t li = 0; li < c.launches.size(); ++li) {
 			const PlanLaunch &l = c.launches[li];
-			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r, b->traceback) : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(b->mode, l.r, s.prof) : (const void *)wave_kernel(b->mode, jump, l.r, s.prof, b->traceback))
-			                                   : (const void *)affine_kernel(l.kind == LK_PACKED ? (b->mode == AT_LOCAL ? 4 : b->mode == AT_GLOBAL ? 5 : 6) : (b->mode == AT_FIT ? (jump ? 3 : 2) : b->mode), l.r, s.prof);
+			const bool scored = !b->subst.empty();
+			const void *fn = l.kind == LK_BITS ? (const void *)bits_kernel(l.r, b->traceback)
+			               : l.kind == LK_WAVE ? (s.banded ? (const void *)wave_banded_kernel(b->mode, l.r, s.prof)
+			                                     : scored ? (const void *)wave_scored_kernel(b->mode, jump, l.r, s.prof)
+			                                     : (const void *)wave_kernel(b->mode, jump, l.r, s.prof, b->traceback))
+			               : (const void *)affine_kernel(l.kind == LK_PACKED ? (b->mode == AT_LOCAL ? 4 : b->mode == AT_GLOBAL ? 5 : 6) : (b->mode == AT_FIT ? (jump ? 3 : 2) : b->mode), l.r, s.prof, scored);
 			const int warps = l.kind >= LK_WAVE ? AT_WAVE_WARPS : AT_FILL_WARPS;
-			const size_t dyn_smem = l.kind >= LK_WAVE ? 0 : fill_smem_bytes(l.r, l.kind == LK_PACKED, s.prof);
-			if (dyn_smem > 48 * 1024) CU(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem));
+			const size_t dyn_smem = l.kind >= LK_WAVE ? (s.table ? wave_smem_bytes_table(s.stab_bytes) : 0)
+			                      : s.table ? fill_smem_bytes_table(l.r, s.stab_bytes) : fill_smem_bytes(l.r, l.kind == LK_PACKED, s.prof);
+			// the opt-in above 48 KB counts static and dynamic shared memory together: the K2 table variants have both, so every
+			// table launch states its dynamic size (K1 has no static shared memory)
+			if (dyn_smem > 48 * 1024 || s.table) CU(h, cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn_smem));
 			int occ = 0;
 			CU(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, fn, 32 * warps, dyn_smem));
 			if (occ < 1) { set_err(h, "fill kernel (mode %d, R %d) cannot be resident: not an sm_100 build?", b->mode, l.r); return AT_E_CUDA; }
@@ -900,8 +1034,9 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 				wa.want_ptr = b->traceback ? 1 : 0;
 				wa.k_and = cell_k_and<false>(); wa.k_or = cell_k_or<false>();
 				wa.band = s.banded ? s.d_band.p : nullptr;
+				wa.sub = subst_args(s);
 				void *kargs[] = {(void *)&wa};
-				CU(h, cudaLaunchKernel(fn, dim3(blocks), dim3(32 * warps), kargs, 0, st));
+				CU(h, cudaLaunchKernel(fn, dim3(blocks), dim3(32 * warps), kargs, dyn_smem, st));
 			} else {
 				FillArgs2 fa;
 				fa.q = s.d_q.p; fa.q_off = s.d_q_off.p; fa.q_len = s.d_q_len.p;
@@ -913,6 +1048,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 				fa.m = b->prm.m; fa.u = b->prm.u; fa.o = b->prm.o; fa.e = b->prm.e; fa.jp = b->prm.j;
 				fa.want_ptr = b->traceback ? 1 : 0; fa.twobit = s.twobit ? 1 : 0;
 				fa.k_and = l.kind == LK_PACKED ? cell_k_and<true>() : cell_k_and<false>(); fa.k_or = l.kind == LK_PACKED ? cell_k_or<true>() : cell_k_or<false>();
+				fa.sub = subst_args(s);
 				void *kargs[] = {(void *)&fa};
 				CU(h, cudaLaunchKernel(fn, dim3(blocks), dim3(32 * warps), kargs, dyn_smem, st));
 			}
@@ -1016,7 +1152,7 @@ static int run_shard(at_batch *b, Shard &s, const std::function<void()> *fills_d
 		if ((int)ci == dom_chunk) {
 			CU(h, cudaEventElapsedTime(&ms, s.evk[0], s.evk[1])); s.domk_ms = ms; s.domk_cells = dom_cells;
 			const PlanLaunch &dl = c.launches[dom_launch];
-			s.domk_kind = (uint32_t)dl.kind; s.domk_r = (uint32_t)dl.r; s.domk_flags = (s.prof ? 1u : 0u) | (jump ? 2u : 0u) | (s.twobit ? 4u : 0u);
+			s.domk_kind = (uint32_t)dl.kind; s.domk_r = (uint32_t)dl.r; s.domk_flags = (s.prof ? 1u : 0u) | (jump ? 2u : 0u) | (s.twobit ? 4u : 0u) | (b->subst.empty() ? 0u : 8u);
 		}
 		if (ci + 1 == s.chunks.size()) { CU(h, cudaEventElapsedTime(&ms, e_first, e_tb)); s.dev_ms = ms; }
 	}

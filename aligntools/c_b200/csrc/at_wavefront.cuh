@@ -69,7 +69,17 @@ struct WaveArgs {
 	int             twobit;  // q / t hold 2-bit codes (AT_SEQ_2BIT resident: four symbols per byte, A C G T = 0..3, byte-aligned records)
 	uint32_t        start_lag;   // a stripe starts once the stripe above it has published this many columns (0: as soon as it can)
 	const int2     *band;        // at_wave_linear<.., BANDED>: [pair] clipped band (lo, hi) on j - i (at_band.h)
+	SubstArgs       sub;         // SCORED: the substitution matrix (at_kernels.cuh)
 };
+
+// SCORED && !PROF (table variant): dynamic shared memory of a CTA -- the target byte -> column offset map, then the table
+__host__ __device__ constexpr size_t wave_smem_bytes_table(uint32_t table_bytes) { return 512u + table_bytes; }
+// copy the map and the table (every thread of the CTA; the caller synchronises)
+__device__ __forceinline__ void wave_table_load(const SubstArgs &s, unsigned char *dyn)
+{
+	for (uint32_t x = threadIdx.x; x < 256u; x += blockDim.x) ((uint16_t *)dyn)[x] = __ldg(s.tcol + x);
+	for (uint32_t x = threadIdx.x; x < s.table_bytes / 16u; x += blockDim.x) ((uint4 *)(dyn + 512))[x] = __ldg((const uint4 *)s.table + x);
+}
 
 // ---- TMA (bulk async copy) + mbarrier + release/acquire helpers ----
 __device__ __forceinline__ uint32_t smem_addr(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -210,10 +220,19 @@ __device__ __forceinline__ void wait_columns(const uint32_t *prog, uint32_t need
 // only for columns inside the producer's window and takes -inf for the others (the slab entries outside the window hold
 // values of the stripe two above).  Target tiles keep their absolute numbering, only those the window reads are staged.
 // Pointer words are stored relative to t0 at the stripe's offset in the pair's block (band_stripe_off).
-template <int MODE, bool JUMP, bool PROF, bool BANDED = false>
+//
+// SCORED (substitution matrix, unbanded): PROF builds the profile from the matrix row of the read symbol; otherwise the
+// TABLE variant: ac[r] = byte offset of the row's read code in the compact table (dynamic shared memory), the column's
+// target code comes from the shared map of its ring byte, and 8 s(i, j) is one LDS.S16 per cell.
+template <int MODE, bool JUMP, bool PROF, bool BANDED = false, bool SCORED = false>
 __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BANDED_MINB : AT_WAVE_AFFINE_MINB) at_wave_affine(const WaveArgs a)
 {
 	static_assert(!BANDED || (MODE == MODE_GLOBAL && !JUMP), "banded affine kernel: global alignment only");
+	static_assert(!BANDED || !SCORED, "no band with a substitution matrix");
+	constexpr bool TABLE = SCORED && !PROF;
+	extern __shared__ __align__(16) unsigned char wave_dyn[];          // TABLE: wave_smem_bytes_table
+	const uint16_t *tmap_s = (const uint16_t *)wave_dyn;
+	const unsigned char *tab = wave_dyn + 512;
 	typedef Lanes<false> V;
 	constexpr int R = 8, RPP = 32 * R;
 	constexpr bool LOCAL = MODE == MODE_LOCAL;
@@ -224,6 +243,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 	Smem &sm = sm_all[threadIdx.x >> 5];
 	const int lane = threadIdx.x & 31;
 	if (PROF) { for (int x = threadIdx.x; x < 256; x += blockDim.x) symmap_s[x] = a.symmap[x]; }
+	if (TABLE) wave_table_load(a.sub, wave_dyn);
 	if (lane == 0) { mbar_init(&sm.rg.bar[0], 1); mbar_init(&sm.rg.bar[1], 1); fence_proxy_async_smem(); }
 	__syncthreads();
 	uint32_t ring_par = 0;      // bit s: parity of the next completion of slot s's mbarrier
@@ -299,11 +319,16 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 		for (int r = 0; r < R; ++r) {
 			const uint32_t ri = row0 + r;
 			const int i = (int)ri + 1;
-			ac[r] = ri < l1 ? (read_sym(q, ri, twobit) << 16) : 0x4u;
+			if (TABLE) ac[r] = ri < l1 ? __ldg(a.sub.qrow + read_sym(q, ri, twobit)) : 0u;      // padded rows: any row of the table
+			else ac[r] = ri < l1 ? (read_sym(q, ri, twobit) << 16) : 0x4u;
 			if (PROF) {
 				const uint32_t qa = ri < l1 ? read_sym(q, ri, twobit) : 0x100u;
 #pragma unroll
-				for (int c = 0; c < 4; ++c) sm.prof[c][lane][r] = 8 * (qa == ((a.syms >> (8 * c)) & 255u) ? m : u);
+				for (int c = 0; c < 4; ++c) {
+					const uint32_t sy = (a.syms >> (8 * c)) & 255u;
+					if (SCORED) sm.prof[c][lane][r] = qa < 0x100u ? 8 * (int)__ldg(a.sub.matrix + qa * 256u + sy) : 0;
+					else sm.prof[c][lane][r] = 8 * (qa == sy ? m : u);
+				}
 			}
 			crow[r] = ri < l1 ? 5 - r : -(1 << 28);                       // on top of Mk = 8 M + 2: key = 8 M + 7 - r
 			// column 0 (left border), tags as cell_update leaves them
@@ -385,7 +410,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 			pH = rH;
 			if (!checked || (j >= 1 && j <= (int)l2)) {
 				const uint32_t y = (uint32_t)(j - 1) + sh;
-				const uint32_t c = PROF ? (uint32_t)symmap_s[sm.rg.tring[y & 511u]] : (uint32_t)sm.rg.tring[y & 511u] << 16;
+				const uint32_t c = PROF ? (uint32_t)symmap_s[sm.rg.tring[y & 511u]] : TABLE ? (uint32_t)tmap_s[sm.rg.tring[y & 511u]] : (uint32_t)sm.rg.tring[y & 511u] << 16;
 				int pw[LS];                                                       // PROF: 8 * s of this lane's rows against the column's symbol
 				if (PROF) {
 					const int2 *pp = (const int2 *)&sm.prof[c][lane][0];
@@ -402,6 +427,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 				for (int r = 0; r < R; ++r) {
 					int s8;                                                       // 8 s(i, j)
 					if (PROF) s8 = pw[r];
+					else if (TABLE) s8 = *(const int16_t *)(tab + ac[r] + c);
 					else { const int tt = (int)min(ac[r] ^ c, mu8); s8 = tt * nsg + m8; }   // tt: 0 on a match, 8|m-u| otherwise
 					D = cell_update<LOCAL, JUMP, false, true>(cc, st[r], D, s8, lup, mo_up, jadd, 16u, 2u, out);
 					if (MSK && (uint32_t)(j - (int)row0 - 1 - r - elo) > (uint32_t)(ehi - elo)) {     // d = j - i out of band
@@ -580,10 +606,18 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS, BANDED ? AT_WAVE_AFFINE_BA
 // PTR (edit only, AT_OUT_EDIT_PATH): the cell is edit_min3_tagged() of at_cell.cuh -- the three candidates x4 with min3's
 // argmin code in the low bits (LEFT 0, DIAGONAL 1, UP 2), one VIMNMX3 -- and the codes are stored in overlap's layout
 // (2 bits, 16 steps per word, code = the tag itself), so K3 walks them with overlap's reader.
-template <int MODE, int R, bool PROF, bool BANDED = false, bool PTR = false>
+//
+// SCORED (overlap with a substitution matrix, unbanded): PROF builds 4 (s - o) - 1 from the matrix; otherwise the TABLE
+// variant as in at_wave_affine, whose table holds 4 s (one add of -4 o - 1 per cell).
+template <int MODE, int R, bool PROF, bool BANDED = false, bool PTR = false, bool SCORED = false>
 __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveArgs a)
 {
 	static_assert(!PTR || (MODE == MODE_EDIT && !BANDED), "PTR: the edit kernel's pointers (overlap stores its own)");
+	static_assert(!SCORED || (MODE == MODE_OVERLAP && !BANDED), "substitution matrix: unbanded overlap only");
+	constexpr bool TABLE = SCORED && !PROF;
+	extern __shared__ __align__(16) unsigned char wave_dyn[];          // TABLE: wave_smem_bytes_table
+	const uint16_t *tmap_s = (const uint16_t *)wave_dyn;
+	const unsigned char *tab = wave_dyn + 512;
 	constexpr int RPP = 32 * R;
 	constexpr bool OV = MODE == MODE_OVERLAP;
 	constexpr bool STORE = OV || PTR;      // the kernel writes 2-bit pointer words
@@ -595,6 +629,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 	Smem &sm = sm_all[threadIdx.x >> 5];
 	const int lane = threadIdx.x & 31;
 	if (PROF) { for (int x = threadIdx.x; x < 256; x += blockDim.x) symmap_s[x] = a.symmap[x]; }
+	if (TABLE) wave_table_load(a.sub, wave_dyn);
 	if (lane == 0) { mbar_init(&sm.rg.bar[0], 1); mbar_init(&sm.rg.bar[1], 1); fence_proxy_async_smem(); }
 	__syncthreads();
 	uint32_t ring_par = 0;
@@ -605,6 +640,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 	const int pw_match = OV ? S * (a.m - a.o) - 1 : 0;               // substitution term of a match (overlap: carried value -> tagged diagonal candidate)
 	const uint32_t pen = OV ? (uint32_t)(S * (a.m >= a.u ? a.m - a.u : a.u - a.m)) : (uint32_t)(a.u >= 0 ? a.u : -a.u);
 	const int nsg = OV ? (a.m >= a.u ? -1 : 1) : (a.u >= 0 ? 1 : -1);
+	const int sub_add = -S * a.o - 1;                                  // TABLE: 4 s + sub_add = 4 (s - o) - 1
 	const bool want_ptr = STORE && a.want_ptr != 0;
 	int nz = lane ? 1 : 0;                                            // lane 0 takes the row above the stripe instead of a neighbour
 	asm volatile("" : "+r"(nz));                                      // opaque: keep x * nz + b a multiply-add (FMA pipe), not a SEL
@@ -672,13 +708,18 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 #pragma unroll
 		for (int r = 0; r < R; ++r) {
 			const uint32_t ri = row0 + r;
-			ac[r] = ri < l1 ? (read_sym(q, ri, twobit) << 16) : 0x4u;
+			if (TABLE) ac[r] = ri < l1 ? __ldg(a.sub.qrow + read_sym(q, ri, twobit)) : 0u;      // padded rows: any row of the table
+			else ac[r] = ri < l1 ? (read_sym(q, ri, twobit) << 16) : 0x4u;
 			Vl[r] = (int)ri + 1;
 			stl[r].a2 = gap + 2; stl[r].x = 0;
 			if (PROF) {
 				const uint32_t qa = ri < l1 ? read_sym(q, ri, twobit) : 0x100u;
 #pragma unroll
-				for (int c = 0; c < 4; ++c) sm.prof[c][lane][r] = pw_match + (qa == ((a.syms >> (8 * c)) & 255u) ? 0 : (int)pen * nsg);
+				for (int c = 0; c < 4; ++c) {
+					const uint32_t sy = (a.syms >> (8 * c)) & 255u;
+					if (SCORED) sm.prof[c][lane][r] = qa < 0x100u ? S * ((int)__ldg(a.sub.matrix + qa * 256u + sy) - a.o) - 1 : 0;
+					else sm.prof[c][lane][r] = pw_match + (qa == sy ? 0 : (int)pen * nsg);
+				}
 			}
 		}
 		if (PROF) __syncwarp();
@@ -727,7 +768,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 			pD = rV + dadd;
 			if (!checked || (j >= 1 && j <= (int)l2)) {
 				const uint32_t y = (uint32_t)(j - 1) + sh;
-				const uint32_t c = PROF ? (uint32_t)symmap_s[sm.rg.tring[y & 511u]] : (uint32_t)sm.rg.tring[y & 511u] << 16;
+				const uint32_t c = PROF ? (uint32_t)symmap_s[sm.rg.tring[y & 511u]] : TABLE ? (uint32_t)tmap_s[sm.rg.tring[y & 511u]] : (uint32_t)sm.rg.tring[y & 511u] << 16;
 				int pw[LS];                                                       // PROF: substitution terms of this lane's rows
 				if (PROF) {
 					const int2 *pp = (const int2 *)&sm.prof[c][lane][0];
@@ -739,6 +780,7 @@ __global__ void __launch_bounds__(32 * AT_WAVE_WARPS) at_wave_linear(const WaveA
 				for (int r = 0; r < R; ++r) {
 					int sub;                                                      // substitution term
 					if (PROF) sub = pw[r];
+					else if (TABLE) sub = (int)*(const int16_t *)(tab + ac[r] + c) + sub_add;
 					else { const int tt = (int)min(ac[r] ^ c, pen); sub = tt * nsg + pw_match; }   // tt: 0 on a match
 					if (OV) {
 						int dn;

@@ -16,8 +16,8 @@
  *
  * Conventions (SURVEY.md Appendix A): s1 = first FASTA record = rows i = "read";
  * s2 = second record = columns j = "target".  Scoring is raw byte equality
- * (src/alignment.h:449, 632, 824, 943, 305).  All results are bit-exact with the
- * reference, quirks included (A.6).
+ * (src/alignment.h:449, 632, 824, 943, 305); at_batch_*_scored (section C) takes a substitution
+ * matrix instead.  All results are bit-exact with the reference, quirks included (A.6).
  */
 #ifndef ALIGNTOOLS_B200_H
 #define ALIGNTOOLS_B200_H
@@ -186,7 +186,7 @@ typedef struct at_timing {
 	uint64_t fill_kernel_cells; /* cells one such launch processes                                   */
 	uint32_t fill_kernel_kind;  /* which kernel that was: enum at_kernel_kind                            */
 	uint32_t fill_kernel_rows;  /* its rows per lane (AT_K_EDIT_BITS: 32-row blocks per lane)            */
-	uint32_t fill_kernel_flags; /* bit 0: query-profile variant, bit 1: jump state, bit 2: sequences 2-bit packed in HBM */
+	uint32_t fill_kernel_flags; /* bit 0: query-profile variant, bit 1: jump state, bit 2: sequences 2-bit packed in HBM, bit 3: substitution matrix */
 	uint32_t reserved_;
 } at_timing;
 
@@ -246,6 +246,27 @@ int  at_batch_create_banded(at_handle *h, int mode, const at_params *p, const at
                             const at_band *band, uint32_t out_flags, at_batch **out);
 int  at_batch_align_banded(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
                            const at_band *band, uint32_t out_flags, at_batch_output *out, at_timing *timing);
+
+/* Substitution scores: s(a, b) = matrix[a * 256 + b] for read byte a (s1, rows) and target byte b (s2, columns).
+ * Any byte may occur, the table need not be symmetric, and p->m / p->u are ignored; o, e, j and jump keep their meaning.
+ * AT_SEQ_2BIT input: codes 0..3 stand for the bytes 'A', 'C', 'G', 'T'.
+ * sc == NULL behaves exactly like at_batch_create / at_batch_align.  Modes AT_GLOBAL, AT_LOCAL, AT_FIT (jump 0, 1 or 2) and
+ * AT_OVERLAP keep the reference's recurrence, borders, max5 first-strictly-greater ties, end-cell search (fit still excludes
+ * column l2), traceback and flush; only s(i, j) = s(s1[i-1], s2[j-1]) comes from the table instead of m / u.  Identity: with
+ * matrix[a * 256 + b] = (a == b ? m : u) the results equal at_batch_align's in every field.
+ * AT_E_ARG (at_last_error names the reason): AT_EDIT with a matrix, a NULL matrix.  AT_E_RANGE: the score-range bound of
+ * at_batch_create with max(|o|, |e|, |j|, max |matrix entry|) in place of max(|m|, |u|, ...).
+ * Kernels: when a shard's targets use at most 4 distinct bytes (DNA, every 2-bit batch) the query-profile variants run with
+ * profiles built from the matrix (no extra work per cell); otherwise the table variants look s up per cell in a compact
+ * [read symbol][target symbol] table in shared memory (at_timing.fill_kernel_flags bit 3 marks a scored run, bit 0 the
+ * profile variant).  Results are sized and fetched with at_batch_run / at_batch_sizes / at_batch_fetch as for any batch. */
+typedef struct at_scoring {
+	const int8_t *matrix;  /* [256 * 256] */
+} at_scoring;
+int  at_batch_create_scored(at_handle *h, int mode, const at_params *p, const at_batch_input *in,
+                            const at_scoring *sc, uint32_t out_flags, at_batch **out);
+int  at_batch_align_scored (at_handle *h, int mode, const at_params *p, const at_batch_input *in,
+                            const at_scoring *sc, uint32_t out_flags, at_batch_output *out, at_timing *timing);
 
 /* Sharding plan (SURVEY.md 8e): cut pairs [0, n) into `parts` CONTIGUOUS slices holding nearly equal
  * numbers of DP cells (sum of l1*l2).  cut[] receives parts+1 ascending indices, cut[0] = 0 and
